@@ -2,6 +2,7 @@
 """bench.py -- CSV bytes indexed per second (BASELINE.json metric) on N B200s of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--no-also]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (csv bytes -> structural index) over one batch of synthetic
 CSV.  N=1: BASELINE config 2 (1 GiB unquoted, 16 numeric fields/row, LF).  N>1: BASELINE config 4
@@ -23,6 +24,12 @@ quote-parity exchange inside every step.
   cpu_baseline / --impl reference
              the reference's CPU path (oracle/csv_oracle.c: the literal SSE restatement, 1 thread
              because the reference is a single serial loop) on the box's host cores
+
+--impl reference times exactly --steps passes like the CUDA arm; at about 1 GB/s on one core the default 100 steps
+over 1 GiB take about 100 s, so pass a smaller --steps for a quicker reference line.
+
+--dump-outputs DIR writes the index of the last timed step (all ranks' segments, sampled: dump_index) as float64
+.npy files, at most 64 MB in all, so that two builds of the project can be compared output for output.
 """
 from __future__ import annotations
 
@@ -239,6 +246,48 @@ def run_reference(args, rank: int, world: int):
     print(json.dumps(line), flush=True)
 
 
+DUMP_SAMPLE = 1 << 21        # entries of the seeded random sample of the index, shared by all ranks
+DUMP_EDGE = 1 << 16          # entries kept whole at each end of the index, shared by all ranks
+DUMP_BLOCK = 1 << 16         # entries per block sum: every entry counts, each sum exact in float64
+DUMP_MAX_BYTES = 64 << 20    # all ranks' files together
+
+
+def dump_index(idx, out_dir: str, rank: int = 0, world: int = 1) -> int:
+    """Writes what a caller of the build receives (the host index and its end quote parity) as float64 .npy files;
+    returns the bytes written.  The index itself is too large to store whole, so it is kept as its length, its first
+    and last entries, a sample at positions drawn from a fixed seed, and exact sums of consecutive blocks of
+    DUMP_BLOCK entries (a difference anywhere in the index changes one of them).  Positions are < 2^53, so float64
+    holds them exactly.  With world > 1 every rank writes its own segment (suffix _rank<k>) with 1/world of the
+    sample, the edges and the byte budget, so that all ranks' files together stay within DUMP_MAX_BYTES."""
+    host = idx.to_host()
+    E = host.size
+    sample, edge = DUMP_SAMPLE // world, DUMP_EDGE // world
+    assert E == 0 or int(host.max()) * DUMP_BLOCK < (1 << 53), "index positions too large for exact float64 block sums"
+    pos = np.unique(np.random.default_rng(rank).integers(0, E, size=min(E, sample))) if E else np.zeros(0, np.int64)
+    full = E - E % DUMP_BLOCK
+    sums = host[:full].reshape(-1, DUMP_BLOCK).sum(axis=1, dtype=np.uint64)
+    if full < E:
+        sums = np.append(sums, host[full:].sum(dtype=np.uint64))
+    arrays = {
+        "index_len": np.array([E], dtype=np.float64),
+        "end_parity": np.array([idx.end_parity], dtype=np.float64),
+        "index_head": host[:edge].astype(np.float64),
+        "index_tail": host[max(E - edge, 0):].astype(np.float64),
+        "index_sample_pos": pos.astype(np.float64),
+        "index_sample": host[pos].astype(np.float64),
+        "index_block_sums": sums.astype(np.float64),
+    }
+    budget = DUMP_MAX_BYTES // world
+    assert sum(a.nbytes for a in arrays.values()) <= budget, f"dump of rank {rank} exceeds its {budget} bytes"
+    os.makedirs(out_dir, exist_ok=True)
+    written = 0
+    for name, a in arrays.items():
+        path = os.path.join(out_dir, name + (f"_rank{rank}" if world > 1 else "") + ".npy")
+        np.save(path, a)
+        written += os.path.getsize(path)
+    return written
+
+
 def pcie_probe(torch, dev, mb: int = 256, reps: int = 3):
     """Pinned H2D and D2H running at the same time (what bounds the end-to-end path): GB/s per direction."""
     n = mb << 20
@@ -322,9 +371,10 @@ def run_ours(args, rank: int, local_rank: int, world: int):
         sampler.start()
 
     # -----------------------------------------------------------------------------------------
-    def measure(wl_name, data, sharded, steps, e2e_steps_cap=10, check=True, ex_=None):
+    def measure(wl_name, data, sharded, steps, e2e_steps_cap=10, check=True, ex_=None, dump_dir=None):
         """One workload on this rank's bytes: device-resident steps (value), per-launch kernel time (roofline),
-        end-to-end host->host steps (e2e), and -- sharded -- element-wise parity against the oracle."""
+        end-to-end host->host steps (e2e), and -- sharded -- element-wise parity against the oracle.  With dump_dir,
+        the index of the last timed step is written there (dump_index) once the timing is over."""
         n = int(data.size)
         sizes = [int(v) for v in gather_obj(n)] if sharded else [n]
         goff = sum(sizes[:rank]) if sharded else 0
@@ -378,7 +428,8 @@ def run_ours(args, rank: int, local_rank: int, world: int):
         e0.record(stream)
         for i in range(steps):
             idx = step_device(resolve=False)
-            idx.free()
+            if dump_dir is None or i + 1 < steps:
+                idx.free()
             if i < 64:   # per-step marks (diagnostic: a stall of one step shows up as max >> median)
                 ev = torch.cuda.Event(enable_timing=True)
                 ev.record(stream)
@@ -396,6 +447,11 @@ def run_ours(args, rank: int, local_rank: int, world: int):
         launches, E_total = all_sum_int(launches, E)
         res.update(ms_per_step=ms_total / steps, launches=launches, E_total=E_total)
         res["value"] = total_bytes / (res["ms_per_step"] * 1e-3) / 1e9
+        if dump_dir is not None:
+            written = dump_index(idx, dump_dir, rank, world)
+            idx.free()
+            written = all_sum_int(written)[0]   # every rank's files: the directory as a whole stays within the budget
+            assert written <= DUMP_MAX_BYTES, f"--dump-outputs wrote {written} bytes, more than {DUMP_MAX_BYTES}"
 
         # ---- roofline of the dominant kernel: per-launch duration from events around each launch ----
         kms = []
@@ -468,7 +524,7 @@ def run_ours(args, rank: int, local_rank: int, world: int):
     # ---- the headline workload -------------------------------------------------------------------------
     data, desc = make_workload(wl, rank, world, size)
     sharded = world > 1 and wl == "cfg4_sharded"
-    m = measure(wl, data, sharded, args.steps, ex_=ex)
+    m = measure(wl, data, sharded, args.steps, ex_=ex, dump_dir=args.dump_outputs)
     n, E_local = m["n"], m["E_local"]
 
     # the same call on ordinary (pageable) memory, as a caller holding an mmap and a Vec would make it: informational
@@ -688,13 +744,18 @@ def main():
     ap.add_argument("--exchange", default="p2p", choices=["p2p", "nccl"],
                     help="N>1: cross-shard exchange over peer-mapped mailboxes (default) or the round-1 NCCL all_gather")
     ap.add_argument("--no-ab", action="store_true", help="N>1: skip the A/B run of the round-1 exchange")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the index of the last timed step to DIR/<name>.npy (float64; sampled, see dump_index) "
+                         "so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs writes what the CUDA path computed: it needs --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
-        if args.steps > 20:
-            args.steps = 20  # 1 GiB per step at ~1 GB/s: keep the arm within a couple of minutes
         run_reference(args, rank, world)
         return
     if world != args.gpus and world == 1 and args.gpus > 1:

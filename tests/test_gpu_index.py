@@ -1484,3 +1484,36 @@ def test_materialize_columns_one_sweep_vs_oracle(ctx, flags):
         offs, out = idx.materialize_column(f, 0, rc - 1, flags)
         assert (got[f][0] == offs).all() and got[f][1].tobytes() == out.tobytes()
     idx.free()
+
+
+def test_bench_dump_outputs_vs_oracle():
+    """bench.py --dump-outputs: the index of the last timed step, as float64 .npy files within 64 MB, equal to the
+    oracle's index of the same seeded bytes (length, end parity, both ends, the seeded sample, every block sum)."""
+    import json
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    size = 8 << 20
+    with tempfile.TemporaryDirectory() as d:
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", "7", "--warmup", "1",
+                              "--size", str(size), "--no-also", "--no-cpu-baseline", "--dump-outputs", d],
+                             capture_output=True, text=True, timeout=600)
+        assert out.returncode == 0, out.stderr[-2000:]
+        lines = [ln for ln in out.stdout.splitlines() if ln.strip()]
+        assert len(lines) == 1 and json.loads(lines[0])["steps"] == 7
+        files = sorted(os.listdir(d))
+        assert sum(os.path.getsize(os.path.join(d, f)) for f in files) <= 64 << 20
+        got = {f[:-4]: np.load(os.path.join(d, f)) for f in files}
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    data, _ = gen.unquoted(size, seed=42)
+    want, par = O.read_closed_form(data)
+    pos = got["index_sample_pos"].astype(np.int64)
+    assert got["index_len"].tolist() == [want.size] and got["end_parity"].tolist() == [par]
+    assert (got["index_head"] == want[:got["index_head"].size]).all()
+    assert (got["index_tail"] == want[want.size - got["index_tail"].size:]).all()
+    assert pos.size > 0 and (got["index_sample"] == want[pos]).all()
+    sums = got["index_block_sums"].astype(np.uint64)
+    block = 1 << 16
+    assert sums.size == -(-want.size // block)
+    for k in range(sums.size):
+        assert int(sums[k]) == int(want[k * block:(k + 1) * block].sum(dtype=np.uint64)), k

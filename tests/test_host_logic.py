@@ -175,7 +175,7 @@ def test_bench_reference_arm_contract():
     import json
     import subprocess
     env = dict(os.environ, RANK="0", LOCAL_RANK="0", WORLD_SIZE="1")
-    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2",
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "25",
                           "--warmup", "1", "--size", str(8 << 20)], capture_output=True, text=True, env=env, timeout=300)
     assert out.returncode == 0, out.stderr[-2000:]
     lines = [ln for ln in out.stdout.splitlines() if ln.strip()]
@@ -185,6 +185,7 @@ def test_bench_reference_arm_contract():
               "vs_baseline", "dtype", "data", "config", "cpu_baseline", "e2e"):
         assert k in d, k
     assert d["impl"] == "reference" and d["metric"] == "csv_bytes_indexed_per_sec" and d["unit"] == "GB/s"
+    assert d["steps"] == 25   # --steps is the number of timed steps, whatever it is
     assert d["value"] > 0 and d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] == 1
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0 and d["config"]["workload"]
     env["RANK"] = "1"
@@ -192,6 +193,36 @@ def test_bench_reference_arm_contract():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1",
                           "--warmup", "0", "--size", str(1 << 20)], capture_output=True, text=True, env=env, timeout=300)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+def test_bench_dump_stays_within_budget_for_every_world_size(tmp_path):
+    """bench.py --dump-outputs: every rank writes its own segment, and all ranks' files together stay within 64 MB
+    (each rank takes 1/world of the sample and the edges); the values are the index's own."""
+    import bench
+
+    class FakeIndex:
+        end_parity = 1
+
+        def __init__(self, k):
+            self.host = np.arange(3_000_000, dtype=np.uint64) * np.uint64(7) + np.uint64(k)
+
+        def to_host(self):
+            return self.host
+
+    for world in (1, 2, 8):
+        d = tmp_path / f"w{world}"
+        written = sum(bench.dump_index(FakeIndex(k), str(d), k, world) for k in range(world))
+        files = sorted(os.listdir(d))
+        assert written == sum(os.path.getsize(d / f) for f in files) <= bench.DUMP_MAX_BYTES, world
+        assert len(files) == 7 * world and all(f.endswith(".npy") for f in files)
+        for k in range(world):
+            sfx = f"_rank{k}" if world > 1 else ""
+            host = FakeIndex(k).host
+            pos = np.load(d / f"index_sample_pos{sfx}.npy").astype(np.int64)
+            assert np.load(d / f"index_len{sfx}.npy").tolist() == [host.size]
+            assert pos.size > 0 and (np.load(d / f"index_sample{sfx}.npy") == host[pos]).all()
+            sums = np.load(d / f"index_block_sums{sfx}.npy")
+            assert sums.dtype == np.float64 and int(sums.astype(np.uint64).sum(dtype=np.uint64)) == int(host.sum(dtype=np.uint64))
 
 
 def test_numa_helpers():

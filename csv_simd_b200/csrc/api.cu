@@ -92,7 +92,8 @@ int ensure_scratch(csvb200_ctx* ctx, size_t bytes)
     return CSVB200_OK;
 }
 
-int next_build_scratch(csvb200_ctx* ctx, size_t bytes, cudaStream_t stream, uint32_t* tag_out, bool reuse_tag)
+// build scratch of at least `bytes` + a fresh descriptor tag for one launch on `stream`
+static int next_build_scratch(csvb200_ctx* ctx, size_t bytes, cudaStream_t stream, uint32_t* tag_out, bool reuse_tag)
 {
     if (bytes > ctx->bscratch_bytes) {
         size_t nb = std::max(bytes, ctx->bscratch_bytes * 2);
@@ -113,6 +114,51 @@ int next_build_scratch(csvb200_ctx* ctx, size_t bytes, cudaStream_t stream, uint
         ctx->desc_tag += 1;
     }
     *tag_out = ctx->desc_tag;
+    return CSVB200_OK;
+}
+
+// kernel choice: the TMA pipeline for anything of size, the one-tile-per-CTA kernel for small inputs;
+// CSVB200_KERNEL=simple|tma forces one (tests cross-check the two against each other)
+static bool build_uses_tma(const csvb200_ctx* ctx, uint64_t n, bool allow_tma)
+{
+    if (!allow_tma || ctx->kernel_override == 1) return false;
+    if (ctx->kernel_override == 2 && n >= 128) return true;
+    return tma_path_usable(n);
+}
+
+int launch_build(csvb200_ctx* ctx, BuildParams& p, size_t cell, cudaStream_t stream, bool allow_tma)
+{
+    // an empty input still runs one (empty) tile: its carry / result live on the device
+    const uint64_t num_tiles = std::max<uint64_t>(1, (p.n + kTileBytes - 1) / kTileBytes);
+    if (num_tiles > 0xffffffffull) return fail(ctx, CSVB200_ERR_INVALID_ARG, "input too large for one launch");
+    // DEBUG (CSVB200_TUNE bit 0x400, timing experiments only): reuse the TAG of the previous build of the same
+    // address and size, so every look-back finds a published prefix on its first poll -- the kernel without its chain.
+    // The result is exact only when the bytes there are unchanged.
+    const bool keep_desc = (ctx->tune & 0x400u) && ctx->dbg_desc_src == p.in && ctx->dbg_desc_n == p.n;
+    int rc = next_build_scratch(ctx, 128 + num_tiles * kDescStride * sizeof(uint64_t), stream, &p.desc_tag, keep_desc);
+    if (rc) return rc;
+    ctx->dbg_desc_src = p.in;
+    ctx->dbg_desc_n = p.n;
+    // the scratch may have moved just now, so its pointers are handed out here.  Head: [0] ticket, [4] CTAs whose
+    // look-back role is over, [8] separator total of the exchange, [16] newlines, [24] non-ASCII flag; all zero at
+    // launch, put back to zero by the last CTA that uses them
+    uint8_t* head = ctx->d_bscratch;
+    p.num_tiles = (uint32_t)num_tiles;
+    p.ticket = reinterpret_cast<uint32_t*>(head);
+    p.desc = reinterpret_cast<uint64_t*>(head + 128);
+    if (p.validate || p.ex.peers) {
+        p.ex_done = reinterpret_cast<uint32_t*>(head + 4);
+        p.scratch_totals = 1u;
+    }
+    if (p.ex.peers) p.total_out = reinterpret_cast<unsigned long long*>(head + 8);
+    if (p.validate) {
+        p.nl_out = reinterpret_cast<unsigned long long*>(head + 16);
+        p.hi_out = reinterpret_cast<uint32_t*>(head + 24);
+    }
+    p.result = ctx->d_cells + cell * kCellWords;
+    p.result_host = ctx->h_cells + cell * kCellWords;
+    CU_TRY(ctx, build_uses_tma(ctx, p.n, allow_tma) ? launch_index_build_tma(p, stream) : launch_index_build(p, stream));
+    ctx->launches += 1;
     return CSVB200_OK;
 }
 
@@ -161,55 +207,31 @@ int enqueue_build(csvb200_index* idx, bool timed, bool redo = false)
 {
     csvb200_ctx* ctx = idx->ctx;
     const size_t n = idx->n;
-    uint64_t num_tiles = (n + kTileBytes - 1) / kTileBytes;
+    const uint64_t num_tiles = (n + kTileBytes - 1) / kTileBytes;
     // an empty shard still runs one (empty) tile when its carry / result live on the device
-    if (num_tiles == 0 && (idx->d_shard_par || idx->d_result2 || idx->speculative)) num_tiles = 1;
-    if (num_tiles > 0xffffffffull) return fail(ctx, CSVB200_ERR_INVALID_ARG, "input too large for one launch");
-    uint64_t* d_cell = ctx->d_cells + idx->cell * kCellWords;
-    uint64_t* h_cell = ctx->h_cells + idx->cell * kCellWords;
-    if (num_tiles == 0) {
+    if (num_tiles == 0 && !(idx->d_shard_par || idx->d_result2 || idx->speculative)) {
         if (idx->out_base == 1 && idx->cap > 0) CU_TRY(ctx, cudaMemsetAsync(idx->d_index, 0, 8, ctx->stream));  // sentinel alone
+        uint64_t* h_cell = ctx->h_cells + idx->cell * kCellWords;
         h_cell[0] = 0;
         h_cell[1] = idx->carry_parity;
     } else {
-        const size_t sbytes = 128 + num_tiles * kDescStride * sizeof(uint64_t);
-        // DEBUG (CSVB200_TUNE bit 0x400, timing experiments only): reuse the TAG of the previous build of the same
-        // bytes, so every look-back finds a published prefix on its first poll -- the kernel without its chain
-        const bool keep_desc = (ctx->tune & 0x400u) && ctx->dbg_desc_src == idx->src && ctx->dbg_desc_n == n;
-        uint32_t tag = 0;
-        int rc = next_build_scratch(ctx, sbytes, ctx->stream, &tag, keep_desc);
-        if (rc) return rc;
-        ctx->dbg_desc_src = idx->src;
-        ctx->dbg_desc_n = n;
         BuildParams p{};
-        p.desc_tag = tag;
         p.in = idx->src;
         p.n = n;
         p.index = idx->d_index;
         p.cap = idx->cap;
         p.out_base = idx->out_base;
         p.pos_bias = idx->pos_bias;
-        p.carry = nullptr;
-        p.carry_count = 0;
         p.carry_parity = idx->carry_parity;
-        p.num_tiles = (uint32_t)num_tiles;
-        p.ticket = reinterpret_cast<uint32_t*>(ctx->d_bscratch);
-        p.desc = reinterpret_cast<uint64_t*>(ctx->d_bscratch + 128);
-        p.result = d_cell;
-        p.result_host = ctx->host_result ? h_cell : nullptr;
         p.write_sentinel = idx->out_base == 1 ? 1u : 0u;
         p.result2 = idx->d_result2;
         p.result2_words = 2;
         p.shard_par = idx->d_shard_par;
         p.shard_rank = idx->shard_rank;
-        p.tune = ctx->tune;
-        static const bool dbg_timeline = std::getenv("CSVB200_DBG_TIMELINE") != nullptr;
-        if (dbg_timeline && !redo && !idx->validate && !idx->ex) {   // debug: per-super-tile timestamps of this build
-            const size_t words = 8 * ((n + kTileBytes - 1) / kTileBytes + 1);
+        if (ctx->dbg_timeline && !redo && !idx->validate && !idx->ex) {   // debug: per-super-tile timestamps of this build
+            const size_t words = 8 * (num_tiles + 1);
             if (ctx->dbg_words < words) {
                 if (ctx->d_dbg) cudaFree(ctx->d_dbg);
-    if (ctx->h_small_in) cudaFreeHost(ctx->h_small_in);
-    if (ctx->h_small_out) cudaFreeHost(ctx->h_small_out);
                 ctx->d_dbg = nullptr;
                 ctx->dbg_words = 0;
                 if (cudaMalloc((void**)&ctx->d_dbg, words * sizeof(uint64_t)) == cudaSuccess) ctx->dbg_words = words;
@@ -219,24 +241,16 @@ int enqueue_build(csvb200_index* idx, bool timed, bool redo = false)
                 p.dbg = ctx->d_dbg;
             }
         }
-        // kernel choice: the TMA pipeline for anything of size, the one-tile-per-CTA kernel for small
-        // inputs; CSVB200_KERNEL=simple|tma forces one (tests cross-check the two against each other)
-        bool use_tma = tma_path_usable(n);
-        if (ctx->kernel_override == 1) use_tma = false;
-        if (ctx->kernel_override == 2 && n >= 128) use_tma = true;
+        const bool use_tma = build_uses_tma(ctx, n, true);
         if (idx->validate) {
             // by-products: newline count and non-ASCII flag accumulate in the zeroed head of the scratch, the per-tile
             // non-ASCII bitmap belongs to the index (K7 later visits the flagged tiles only)
             const size_t words = (size_t)(num_tiles + 31) / 32;
             if (!idx->d_nonascii) CU_TRY(ctx, pool_malloc((void**)&idx->d_nonascii, words * sizeof(uint32_t), ctx->stream));
             CU_TRY(ctx, cudaMemsetAsync(idx->d_nonascii, 0, words * sizeof(uint32_t), ctx->stream));
-            idx->flag_tile_bytes = build_flag_tile_bytes(n, use_tma, ctx->tune);
+            idx->flag_tile_bytes = build_flag_tile_bytes(use_tma);
             p.validate = 1u;
             p.nonascii_bitmap = idx->d_nonascii;
-            p.nl_out = reinterpret_cast<unsigned long long*>(ctx->d_bscratch + 16);
-            p.hi_out = reinterpret_cast<uint32_t*>(ctx->d_bscratch + 24);
-            p.ex_done = reinterpret_cast<uint32_t*>(ctx->d_bscratch + 4);
-            p.scratch_totals = 1u;
         }
         if (idx->speculative) {
             uint64_t* d_carry = ctx->d_cells + idx->carry_cell * kCellWords;
@@ -247,9 +261,6 @@ int enqueue_build(csvb200_index* idx, bool timed, bool redo = false)
             } else if (idx->ex) {
                 // exchange inside the launch: separator total and the "look-back role over" counter live in the
                 // zeroed head of the scratch; the last CTA posts the row and resolves the carry chain into d_carry
-                p.total_out = reinterpret_cast<unsigned long long*>(ctx->d_bscratch + 8);
-                p.ex_done = reinterpret_cast<uint32_t*>(ctx->d_bscratch + 4);
-                p.scratch_totals = 1u;
                 p.ex.peers = idx->ex->d_peers;
                 p.ex.rank = idx->ex->rank;
                 p.ex.world = idx->ex->world;
@@ -265,8 +276,8 @@ int enqueue_build(csvb200_index* idx, bool timed, bool redo = false)
         }
         // the conditional re-index of the exchange form sits right behind the build: launched programmatically
         // dependent, its CTAs are scheduled as the build's CTAs leave, wait for the build's completion inside the kernel and
-        // exit on the flag -- the launch latency hides behind the build's tail (CSVB200_TUNE bit 0x800: plain stream order)
-        if (redo && idx->ex && use_tma && ctx->host_result && !(ctx->tune & 0x800u)) p.pdl_wait = 2u;
+        // exit on the flag -- the launch latency hides behind the build's tail
+        if (redo && idx->ex && use_tma) p.pdl_wait = 2u;
         if (timed) CU_TRY(ctx, cudaEventRecord(ctx->ev_k0, ctx->stream));
         if (idx->speculative && !redo && !idx->verified) {
             // predicted carry-in parity (rank 0 and empty shards: known to be 0) into the device cell the launch reads;
@@ -277,20 +288,15 @@ int enqueue_build(csvb200_index* idx, bool timed, bool redo = false)
             } else {
                 CU_TRY(ctx, launch_predict_carry(idx->src, n, idx->predict_window, d_carry, ctx->stream));
                 ctx->launches += 1;
-                p.pdl_wait = (use_tma && !(ctx->tune & 0x800u)) ? 1u : 0u;   // CSVB200_TUNE bit 0x800: plain stream order (A/B)
+                p.pdl_wait = use_tma ? 1u : 0u;
             }
         }
-        if (use_tma)
-            CU_TRY(ctx, launch_index_build_tma(p, ctx->stream));
-        else
-            CU_TRY(ctx, launch_index_build(p, ctx->stream));
-        ctx->launches += 1;
+        const int rc = launch_build(ctx, p, idx->cell, ctx->stream);
+        if (rc) return rc;
         if (timed) {
             CU_TRY(ctx, cudaEventRecord(ctx->ev_k1, ctx->stream));
             ctx->timed = true;
         }
-        if (!ctx->host_result)
-            CU_TRY(ctx, cudaMemcpyAsync(h_cell, d_cell, kCellWords * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
     }
     CU_TRY(ctx, cudaEventRecord(idx->done, ctx->stream));
     idx->synced = false;
@@ -500,12 +506,7 @@ int csvb200_ctx_create(int device, csvb200_ctx** out)
         if (std::strcmp(k, "tma") == 0) ctx->kernel_override = 2;
     }
     if (const char* t = std::getenv("CSVB200_TUNE")) ctx->tune = (uint32_t)std::atoi(t);
-    if (const char* t = std::getenv("CSVB200_HOST_RESULT")) ctx->host_result = std::atoi(t) != 0;
-    if (const char* t = std::getenv("CSVB200_E2E_RAMP")) ctx->e2e_ramp = std::atoi(t) != 0;
-    if (const char* t = std::getenv("CSVB200_E2E_CHUNK_MB")) {
-        const long mb = std::atol(t);
-        if (mb >= 1 && mb <= 4096) ctx->e2e_chunk = (size_t)mb << 20;
-    }
+    ctx->dbg_timeline = std::getenv("CSVB200_DBG_TIMELINE") != nullptr;
     auto bail = [&](cudaError_t) {
         cudaGetLastError();
         csvb200_ctx_destroy(ctx);
@@ -546,6 +547,8 @@ void csvb200_ctx_destroy(csvb200_ctx* ctx)
     delete ctx->pool;
     delete ctx->pool_down;
     if (ctx->d_dbg) cudaFree(ctx->d_dbg);
+    if (ctx->h_small_in) cudaFreeHost(ctx->h_small_in);
+    if (ctx->h_small_out) cudaFreeHost(ctx->h_small_out);
     for (int i = 0; i < 2; ++i) {
         if (ctx->h_bounce[i]) cudaFreeHost(ctx->h_bounce[i]);
         if (ctx->bounce_done[i]) cudaEventDestroy(ctx->bounce_done[i]);
@@ -831,7 +834,7 @@ static int build_to_host_serial(csvb200_ctx* ctx, const uint8_t* host_bytes, siz
 // around a ~5 us kernel cost 46-63 us, while the reference's loop indexes 64 KiB in 10 us.  Here the kernel reads the
 // bytes straight out of pinned host memory and writes the entries straight into pinned host memory (zero-copy over
 // PCIe; both buffers are the context's own and reused, or the caller's destination when that is pinned): one launch, one
-// synchronisation, no device allocation.  CSVB200_SMALL_DIRECT=0 takes the general path (A/B, tests).
+// synchronisation, no device allocation.
 constexpr size_t kSmallDirectBytes = 256u << 10;
 static int build_to_host_small(csvb200_ctx* ctx, const uint8_t* host_bytes, size_t n, uint64_t* dst, size_t dst_cap,
                                size_t* len_out)
@@ -852,38 +855,24 @@ static int build_to_host_small(csvb200_ctx* ctx, const uint8_t* host_bytes, size
     const size_t cap = direct ? dst_cap : kSmallDirectBytes + 2;
     CellLease lease(ctx, 1);
     if (!lease.ok()) return fail(ctx, CSVB200_ERR_OOM, "no free result cell (4095 live index objects)");
-    uint64_t* d_cell = ctx->d_cells + lease.first * kCellWords;
-    uint64_t* h_cell = ctx->h_cells + lease.first * kCellWords;
-    const uint64_t num_tiles = (n + kTileBytes - 1) / kTileBytes;
-    uint32_t tag = 0;
-    int rc = next_build_scratch(ctx, 128 + num_tiles * kDescStride * sizeof(uint64_t), ctx->stream, &tag);
-    if (rc) return rc;
     BuildParams p{};
-    p.desc_tag = tag;
     p.in = ctx->h_small_in;       // unified addressing: pinned host memory is addressable from the device as it is
     p.n = n;
     p.index = out;
     p.cap = cap;
     p.out_base = 1;
     p.write_sentinel = 1u;
-    p.num_tiles = (uint32_t)num_tiles;
-    p.ticket = reinterpret_cast<uint32_t*>(ctx->d_bscratch);
-    p.desc = reinterpret_cast<uint64_t*>(ctx->d_bscratch + 128);
-    p.result = d_cell;
-    p.result_host = h_cell;
-    p.result2_words = 2;
-    p.tune = ctx->tune;
-    CU_TRY(ctx, launch_index_build(p, ctx->stream));
-    ctx->launches += 1;
+    int rc = launch_build(ctx, p, lease.first, ctx->stream, false);
+    if (rc) return rc;
     CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    const size_t len = 1 + (size_t)h_cell[0];
+    const size_t len = 1 + (size_t)ctx->h_cells[lease.first * kCellWords];
     *len_out = len;
     if (len > dst_cap) return fail(ctx, CSVB200_ERR_CAPACITY, "destination index buffer too small");
     if (!direct) std::memcpy(dst, ctx->h_small_out, len * sizeof(uint64_t));
     return CSVB200_OK;
 }
 
-// End-to-end pipeline: the input goes up in e2e_chunk pieces, each piece is indexed by its own launch
+// End-to-end pipeline: the input goes up in kE2eChunk pieces, each piece is indexed by its own launch
 // chained to the previous one through a device-resident carry cell {entries so far, quote parity}
 // (no host round trip between launches), and every finished index segment goes down on a second
 // stream while later pieces are still going up -- PCIe is full duplex, so the step costs about
@@ -909,13 +898,12 @@ int pipeline_to_host(csvb200_ctx* ctx, const uint8_t* host_bytes, size_t n, uint
     // (measured: 27.16 vs 27.28 ms per GiB of cfg2 -- the step is bound by the D2H volume, the fill is ~1 ms of it)
     std::vector<size_t> chunk_off;
     {
-        const size_t full = ctx->e2e_chunk;
-        size_t off = 0, len = ctx->e2e_ramp ? std::max<size_t>(full / 8, 1u << 20) : full;
-        len = (len + 127) & ~size_t(127);   // chunk boundaries stay 128-byte aligned (TMA rows)
+        static_assert(kE2eChunk / 8 % 128 == 0, "chunk boundaries stay 128-byte aligned (TMA rows)");
+        size_t off = 0, len = kE2eChunk / 8;
         while (off < n) {
             chunk_off.push_back(off);
             off += std::min(len, n - off);
-            len = std::min(full, len * 2);
+            len = std::min(kE2eChunk, len * 2);
         }
         if (chunk_off.empty()) chunk_off.push_back(0);   // an empty shard still runs one empty launch
         chunk_off.push_back(n);
@@ -972,37 +960,21 @@ int pipeline_to_host(csvb200_ctx* ctx, const uint8_t* host_bytes, size_t n, uint
             e = launch_predict_carry(d_bytes, len, kDefaultPredictWindow, d_cells, s_up);   // cell0 <- {0, guess, found, 0}
             ctx->launches += 1;
         }
-        const uint64_t num_tiles = std::max<uint64_t>(1, (len + kTileBytes - 1) / kTileBytes);   // an empty shard runs one empty tile
-        const size_t sbytes = 128 + num_tiles * kDescStride * sizeof(uint64_t);
-        uint32_t tag = 0;
-        rc = next_build_scratch(ctx, sbytes, s_up, &tag);
-        if (rc) break;
         BuildParams p{};
-        p.desc_tag = tag;
         p.in = d_bytes + off;
-        p.n = len;
+        p.n = len;                         // an empty shard runs one empty tile
         p.index = d_index;
         p.cap = cap;
         p.out_base = out_base;
         p.pos_bias = o.pos_bias + off;
         p.carry = d_cells + c * kCellWords;
-        p.num_tiles = (uint32_t)num_tiles;
-        p.ticket = reinterpret_cast<uint32_t*>(ctx->d_bscratch);
-        p.desc = reinterpret_cast<uint64_t*>(ctx->d_bscratch + 128);
-        p.result = d_cells + (c + 1) * kCellWords;
-        p.result_host = ctx->host_result ? h_cells + (c + 1) * kCellWords : nullptr;
         p.write_sentinel = (c == 0 && out_base) ? 1u : 0u;
-        p.result2_words = 2;
         if (o.d_result4) p.total_out = reinterpret_cast<unsigned long long*>(o.d_result4 + 3);
-        p.tune = ctx->tune;
-        bool use_tma = tma_path_usable(len);
-        if (ctx->kernel_override == 1) use_tma = false;
-        if (e == cudaSuccess) e = use_tma ? launch_index_build_tma(p, s_up) : launch_index_build(p, s_up);
-        ctx->launches += 1;
-        if (e == cudaSuccess && !ctx->host_result)
-            e = cudaMemcpyAsync(h_cells + (c + 1) * kCellWords, d_cells + (c + 1) * kCellWords, 2 * sizeof(uint64_t),
-                                cudaMemcpyDeviceToHost, s_up);
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&done[c], cudaEventDisableTiming);
+        if (e == cudaSuccess) {
+            rc = launch_build(ctx, p, cell0 + c + 1, s_up);
+            if (rc) break;
+            e = cudaEventCreateWithFlags(&done[c], cudaEventDisableTiming);
+        }
         if (e == cudaSuccess) e = cudaEventRecord(done[c], s_up);
         if (e != cudaSuccess) {
             cudaGetLastError();
@@ -1022,11 +994,7 @@ int pipeline_to_host(csvb200_ctx* ctx, const uint8_t* host_bytes, size_t n, uint
       }
       if (rc != CSVB200_OK) enqueue_failed.store(true, std::memory_order_release);
     };
-    static const bool upload_thread = [] {
-        const char* e = std::getenv("CSVB200_E2E_UPLOAD_THREAD");   // 0: enqueue everything first, on the calling thread (A/B)
-        return !(e && e[0] == '0');
-    }();
-    const bool two_threads = upload_thread && !o.d_bytes_in && n >= (64u << 20) && !is_pinned(host_bytes);
+    const bool two_threads = !o.d_bytes_in && n >= (64u << 20) && !is_pinned(host_bytes);
     std::thread uploader;
     bool spawned = false;
     if (two_threads) {
@@ -1123,12 +1091,9 @@ int csvb200_index_build_to_host(csvb200_ctx* ctx, const uint8_t* host_bytes, siz
                                 size_t* len_out)
 {
     if (!ctx || !len_out || (n && !host_bytes)) return fail(ctx, CSVB200_ERR_INVALID_ARG, "null argument");
-    static const bool small_direct = [] {
-        const char* e = std::getenv("CSVB200_SMALL_DIRECT");
-        return !(e && e[0] == '0');
-    }();
-    if (small_direct && n > 0 && n <= kSmallDirectBytes && dst && ctx->kernel_override != 2) return build_to_host_small(ctx, host_bytes, n, dst, dst_cap, len_out);
-    const size_t nchunks = (n + ctx->e2e_chunk - 1) / ctx->e2e_chunk;
+    // (CSVB200_KERNEL=tma sends small inputs to the general path: the zero-copy one runs the one-tile-per-CTA kernel only)
+    if (n > 0 && n <= kSmallDirectBytes && dst && ctx->kernel_override != 2) return build_to_host_small(ctx, host_bytes, n, dst, dst_cap, len_out);
+    const size_t nchunks = (n + kE2eChunk - 1) / kE2eChunk;
     if (nchunks < 2 || nchunks + 1 >= kRingCells || !dst) return build_to_host_serial(ctx, host_bytes, n, dst, dst_cap, len_out);
     bool overflow = false;
     int rc = pipeline_to_host(ctx, host_bytes, n, dst, dst_cap, len_out, PipeOpts{}, &overflow);

@@ -54,7 +54,8 @@ struct csvb200_ctx {
     csvb200::SlicePool* pool_down = nullptr;   // a second set for the download side of the pageable pipeline (io_pool_down)
     uint8_t* h_small_in = nullptr;             // pinned, device-mapped staging of the small-input fast path (build_to_host_small)
     uint64_t* h_small_out = nullptr;
-    uint64_t* d_dbg = nullptr;                 // CSVB200_DBG_TIMELINE: 8 words per super-tile of the last device-resident build
+    bool dbg_timeline = false;                 // CSVB200_DBG_TIMELINE: device-resident builds run the instrumented kernel
+    uint64_t* d_dbg = nullptr;                 // ... and leave 8 words per super-tile here
     size_t dbg_words = 0;
     int io_threads = 0;                        // slices per pool; 0 = default_io_threads() (csvb200_multi_create divides them over its devices)
     uint8_t* h_seek_stage = nullptr;   // pinned staging of the batched seeks from pageable arrays (kept across calls)
@@ -69,12 +70,9 @@ struct csvb200_ctx {
     bool reserve_explicit = false;    // csvb200_ctx_set_reserve was called: the ratio is the caller's, no hint
     uint64_t launches = 0;
     int kernel_override = 0;  // 0 = auto, 1 = simple, 2 = tma (CSVB200_KERNEL)
-    uint32_t tune = 0;        // CSVB200_TUNE experiment knob
-    const uint8_t* dbg_desc_src = nullptr;   // (debug) input the look-back descriptors in d_scratch belong to
+    uint32_t tune = 0;        // CSVB200_TUNE: bit 0x400 = the no-chain timing experiment (launch_build)
+    const uint8_t* dbg_desc_src = nullptr;   // (debug) input the look-back descriptors in d_bscratch belong to
     size_t dbg_desc_n = 0;
-    bool host_result = true;  // kernels write {entries, end parity} straight into the pinned cell (CSVB200_HOST_RESULT=0: D2H copy node)
-    bool e2e_ramp = true;     // host -> host pipeline starts with small chunks (CSVB200_E2E_RAMP=0: uniform chunks)
-    size_t e2e_chunk = csvb200::kE2eChunk;   // granularity of the host -> host pipeline (CSVB200_E2E_CHUNK_MB)
     std::string err;
 };
 
@@ -155,8 +153,11 @@ struct CellLease {
     bool ok() const { return first != SIZE_MAX; }
 };
 int ensure_scratch(csvb200_ctx* ctx, size_t bytes);
-// build scratch of at least `bytes` + a fresh descriptor tag for one launch on `stream`
-int next_build_scratch(csvb200_ctx* ctx, size_t bytes, cudaStream_t stream, uint32_t* tag_out, bool reuse_tag = false);
+// One launch of the index build on `stream`.  The caller fills the input, the output and its capacity, the carry, the
+// sentinel and the validate / exchange / speculative extras of p; this fills the rest (tile count, build scratch and
+// descriptor tag, the scratch-head counters of the extras, the result cell `cell`), picks the kernel and launches it.
+// allow_tma = false: the input is mapped host memory, which only the one-tile-per-CTA kernel reads.
+int launch_build(csvb200_ctx* ctx, BuildParams& p, size_t cell, cudaStream_t stream, bool allow_tma = true);
 bool is_pinned(const void* p);
 SlicePool& io_pool(csvb200_ctx* ctx);   // the context's host-thread pool (CSVB200_IO_THREADS)
 // host -> device copy of n bytes on the context's stream; pinned sources go straight to cudaMemcpyAsync,

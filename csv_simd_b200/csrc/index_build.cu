@@ -210,10 +210,7 @@ __global__ void __launch_bounds__(kThreads, 3) index_build_kernel(const BuildPar
 
         uint32_t pin;
         uint64_t base;
-        if (p.tune == 2)
-            decoupled_lookback<2>(p, tile, lane, pin, base);
-        else
-            decoupled_lookback<1>(p, tile, lane, pin, base);
+        decoupled_lookback<1>(p, tile, lane, pin, base);
         if (lane == 0) {
             const uint32_t pend = pin ^ par;
             const uint64_t cend = base + (pin ? o1 : o0);

@@ -258,17 +258,14 @@ __device__ __forceinline__ void decoupled_lookback(const BuildParams& p, uint32_
         const uint32_t ls_stop = __shfl_sync(0xffffffffu, stop, (int)(ls & 31u));
         if (ls < 32u && ls_stop == 1u) {   // an unpublished tile lies before the nearest prefix: poll again
             if (kDbg) ++dbg_polls;
-            if (!(p.tune & 1u)) {   // default since kv18 / kv20 (0.3-1.1 % on both 1 GiB inputs); CSVB200_TUNE bit 1: re-poll the window (A/B)
-                // wait on THAT descriptor alone (one line instead of the whole window per poll: hundreds of look-back
-                // warps poll at the same time and their traffic competes with the data streams in L2), then rescan
-                const int64_t widx = idx0 - (int64_t)ls * kLookbackPerLane - (kLookbackPerLane - 1);
-                if (lane == 0 && widx >= 0) {
-                    while ((ld_relaxed_u64(p.desc + widx * kDescStride) >> 62) == 0ull) __nanosleep(32);
-                }
-                __syncwarp();
-            } else {
-                __nanosleep(64);
+            // wait on THAT descriptor alone (one line instead of the whole window per poll: hundreds of look-back warps
+            // poll at the same time and their traffic competes with the data streams in L2), then rescan; re-polling
+            // the whole window measured 0.3-1.1 % slower on both 1 GiB inputs (kv18 / kv20)
+            const int64_t widx = idx0 - (int64_t)ls * kLookbackPerLane - (kLookbackPerLane - 1);
+            if (lane == 0 && widx >= 0) {
+                while ((ld_relaxed_u64(p.desc + widx * kDescStride) >> 62) == 0ull) __nanosleep(32);
             }
+            __syncwarp();
             continue;
         }
         // lanes 0..ls contribute (lane ls only the tiles nearer than its prefix)

@@ -86,7 +86,6 @@ struct BuildParams {
     // this shard is the XOR of shard_par[0 .. shard_rank) (overrides carry_parity when non-null)
     const uint32_t* shard_par;
     uint32_t shard_rank;
-    uint32_t tune;           // experiment knob (CSVB200_TUNE)
     uint64_t* dbg;           // debug timeline (CSVB200_DBG_TIMELINE): 8 words per super-tile, see tools/timeline.py; null normally
     // speculative multi-GPU build: when non-null the launch is a conditional redo and exits at once
     // unless *run_flag != 0 (the carry prediction turned out wrong)
@@ -188,7 +187,7 @@ cudaError_t launch_utf8_validate(const uint8_t* in, uint64_t n, uint64_t* result
 cudaError_t launch_utf8_validate_flagged(const uint8_t* in, uint64_t n, const uint32_t* bitmap, uint64_t tile_bytes,
                                          uint64_t* result, cudaStream_t stream);
 // bytes per bit of the non-ASCII bitmap for an input of n bytes (depends on the kernel the build picks)
-uint64_t build_flag_tile_bytes(uint64_t n, bool use_tma, uint32_t tune);
+uint64_t build_flag_tile_bytes(bool use_tma);
 
 // K6 column materialisation (materialize.cu)
 struct MaterializeParams {

@@ -40,7 +40,7 @@ struct Slot {
     uint64_t* h_out = nullptr;     // pinned, out_cap entries
     uint8_t* d_in = nullptr;
     uint64_t* d_seg = nullptr;     // chunk + 2 entries: the worst case (one entry per byte) + sentinel
-    cudaEvent_t k_done = nullptr;  // kernel + count read-back of the chunk in this slot
+    cudaEvent_t k_done = nullptr;  // kernel of the chunk in this slot (it writes its count to the pinned cell)
     cudaEvent_t d_done = nullptr;  // last D2H out of d_seg
     size_t bytes = 0;              // bytes of the chunk in flight
     uint64_t offset = 0;           // global byte offset of the chunk
@@ -115,7 +115,7 @@ struct Pipeline {
 
     size_t cell_of(uint32_t c) const { return cells0 + c % (kSlots + 1); }
 
-    // enqueue H2D + kernel + count read-back of the chunk sitting in slot s (s.bytes > 0)
+    // enqueue H2D + kernel of the chunk sitting in slot s (s.bytes > 0)
     int launch(Slot& s)
     {
         const uint32_t c = chunks;
@@ -125,12 +125,6 @@ struct Pipeline {
         cudaStream_t st = ctx->stream;
         CU_TRY(ctx, cudaStreamWaitEvent(st, s.d_done, 0));   // the previous segment in this slot has left d_seg
         CU_TRY(ctx, cudaMemcpyAsync(s.d_in, s.h_in, s.bytes, cudaMemcpyHostToDevice, st));
-        const bool use_tma = tma_path_usable(s.bytes) && ctx->kernel_override != 1;
-        const uint64_t num_tiles = (s.bytes + kTileBytes - 1) / kTileBytes;
-        const size_t sbytes = 128 + num_tiles * kDescStride * sizeof(uint64_t);
-        uint32_t tag = 0;
-        int rc = next_build_scratch(ctx, sbytes, st, &tag);
-        if (rc) return rc;
         BuildParams p{};
         p.in = s.d_in;
         p.n = s.bytes;
@@ -140,20 +134,9 @@ struct Pipeline {
         p.pos_bias = s.offset;
         p.carry = ctx->d_cells + prev_cell * kCellWords;
         p.carry_parity_only = 1;
-        p.num_tiles = (uint32_t)num_tiles;
-        p.desc_tag = tag;
-        p.ticket = reinterpret_cast<uint32_t*>(ctx->d_bscratch);
-        p.desc = reinterpret_cast<uint64_t*>(ctx->d_bscratch + 128);
-        p.result = ctx->d_cells + s.cell * kCellWords;
-        p.result_host = ctx->host_result ? ctx->h_cells + s.cell * kCellWords : nullptr;
         p.write_sentinel = c == 0 ? 1u : 0u;     // sentinel (src/reader.rs:216)
-        p.result2_words = 2;
-        p.tune = ctx->tune;
-        CU_TRY(ctx, use_tma ? launch_index_build_tma(p, st) : launch_index_build(p, st));
-        ctx->launches += 1;
-        if (!ctx->host_result)
-            CU_TRY(ctx, cudaMemcpyAsync(ctx->h_cells + s.cell * kCellWords, ctx->d_cells + s.cell * kCellWords,
-                                        2 * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+        const int rc = launch_build(ctx, p, s.cell, st);
+        if (rc) return rc;
         CU_TRY(ctx, cudaEventRecord(s.k_done, st));
         s.busy = true;
         total_bytes += s.bytes;

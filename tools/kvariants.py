@@ -1,6 +1,10 @@
-"""A/B of CSVB200_TUNE values (kernel shapes / experiment knobs) in ONE process on the same box and the same bytes.
+"""A/B of CSVB200_TUNE values in ONE process on the same box and the same bytes.
 
-    python tools/kvariants.py "0 256 512 768" [builds] [bytes] [workloads]
+    python tools/kvariants.py "0 1024" [builds] [bytes] [workloads]
+
+Round 2 ran every kernel shape and experiment knob through it (profiles/r02_kvariants.md, decoded by
+tools/kvariants_table.py); the losers are deleted, and the one value left is 1024 (bit 0x400): the no-chain timing
+experiment, where each build reuses the look-back descriptors of the build before it.
 
 For every workload (cfg2_unquoted, cfg3_quoted) and every tune value: a fresh context with CSVB200_TUNE set,
 3 warm-up builds, `builds` timed device-resident builds (CUDA events around each launch), and an element-wise

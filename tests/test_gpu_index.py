@@ -227,6 +227,19 @@ def test_batched_seeks_vs_oracle(ctx):
     for i in range(300):
         a, b = int(got[i, 0]), int(got[i, 1])
         assert blob[int(offs[i]):int(offs[i + 1])].tobytes() == raw[a:b]
+    # past the first sweep of the gather kernel (lookup.cu: SMs x 16 blocks of 32 ranges, ~75 K ranges on a B200),
+    # None probes scattered through every sweep: every byte against the oracle's slices
+    rec, fld = gen.queries(260_000, rc, 256, seed=47)
+    rec[::997] = rc - 1 + np.arange(rec[::997].size, dtype=np.uint32) % 3
+    fld[5::1009] = 256 + np.arange(fld[5::1009].size, dtype=np.uint32) % 5
+    offs, blob = idx.gather_fields(rec, fld)
+    live = (rec + 1 < rc) & (fld < 256)
+    s = np.where(live, (rec.astype(np.int64) + 1) * 256 + fld, 0)
+    a = np.where(live, want_idx[s] + 1, 0).astype(np.int64)
+    lens = np.where(live, want_idx[s + 1].astype(np.int64) - a, 0)
+    assert (~live).sum() > 400 and offs[0] == 0 and (np.diff(offs.astype(np.int64)) == lens).all()
+    src = np.repeat(a, lens) + np.arange(int(lens.sum())) - np.repeat(offs[:-1].astype(np.int64), lens)
+    assert blob.size == src.size and (blob == np.frombuffer(raw, dtype=np.uint8)[src]).all()
     idx.free()
 
 
@@ -859,6 +872,37 @@ def test_validate_utf8_vs_python_decoder(ctx):
     txt = "αβγ,δεζ\nκόσμε,🙂\n".encode()
     for pad in range(0, 40):
         assert ctx.validate_utf8(b"y" * pad + txt * 100)[0] is None
+    # past the first sweep of the grid-stride kernel (validate.cu: SMs x 8 blocks of 256 threads, each judging groups
+    # g and g + half of every sweep of 2 x half 32-byte groups; ~19 MB per sweep on a B200)
+    import torch
+    half = torch.cuda.get_device_properties(ctx.device).multi_processor_count * 8 * 256
+    sweep = 64 * half
+    n = max(64 << 20, 3 * sweep + sweep // 2)
+    base = np.resize(np.frombuffer(b"id,x\n1,ab\n", dtype=np.uint8), n)
+    smile = np.frombuffer("🙂".encode(), dtype=np.uint8)
+    e_acute = np.frombuffer("é".encode(), dtype=np.uint8)
+    t = 1000                                                      # one thread of the first block
+    inputs = []
+    v = base.copy()                                               # errors in the second and third sweeps only
+    v[100:102] = e_acute
+    v[sweep + 4321] = 0x80
+    v[2 * sweep + 77] = 0xC0
+    inputs.append(v)
+    v = base.copy()                                               # two errors one thread meets in iterations 1 and 2
+    v[32 * (t + 3 * half) + 5] = 0xFF
+    v[32 * (t + 4 * half) + 9] = 0x80
+    inputs.append(v)
+    v = base.copy()                                               # the reverse: only the later iteration's error
+    v[32 * (t + 4 * half) + 9] = 0x80
+    inputs.append(v)
+    v = base.copy()                                               # valid 4-byte sequences across sweep / group edges
+    for at in (half * 32 - 1, sweep - 2, 2 * sweep - 3, 3 * sweep - 1):
+        v[at:at + 4] = smile
+    inputs.append(v)
+    for v in inputs:
+        got, asc = ctx.validate_utf8(v)
+        assert got == O.utf8_valid_up_to(v.tobytes()) and asc == O.is_ascii(v)
+    assert got is None and asc is False
 
 
 def test_index_save_load_roundtrip(ctx):

@@ -1800,48 +1800,13 @@ static int materialize_prepare(csvb200_index* idx, uint32_t flags)
     return CSVB200_OK;
 }
 
-int csvb200_materialize_column_device(csvb200_index* idx, uint32_t field_idx, uint32_t first_record, uint32_t nrec,
-                                      uint32_t flags, uint64_t* d_offsets, uint8_t* d_out, size_t out_cap)
-{
-    int rc = materialize_prepare(idx, flags);
-    if (rc) return rc;
-    if (!d_offsets || (out_cap && !d_out)) return fail(idx->ctx, CSVB200_ERR_INVALID_ARG, "null argument");
-    return materialize_enqueue(idx, field_idx, first_record, nrec, flags, d_offsets, d_out, out_cap, true, d_out != nullptr);
-}
-
-int csvb200_materialize_column(csvb200_index* idx, uint32_t field_idx, uint32_t first_record, uint32_t nrec,
-                               uint32_t flags, uint64_t* out_offsets, uint8_t* out, size_t out_cap, size_t* out_len)
-{
-    int rc = materialize_prepare(idx, flags);
-    if (rc) return rc;
-    csvb200_ctx* ctx = idx->ctx;
-    if (!out_offsets || !out_len) return fail(ctx, CSVB200_ERR_INVALID_ARG, "null argument");
-    DevBuf d_off, d_out;
-    CU_TRY(ctx, d_off.alloc(((size_t)nrec + 1) * sizeof(uint64_t), ctx->stream));
-    rc = materialize_enqueue(idx, field_idx, first_record, nrec, flags, d_off.as<uint64_t>(), nullptr, 0, true, false);
-    if (rc) return rc;
-    CU_TRY(ctx, cudaMemcpyAsync(out_offsets, d_off.p, ((size_t)nrec + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
-    CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    const uint64_t total = out_offsets[nrec];
-    *out_len = (size_t)total;
-    if (total > out_cap) return fail(ctx, CSVB200_ERR_CAPACITY, "materialize destination too small");
-    if (total == 0) return CSVB200_OK;
-    if (!out) return fail(ctx, CSVB200_ERR_INVALID_ARG, "null argument");
-    CU_TRY(ctx, d_out.alloc(total, ctx->stream));
-    rc = materialize_enqueue(idx, field_idx, first_record, nrec, flags, d_off.as<uint64_t>(), d_out.as<uint8_t>(), total, false, true);
-    if (rc) return rc;
-    CU_TRY(ctx, cudaMemcpyAsync(out, d_out.p, total, cudaMemcpyDeviceToHost, ctx->stream));
-    CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    return CSVB200_OK;
-}
-
 // several columns, one sweep per pass (materialize.cu: a thread owns a row and walks its requested fields)
 static int materialize_multi_enqueue(csvb200_index* idx, const uint32_t* fields, uint32_t ncols, uint32_t first_record,
                                      uint32_t nrec, uint32_t flags, uint64_t* const* d_offsets, uint8_t* const* d_outs,
                                      const size_t* out_caps, bool offsets_pass, bool write_pass)
 {
     csvb200_ctx* ctx = idx->ctx;
-    if (ncols == 1 && !getenv("CSVB200_MAT_SWEEP"))   // one column: the single-column kernels (1024-record tiles) are the faster form
+    if (ncols == 1)   // one column: the single-column kernels (1024-record tiles) are the faster form
         return materialize_enqueue(idx, fields[0], first_record, nrec, flags, d_offsets[0], d_outs ? d_outs[0] : nullptr,
                                    out_caps ? out_caps[0] : 0, offsets_pass, write_pass);
     MaterializeMultiParams p{};
@@ -1857,12 +1822,7 @@ static int materialize_multi_enqueue(csvb200_index* idx, const uint32_t* fields,
     p.nrec = nrec;
     p.flags = flags;
     p.ncols = ncols;
-    bool distinct = true;   // the sweep unquotes in place in shared memory: a column listed twice takes the per-row kernels
-    for (uint32_t c = 0; c < ncols && distinct; ++c)
-        for (uint32_t k = 0; k < c; ++k)
-            if (fields[k] == fields[c]) distinct = false;
-    p.rows_per_tile = distinct ? materialize_sweep_plan(idx->n, idx->record_cnt, p.row_size, ncols, &p.cap_bytes) : 0u;
-    p.tiles = p.rows_per_tile ? (nrec + p.rows_per_tile - 1) / p.rows_per_tile : (nrec + 255) / 256;
+    p.tiles = (nrec + kMultiThreads - 1) / kMultiThreads;
     for (uint32_t c = 0; c < ncols; ++c) {
         p.field_idx[c] = fields[c];
         p.offsets[c] = d_offsets[c];
@@ -1870,7 +1830,7 @@ static int materialize_multi_enqueue(csvb200_index* idx, const uint32_t* fields,
         p.out_cap[c] = out_caps ? out_caps[c] : 0;
     }
     if (offsets_pass) {
-        const size_t sbytes = materialize_multi_scratch_bytes(nrec, ncols, p.rows_per_tile);
+        const size_t sbytes = materialize_multi_scratch_bytes(nrec, ncols);
         int rc = ensure_scratch(ctx, sbytes);
         if (rc) return rc;
         CU_TRY(ctx, cudaMemsetAsync(ctx->d_scratch, 0, sbytes, ctx->stream));
@@ -1878,17 +1838,8 @@ static int materialize_multi_enqueue(csvb200_index* idx, const uint32_t* fields,
         p.tile_desc = reinterpret_cast<uint64_t*>(ctx->d_scratch + 128);
         if (nrec == 0)
             for (uint32_t c = 0; c < ncols; ++c) CU_TRY(ctx, cudaMemsetAsync(d_offsets[c], 0, sizeof(uint64_t), ctx->stream));
-        if (!p.rows_per_tile) {
-            CU_TRY(ctx, launch_materialize_multi_offsets(p, ctx->stream));
-            if (nrec) ctx->launches += 1;
-        }
-    }
-    if (p.rows_per_tile) {   // row sweep: offsets and values in ONE pass when both are asked for
-        if (nrec) {
-            CU_TRY(ctx, launch_materialize_sweep(p, offsets_pass, write_pass, ctx->stream));
-            if (offsets_pass || write_pass) ctx->launches += 1;
-        }
-        return CSVB200_OK;
+        CU_TRY(ctx, launch_materialize_multi_offsets(p, ctx->stream));
+        if (nrec) ctx->launches += 1;
     }
     if (write_pass && nrec) {
         CU_TRY(ctx, launch_materialize_multi_write(p, ctx->stream));
@@ -1905,6 +1856,9 @@ int csvb200_materialize_columns_device(csvb200_index* idx, const uint32_t* field
     if (rc) return rc;
     if (!fields || !d_offsets || ncols == 0 || ncols > kMatMaxCols)
         return fail(idx->ctx, CSVB200_ERR_INVALID_ARG, "1 <= ncols <= 32 and non-null arrays");
+    for (uint32_t c = 0; c < ncols; ++c)
+        if (!d_offsets[c] || (out_caps && out_caps[c] && (!d_outs || !d_outs[c])))
+            return fail(idx->ctx, CSVB200_ERR_INVALID_ARG, "null argument");
     return materialize_multi_enqueue(idx, fields, ncols, first_record, nrec, flags, d_offsets, d_outs, out_caps, true,
                                      d_outs != nullptr);
 }
@@ -1954,6 +1908,19 @@ int csvb200_materialize_columns(csvb200_index* idx, const uint32_t* fields, uint
         if (out_lens[c]) CU_TRY(ctx, cudaMemcpyAsync(outs[c], p_out[c], out_lens[c], cudaMemcpyDeviceToHost, ctx->stream));
     CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     return CSVB200_OK;
+}
+
+int csvb200_materialize_column_device(csvb200_index* idx, uint32_t field_idx, uint32_t first_record, uint32_t nrec,
+                                      uint32_t flags, uint64_t* d_offsets, uint8_t* d_out, size_t out_cap)
+{
+    return csvb200_materialize_columns_device(idx, &field_idx, 1, first_record, nrec, flags, &d_offsets, d_out ? &d_out : nullptr,
+                                              &out_cap);
+}
+
+int csvb200_materialize_column(csvb200_index* idx, uint32_t field_idx, uint32_t first_record, uint32_t nrec,
+                               uint32_t flags, uint64_t* out_offsets, uint8_t* out, size_t out_cap, size_t* out_len)
+{
+    return csvb200_materialize_columns(idx, &field_idx, 1, first_record, nrec, flags, &out_offsets, &out, &out_cap, out_len);
 }
 
 int csvb200_validate_utf8_device(csvb200_ctx* ctx, const void* dev_bytes, size_t n, uint64_t* d_result)

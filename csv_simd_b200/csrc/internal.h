@@ -211,6 +211,7 @@ size_t materialize_scratch_bytes(uint32_t nrec);   // [128 B ticket cell][descri
 // (adjacent index slots, adjacent bytes: the sectors one column drags in serve its neighbours), so the input and the
 // index cross DRAM once per pass instead of once per column and pass.
 constexpr uint32_t kMatMaxCols = 32;
+constexpr int kMultiThreads = 256;   // threads per CTA of the multi-column kernels = records per tile
 struct MaterializeMultiParams {
     const uint64_t* index;
     uint64_t index_len;
@@ -228,12 +229,8 @@ struct MaterializeMultiParams {
     uint64_t* tile_desc;              // [ncols][tiles] look-back descriptors (zeroed)
     uint32_t* ticket;                 // zeroed
     uint32_t tiles;
-    uint32_t rows_per_tile;           // > 0: row sweep over tiles of this many records (32 / 64 / 128); 0: one thread per row
-    uint32_t cap_bytes;               // row sweep: input bytes staged per tile
 };
-uint32_t materialize_sweep_plan(uint64_t n, uint32_t record_cnt, uint32_t row_size, uint32_t ncols, uint32_t* cap_bytes);
-cudaError_t launch_materialize_sweep(const MaterializeMultiParams& p, bool offsets, bool write, cudaStream_t stream);
-size_t materialize_multi_scratch_bytes(uint32_t nrec, uint32_t ncols, uint32_t rows_per_tile);
+size_t materialize_multi_scratch_bytes(uint32_t nrec, uint32_t ncols);
 cudaError_t launch_materialize_multi_offsets(const MaterializeMultiParams& p, cudaStream_t stream);
 cudaError_t launch_materialize_multi_write(const MaterializeMultiParams& p, cudaStream_t stream);
 cudaError_t launch_materialize_offsets(const MaterializeParams& p, cudaStream_t stream);

@@ -11,9 +11,6 @@
 // (2) the write.  Both read two index entries per record and the field's bytes: HBM sector-bound.
 #include "internal.h"
 
-#include <cstdlib>
-#include <mutex>
-
 namespace csvb200 {
 
 namespace {
@@ -40,45 +37,25 @@ __device__ __forceinline__ void st_relaxed(uint64_t* p, uint64_t v)
     asm volatile("st.relaxed.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
 }
 
-// Decoupled look-back by a whole warp: publishes this tile's total, sums the totals of the tiles before it back to the
-// nearest published prefix, publishes prefix + total and returns the prefix (every lane).  Tiles are small, so tiles
-// start faster than one 32-descriptor hop (~0.7 us of L2 latency) could follow: with one window per hop the nearest
-// published prefix drifts away until every look-back walks all the tiles in flight.  Four windows (128 tiles) are
-// fetched at once per hop, the loads overlapped.  Tiles must be taken in ticket order.
-__device__ __forceinline__ uint64_t lookback_warp(uint64_t* desc, uint32_t tile, uint64_t total, uint32_t lane)
+// Decoupled look-back by one thread over the tile totals (status in the top two bits): publishes this tile's total,
+// sums the totals of the tiles before it back to the nearest published prefix, publishes prefix + total and returns the
+// prefix.  Tiles must be taken in ticket order.
+__device__ __forceinline__ uint64_t lookback(uint64_t* desc, uint32_t tile, uint64_t total)
 {
-    if (lane == 0) st_relaxed(desc + tile, kMatAgg | (total & kMatMask));
+    st_relaxed(desc + tile, kMatAgg | (total & kMatMask));
     uint64_t prefix = 0;
     for (int64_t t = (int64_t)tile - 1; t >= 0;) {
-        uint64_t d[4];
-#pragma unroll
-        for (int w = 0; w < 4; ++w) {
-            const int64_t mine = t - 32 * w - (int64_t)lane;
-            d[w] = mine >= 0 ? ld_relaxed(desc + mine) : kMatPrefix;          // before tile 0: prefix 0
+        const uint64_t d = ld_relaxed(desc + t);
+        const uint64_t st = d >> 62;
+        if (st == 0) {
+            __nanosleep(40);
+            continue;
         }
-        bool done = false, retry = false;
-#pragma unroll
-        for (int w = 0; w < 4; ++w) {
-            if (done || retry) break;
-            const uint32_t st = (uint32_t)(d[w] >> 62);
-            const uint32_t pref = __ballot_sync(0xffffffffu, st == 2u), wait = __ballot_sync(0xffffffffu, st == 0u);
-            const uint32_t upto = pref ? (uint32_t)__ffs((int)pref) - 1u : 31u;  // lanes 0 .. upto count
-            const uint32_t use = 0xffffffffu >> (31u - upto);
-            if (wait & use) {
-                retry = true;                                                 // resume from this window
-                break;
-            }
-            uint64_t v = (use >> lane & 1u) ? (d[w] & kMatMask) : 0ull;
-#pragma unroll
-            for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-            prefix += v;
-            t -= 32;
-            done = pref != 0u;
-        }
-        if (done) break;
-        if (retry) __nanosleep(40);
+        prefix += d & kMatMask;
+        if (st == 2) break;
+        --t;
     }
-    if (lane == 0) st_relaxed(desc + tile, kMatPrefix | ((prefix + total) & kMatMask));
+    st_relaxed(desc + tile, kMatPrefix | ((prefix + total) & kMatMask));
     return prefix;
 }
 
@@ -208,7 +185,24 @@ __device__ __forceinline__ uint64_t value_len(const FieldView& p, uint32_t r)
     return value_len_range(p, a, b);
 }
 
-constexpr int kMultiThreads = 256;
+// put(byte) for every byte of the value made of the raw slice [a, b); x is the caller's restrict-qualified copy of
+// p.bytes (without it every byte load has to wait for the previous byte store)
+template <class Put>
+__device__ __forceinline__ void emit_value(const FieldView& p, const uint8_t* __restrict__ x, uint64_t a, uint64_t b, Put put)
+{
+    if (!trim_and_test(p, a, b)) {
+        if (b - a < 16) {   // short raw values: a handful of byte loads beat 16 predicated steps per chunk
+            for (; a < b; ++a) put(x[a]);
+        } else {
+            scan_bytes(x, p.n, a, b, put);
+        }
+    } else {
+        Unquoter<Put> u{put};
+        scan_bytes(x, p.n, a, b, u);
+        u.finish();
+    }
+}
+
 constexpr int kColBatch = 4;
 constexpr uint32_t kColBatchMin = 8;   // columns from which the batched form pays
 
@@ -308,24 +302,7 @@ __global__ void __launch_bounds__(kMatThreads) materialize_offsets_kernel(const 
         if (w < (int)warp) wbase += s_warp[w];
         total += s_warp[w];
     }
-    // decoupled look-back over the tile totals (status in the top two bits)
-    if (tid == 0) {
-        st_relaxed(p.tile_desc + tile, kMatAgg | (total & kMatMask));
-        uint64_t prefix = 0;
-        for (int64_t t = (int64_t)tile - 1; t >= 0;) {
-            const uint64_t d = ld_relaxed(p.tile_desc + t);
-            const uint64_t st = d >> 62;
-            if (st == 0) {
-                __nanosleep(40);
-                continue;
-            }
-            prefix += d & kMatMask;
-            if (st == 2) break;
-            --t;
-        }
-        st_relaxed(p.tile_desc + tile, kMatPrefix | ((prefix + total) & kMatMask));
-        s_prefix = prefix;
-    }
+    if (tid == 0) s_prefix = lookback(p.tile_desc, tile, total);
     __syncthreads();
     uint64_t off = s_prefix + wbase + (inc - tsum);
 #pragma unroll
@@ -350,18 +327,7 @@ __global__ void __launch_bounds__(kMatThreads) materialize_write_kernel(const Ma
         uint64_t o = p.offsets[i];
         const uint64_t o_end = p.offsets[i + 1];
         if (o_end > p.out_cap) continue;   // host form checks the capacity first; device form clips whole values
-        auto put = [&](uint32_t c) { out[o++] = (uint8_t)c; };
-        if (!trim_and_test(fv, a, b)) {
-            if (b - a < 16) {   // short raw values: a handful of byte loads beat 16 predicated steps per chunk
-                for (; a < b; ++a) put(x[a]);
-            } else {
-                scan_bytes(x, p.n, a, b, put);
-            }
-        } else {
-            Unquoter<decltype(put)> u{put};
-            scan_bytes(x, p.n, a, b, u);
-            u.finish();
-        }
+        emit_value(fv, x, a, b, [&](uint32_t c) { out[o++] = (uint8_t)c; });
     }
 }
 
@@ -370,6 +336,8 @@ __global__ void __launch_bounds__(kMatThreads) materialize_write_kernel(const Ma
 // slots and bytes of neighbouring columns come out of the sectors the first column fetched.  Per column: a block scan
 // of the 256 lengths (warp w scans columns w, w + 8, ...), one decoupled look-back chain over the tile totals
 // (thread c looks back for column c), then the exclusive offsets go out coalesced.
+// A row sweep (tiles of 32-128 records staged through shared memory) was built, measured against these kernels and
+// removed: it won on quoted columns and lost on unquoted ones (DESIGN 4.8, profiles/r02_mat_sweep_ab.jsonl).
 using ColBatch = RangeBatch<kColBatch>;
 __device__ __forceinline__ void col_batch_load(const MaterializeMultiParams& p, uint32_t r, uint32_t c0, bool row_live, ColBatch& cb)
 {
@@ -444,27 +412,9 @@ __global__ void __launch_bounds__(kMultiThreads) materialize_multi_offsets_kerne
     }
     __syncthreads();
     // one chain per column, thread c walks column c's: all the chains of the tile advance together in one warp
-    // (a warp per chain with 128-descriptor hops, as the sweep below does, measured slower here: 0.404 against 0.362 ms
-    // for 8 columns, 0.697 against 0.513 ms for 16 -- with 256-row tiles the walks are short and the chains queue up)
-    if (tid < p.ncols) {
-        uint64_t* desc = p.tile_desc + (uint64_t)tid * p.tiles;
-        const uint64_t total = s_total[tid];
-        st_relaxed(desc + tile, kMatAgg | (total & kMatMask));
-        uint64_t prefix = 0;
-        for (int64_t t = (int64_t)tile - 1; t >= 0;) {
-            const uint64_t d = ld_relaxed(desc + t);
-            const uint64_t st = d >> 62;
-            if (st == 0) {
-                __nanosleep(40);
-                continue;
-            }
-            prefix += d & kMatMask;
-            if (st == 2) break;
-            --t;
-        }
-        st_relaxed(desc + tile, kMatPrefix | ((prefix + total) & kMatMask));
-        s_base[tid] = prefix;
-    }
+    // (a warp per chain with 128-descriptor hops measured slower here: 0.404 against 0.362 ms for 8 columns, 0.697
+    // against 0.513 ms for 16 -- with 256-row tiles the walks are short and the chains queue up)
+    if (tid < p.ncols) s_base[tid] = lookback(p.tile_desc + (uint64_t)tid * p.tiles, tile, s_total[tid]);
     __syncthreads();
     for (uint32_t c = 0; c < p.ncols; ++c) {
         const uint64_t off = s_base[c] + s_len[c * kMultiThreads + tid];
@@ -486,18 +436,7 @@ __global__ void __launch_bounds__(kMultiThreads) materialize_multi_write_kernel(
         if (!field_range(fv, p.first_record + (uint32_t)i, a, b)) continue;
         uint64_t o = p.offsets[c][i];
         if (p.offsets[c][i + 1] > p.out_cap[c]) continue;
-        auto put = [&](uint32_t ch) { out[o++] = (uint8_t)ch; };
-        if (!trim_and_test(fv, a, b)) {
-            if (b - a < 16) {
-                for (; a < b; ++a) put(x[a]);
-            } else {
-                scan_bytes(x, p.n, a, b, put);
-            }
-        } else {
-            Unquoter<decltype(put)> u{put};
-            scan_bytes(x, p.n, a, b, u);
-            u.finish();
-        }
+        emit_value(fv, x, a, b, [&](uint32_t ch) { out[o++] = (uint8_t)ch; });
     }
     for (uint32_t c0 = 0; kBatched && c0 < p.ncols; c0 += kColBatch) {
         ColBatch cb;
@@ -534,404 +473,17 @@ __global__ void __launch_bounds__(kMultiThreads) materialize_multi_write_kernel(
                 u.finish();
                 continue;
             }
-            const FieldView fv = view_of(p, c);
-            if (!trim_and_test(fv, a, b)) {
-                scan_bytes(x, p.n, a, b, put);
-            } else {
-                Unquoter<decltype(put)> u{put};
-                scan_bytes(x, p.n, a, b, u);
-                u.finish();
-            }
+            emit_value(view_of(p, c), x, a, b, put);   // padded: trim first
         }
     }
-}
-
-// ---- several columns, row sweep -------------------------------------------------------------------------------------
-// When the requested columns cover a fair share of every row, the cheapest way to fetch them is to stream the rows:
-// a tile is R consecutive records (R = 32, 64 or 128, chosen on the host from the average row length); its bytes are
-// ONE contiguous range of the input and its index slots one contiguous range of the index.  One kernel, three forms:
-// offsets only, write only (the host form's second call), or both in ONE pass over the input (the device form called
-// with its destinations: lengths, scan, look-back, offsets and values without reading anything twice).  The CTA
-//   A. loads the row's slots (a warp per row: whole 128-byte lines of the index) as offsets relative to the tile's
-//      first byte, and
-//   B. copies the tile's bytes into shared memory with 16-byte loads (every input sector is fetched once, coalesced);
-//   C. warp (g, c) owns records 32 g .. 32 g + 31 of column c, one value per lane: trim / quote test / "" collapse run
-//      on shared memory (a byte walk costs an LDS, not an L2 round trip; quoted values are compacted in place), then
-//      a warp scan of the lengths gives the value's offset inside the tile;
-//   D. (offsets) one decoupled look-back chain per column over the tile totals, a 32-tile window per step;
-//   E. (offsets) base + local offsets leave coalesced;
-//   F. (write) values are packed per column into a staging area laid out so that its 16-byte chunks map to 16-byte
-//      aligned destinations, and leave as 16-byte stores.
-// A tile whose bytes do not fit (one huge quoted field), whose slot arithmetic wraps u32 or whose slots are not
-// monotonic takes the per-value global path of the kernels above for steps C and F.
-constexpr int kSweepThreads = 256;
-constexpr int kSweepWarps = kSweepThreads / 32;
-constexpr uint32_t kSweepMaxCap = 32u * 1024u - 16u; // input bytes staged per tile (relative offsets fit 15 bits)
-constexpr uint32_t kSweepMaxSlotWords = 4096;        // R * slot pitch
-constexpr uint32_t kSweepMaxPairs = 2048;            // R * ncols
-constexpr uint32_t kSlotNone = 0xffffffffu;
-
-__device__ __forceinline__ uint32_t sweep_width(uint32_t ncols) { return ncols | 1u; }           // odd pitches: lanes = rows
-__device__ __forceinline__ uint32_t sweep_slot_pitch(uint32_t row_size) { return (row_size + 1u) | 1u; }   // hit 32 banks
-
-template <bool kOffsets, bool kWrite>
-__global__ void __launch_bounds__(kSweepThreads) materialize_sweep_kernel(const MaterializeMultiParams p)
-{
-    extern __shared__ __align__(16) uint8_t s_raw[];
-    __shared__ uint64_t s_base[kMatMaxCols];
-    __shared__ uint32_t s_gtot[kMatMaxCols][4], s_gpre[kMatMaxCols][4];
-    __shared__ uint32_t s_colstart[kMatMaxCols + 1], s_mis[kMatMaxCols], s_keep[kMatMaxCols];
-    __shared__ uint32_t s_tile, s_fits;
-    const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
-    const uint32_t R = p.rows_per_tile, G = R >> 5, W = sweep_width(p.ncols), pitch = sweep_slot_pitch(p.row_size);
-    const uint32_t cap = p.cap_bytes;
-    const uint32_t stage_cap = cap + 16u * (kMatMaxCols + 1);
-    uint8_t* s_in = s_raw;
-    uint8_t* s_out = s_raw + cap + 16u;
-    uint32_t* s_slot = reinterpret_cast<uint32_t*>(s_out + (kWrite ? stage_cap : 0u));
-    uint32_t* s_val = s_slot + R * pitch;                     // [R][W] start | len << 16 of the (trimmed, unquoted) value
-    uint32_t* s_loc = s_val + R * W;                          // [R][W] exclusive offset inside the 32-record group
-    if (kOffsets) {
-        if (tid == 0) s_tile = atomicAdd(p.ticket, 1u);       // tiles are taken in order: look-back only waits on started tiles
-        __syncthreads();
-    }
-    const uint32_t tile = kOffsets ? s_tile : blockIdx.x;
-    const uint32_t r0 = tile * R, nr = p.nrec - r0 < R ? p.nrec - r0 : R;
-    // rows of the tile in the reference's numbering (the header is row 0); a row at or past record_cnt is Ok(None)
-    const uint64_t first_row = (uint64_t)p.first_record + r0 + 1u;
-    uint32_t nrv = first_row < p.record_cnt ? (p.record_cnt - first_row < nr ? (uint32_t)(p.record_cnt - first_row) : nr) : 0u;
-    const uint64_t slot_first = first_row * p.row_size, slot_last = slot_first + (uint64_t)nrv * p.row_size;
-    if (slot_first >= p.index_len) nrv = 0;
-    const bool wraps = slot_last >= 0xffffffffull;            // the reference computes slots in u32: take the exact path
-    // ---- A + B: slots and bytes, every global load of a step in flight before the first one is used ----
-    // The tile's slots are one contiguous run of the index: the rows' own slots (nmain of them) + the one that ends the
-    // last row (= the tile's last slot, fetched as `hi`).  (row, f) of slot j advance incrementally (no division in
-    // the loop); the slot that ends a row is also the next row's first.
-    constexpr int kSlotBatch = 8, kByteBatch = 4;
-    const uint32_t rs = p.row_size, nmain = (nrv && !wraps) ? nrv * rs : 0u;
-    const uint64_t* __restrict__ src = p.index + slot_first;
-    const uint64_t avail = nmain ? p.index_len - slot_first : 0ull;
-    uint64_t lo = 0, hi = 0, v[kSlotBatch];
-    if (nmain) {
-        lo = ldg_u64(src);
-        hi = ldg_u64(p.index + (slot_last < p.index_len ? slot_last : p.index_len - 1u));
-    }
-#pragma unroll
-    for (int k = 0; k < kSlotBatch; ++k) {
-        const uint32_t j = tid + (uint32_t)k * kSweepThreads;
-        v[k] = (j < nmain && j < avail) ? ldg_u64(src + j) : 0ull;
-    }
-    lo = lo + 1u - p.pos_bias;                                // first byte of the tile's first row
-    hi = hi - p.pos_bias;                                     // the separator that ends its last row (or the last entry)
-    const uint64_t lo16 = lo & ~15ull;
-    int bad = (!nmain || hi < lo || hi > p.n || hi - lo16 > cap) ? (nrv ? 1 : 0) : 0;
-    const bool want_bytes = nmain && !bad && (p.flags != 0u || kWrite);
-    const uint32_t span0 = want_bytes ? (uint32_t)(hi - lo16) : 0u;   // (the slots are still to be checked)
-    uint4 bytes[kByteBatch];
-#pragma unroll
-    for (int k = 0; k < kByteBatch; ++k) {
-        const uint32_t j = (tid + (uint32_t)k * kSweepThreads) * 16u;
-        bytes[k] = make_uint4(0, 0, 0, 0);
-        if (j < span0 && lo16 + j + 16 <= p.n) bytes[k] = ldg_128(p.bytes + lo16 + j);
-    }
-    if (nmain && !bad) {
-        const uint64_t sub = p.pos_bias + lo16 - 1u;
-        const uint32_t drow = kSweepThreads / rs, df = kSweepThreads - drow * rs;
-        uint32_t row = tid / rs, f = tid - row * rs;
-        auto put_slot = [&](uint64_t raw, bool present) {
-            uint32_t rel = kSlotNone;                         // stored: the byte AFTER the separator, relative to lo16
-            if (present) {
-                const uint64_t d = raw - sub;
-                if (d > (uint64_t)cap + 1u) bad = 1;          // not inside the tile's range: a slot out of order
-                rel = (uint32_t)d;
-            }
-            s_slot[row * pitch + f] = rel;
-            if (f == 0u && row > 0u) s_slot[(row - 1u) * pitch + rs] = rel;
-            row += drow;
-            f += df;
-            if (f >= rs) {
-                f -= rs;
-                ++row;
-            }
-        };
-#pragma unroll
-        for (int k = 0; k < kSlotBatch; ++k) {
-            const uint32_t j = tid + (uint32_t)k * kSweepThreads;
-            if (j < nmain) put_slot(v[k], j < avail);
-        }
-        for (uint32_t j = tid + kSlotBatch * kSweepThreads; j < nmain; j += kSweepThreads)   // long rows only
-            put_slot(j < avail ? ldg_u64(src + j) : 0ull, j < avail);
-        if (tid == 0)                                         // the slot that ends the last row
-            s_slot[(nrv - 1u) * pitch + rs] = slot_last < p.index_len ? (uint32_t)(hi + 1u - lo16) : kSlotNone;
-    }
-    const bool staged = __syncthreads_or(bad) == 0;
-    const uint32_t span = (staged && nmain) ? (uint32_t)(hi - lo16) : 0u;
-    if (staged && want_bytes) {
-#pragma unroll
-        for (int k = 0; k < kByteBatch; ++k) {
-            const uint32_t j = (tid + (uint32_t)k * kSweepThreads) * 16u;
-            if (j < span) {
-                if (lo16 + j + 16 > p.n) {                    // the last bytes of the input, one at a time
-                    uint32_t w[4] = {0, 0, 0, 0};
-                    for (uint32_t b = 0; b < 16 && lo16 + j + b < p.n; ++b) w[b >> 2] |= (uint32_t)p.bytes[lo16 + j + b] << (8 * (b & 3));
-                    bytes[k] = make_uint4(w[0], w[1], w[2], w[3]);
-                }
-                *reinterpret_cast<uint4*>(s_in + j) = bytes[k];
-            }
-        }
-        for (uint32_t j = (tid + kByteBatch * kSweepThreads) * 16u; j < span; j += kSweepThreads * 16u) {
-            const uint64_t g = lo16 + j;
-            uint4 b4;
-            if (g + 16 <= p.n) {
-                b4 = ldg_128(p.bytes + g);
-            } else {
-                uint32_t w[4] = {0, 0, 0, 0};
-                for (uint32_t b = 0; b < 16 && g + b < p.n; ++b) w[b >> 2] |= (uint32_t)p.bytes[g + b] << (8 * (b & 3));
-                b4 = make_uint4(w[0], w[1], w[2], w[3]);
-            }
-            *reinterpret_cast<uint4*>(s_in + j) = b4;
-        }
-    }
-    if (staged && want_bytes) __syncthreads();
-    // ---- C: one value per lane ----
-    const uint32_t g = warp % G, row = 32u * g + lane;
-    for (uint32_t c = warp / G; c < p.ncols; c += kSweepWarps / G) {
-        const uint32_t f = p.field_idx[c];
-        uint32_t a = 0, len = 0;
-        if (staged) {
-            bool ok = row < nrv && f < p.field_cnt;
-            uint32_t b = 0;
-            if (ok) {
-                a = s_slot[row * pitch + f];
-                const uint32_t nb = s_slot[row * pitch + f + 1u];
-                b = nb - 1u;                                  // the next separator itself
-                ok = a != kSlotNone && nb != kSlotNone && nb != 0u && a <= b;
-            }
-            if (ok) {
-                if (p.flags & 2u) {
-                    while (a < b && (s_in[a] == 0x20u || s_in[a] == 0x09u)) ++a;
-                    while (b > a && (s_in[b - 1] == 0x20u || s_in[b - 1] == 0x09u)) --b;
-                }
-                if ((p.flags & 1u) && b - a >= 2u && s_in[a] == 0x22u && s_in[b - 1] == 0x22u) {
-                    ++a;
-                    --b;
-                    if (kWrite) {                             // collapse "" in place: the output never passes the input
-                        uint8_t* dst = s_in + a;
-                        auto put = [&](uint32_t ch) { *dst++ = (uint8_t)ch; };
-                        Unquoter<decltype(put)> u{put};
-                        for (uint32_t k = a; k < b; ++k) u(s_in[k]);
-                        u.finish();
-                        len = (uint32_t)(dst - (s_in + a));
-                    } else {
-                        auto count = [&](uint32_t) { ++len; };
-                        Unquoter<decltype(count)> u{count};
-                        for (uint32_t k = a; k < b; ++k) u(s_in[k]);
-                        u.finish();
-                    }
-                } else {
-                    len = b - a;
-                }
-            }
-        } else if (row < nr) {
-            len = (uint32_t)value_len(view_of(p, c), p.first_record + r0 + row);
-        }
-        uint32_t inc = len;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            const uint32_t u = __shfl_up_sync(0xffffffffu, inc, d);
-            if (lane >= (uint32_t)d) inc += u;
-        }
-        s_val[row * W + c] = staged ? a | (len << 16) : len;
-        s_loc[row * W + c] = inc - len;
-        if (lane == 31) s_gtot[c][g] = inc;
-    }
-    __syncthreads();
-    // ---- D: column bases ----
-    if (kOffsets) {
-        for (uint32_t c = warp; c < p.ncols; c += kSweepWarps) {
-            uint64_t* desc = p.tile_desc + (uint64_t)c * p.tiles;
-            uint64_t total = 0;
-            for (uint32_t k = 0; k < G; ++k) {
-                if (lane == 0) s_gpre[c][k] = (uint32_t)total;
-                total += s_gtot[c][k];
-            }
-            const uint64_t prefix = lookback_warp(desc, tile, total, lane);
-            if (lane == 0) {
-                s_base[c] = prefix;
-                if (r0 + nr == p.nrec) p.offsets[c][p.nrec] = prefix + total;
-            }
-        }
-    } else if (tid < p.ncols) {
-        s_base[tid] = p.offsets[tid][r0];
-        uint32_t run = 0;
-        for (uint32_t k = 0; k < G; ++k) {
-            s_gpre[tid][k] = run;
-            run += s_gtot[tid][k];
-        }
-    }
-    __syncthreads();
-    // ---- E: offsets ----
-    if (kOffsets && row < nr) {
-        for (uint32_t c = warp / G; c < p.ncols; c += kSweepWarps / G) {
-            p.offsets[c][r0 + row] = s_base[c] + s_gpre[c][g] + s_loc[row * W + c];
-        }
-    }
-    if (!kWrite) return;
-    // ---- F: values ----
-    if (tid == 0) {
-        uint32_t at = 0;
-        bool fits = staged;
-        for (uint32_t c = 0; c < p.ncols && fits; ++c) {
-            uint32_t total = 0;
-            for (uint32_t k = 0; k < G; ++k) total += s_gtot[c][k];
-            const uint32_t mis = (uint32_t)((reinterpret_cast<uintptr_t>(p.out[c]) + s_base[c]) & 15u);
-            s_colstart[c] = at;
-            s_mis[c] = mis;
-            s_keep[c] = 0;
-            at += (mis + total + 15u) & ~15u;
-            if (at > stage_cap) fits = false;                  // cannot happen with distinct columns (the host checks)
-        }
-        s_colstart[p.ncols] = at;
-        s_fits = fits ? 1u : 0u;
-    }
-    __syncthreads();
-    const bool fits = s_fits != 0u;
-    for (uint32_t c = warp / G; c < p.ncols; c += kSweepWarps / G) {
-        if (row >= nr) break;
-        const uint32_t local = s_gpre[c][g] + s_loc[row * W + c];
-        const uint32_t av = s_val[row * W + c];
-        if (fits) {
-            const uint32_t a = av & 0xffffu, len = av >> 16;
-            if (len == 0u || s_base[c] + local + len > p.out_cap[c]) continue;          // the device form clips whole values
-            atomicMax(&s_keep[c], local + len);
-            uint8_t* dst = s_out + s_colstart[c] + s_mis[c] + local;
-            const uint8_t* src = s_in + a;
-            for (uint32_t k = 0; k < len; ++k) dst[k] = src[k];
-        } else {                                               // per value, straight from and to global memory
-            const FieldView fv = view_of(p, c);
-            const uint8_t* __restrict__ x = p.bytes;
-            uint8_t* __restrict__ out = p.out[c];
-            uint64_t va, vb;
-            if (!field_range(fv, p.first_record + r0 + row, va, vb)) continue;
-            uint64_t o = s_base[c] + local;
-            const uint64_t len = staged ? av >> 16 : av;       // staged, but the staging area overflowed: see s_fits
-            if (o + len > p.out_cap[c]) continue;
-            auto put = [&](uint32_t ch) { out[o++] = (uint8_t)ch; };
-            if (!trim_and_test(fv, va, vb)) {
-                scan_bytes(x, p.n, va, vb, put);
-            } else {
-                Unquoter<decltype(put)> u{put};
-                scan_bytes(x, p.n, va, vb, u);
-                u.finish();
-            }
-        }
-    }
-    if (!fits) return;
-    __syncthreads();
-    const uint32_t chunks = s_colstart[p.ncols] >> 4;
-    for (uint32_t q = tid; q < chunks; q += kSweepThreads) {
-        const uint32_t at = q << 4;
-        uint32_t c = 0;
-        while (c + 1 < p.ncols && s_colstart[c + 1] <= at) ++c;
-        const uint32_t local = at - s_colstart[c];              // byte offset inside the column's region (mis included)
-        const uint32_t first = s_mis[c], last = s_mis[c] + s_keep[c];   // live bytes of the region: [first, last)
-        uint8_t* gp = p.out[c] + s_base[c] - s_mis[c] + local;
-        if (local >= first && local + 16u <= last) {
-            *reinterpret_cast<uint4*>(gp) = *reinterpret_cast<const uint4*>(s_out + at);
-        } else {
-            for (uint32_t b = 0; b < 16; ++b)
-                if (local + b >= first && local + b < last) gp[b] = s_out[at + b];
-        }
-    }
-}
-
-size_t sweep_smem_bytes(const MaterializeMultiParams& p, bool write)
-{
-    const size_t R = p.rows_per_tile;
-    return (size_t)p.cap_bytes + 16 + (write ? (size_t)p.cap_bytes + 16 * (kMatMaxCols + 1) : 0) +
-           (R * (((size_t)p.row_size + 1) | 1) + 2 * R * (p.ncols | 1u)) * sizeof(uint32_t);
 }
 
 }  // namespace
 
-// Plan of the row sweep: rows per tile (0 = use the per-row kernels) and the bytes of input staged per tile.
-// OPT-IN (CSVB200_MAT_SWEEP): measured on a B200 (256 MiB of the 16-field workloads, UNQUOTE | TRIM, offsets + values in
-// one call, ms; profiles/r02_mat_sweep_ab.jsonl):
-//                         4 columns        8 columns        16 columns
-//     unquoted  per-row   0.535            0.933            1.785
-//               sweep     0.684            1.095            1.694
-//     quoted    per-row   0.865            1.661            1.850
-//               sweep     0.677            1.356            2.214
-// The sweep reads every input byte and index slot once, coalesced (DRAM traffic 0.72 GB against 1.9 GB for 8 columns),
-// but a tile publishes its column totals only after all of its work, so every tile ends up waiting in the look-back
-// for the slowest of the ~100 tiles in flight before it (ncu: a third of the warp samples), and the kernel needs
-// ~450 thread instructions per value.  It wins on quoted columns (the byte walks run on shared memory) and loses on
-// short unquoted values, so the per-row kernels stay the default; what would make it win everywhere is the deferred
-// look-back of the index build (classify tile t + 1 while tile t's prefix resolves).
-uint32_t materialize_sweep_plan(uint64_t n, uint32_t record_cnt, uint32_t row_size, uint32_t ncols, uint32_t* cap_bytes)
+size_t materialize_multi_scratch_bytes(uint32_t nrec, uint32_t ncols)
 {
-    // CSVB200_MAT_SWEEP: unset / 0 = per-row kernels, 1 = sweep, 32 / 64 / 128 = sweep with that many rows per tile;
-    // CSVB200_MAT_CAP: staged bytes per tile (tests: small values push tiles onto the per-value path).  Read per call.
-    const char* env = getenv("CSVB200_MAT_SWEEP");
-    const int force = env ? atoi(env) : -1;
-    *cap_bytes = 0;
-    if (force <= 0 || ncols == 0) return 0;
-    const uint64_t avg_row = n / (record_cnt ? record_cnt : 1u) + 1;
-    const uint64_t pitch = ((uint64_t)row_size + 1) | 1;
-    uint32_t rows = 0;
-    for (uint32_t r = 128; r >= 32; r >>= 1) {
-        if (force > 1 && r != (uint32_t)force) continue;
-        if (force <= 1 && (r * avg_row * 3 / 2 > kSweepMaxCap || r * pitch > kSweepMaxSlotWords || r * ncols > kSweepMaxPairs)) continue;
-        rows = r;
-        break;
-    }
-    if (rows == 0 || rows * pitch > kSweepMaxSlotWords || rows * ncols > kSweepMaxPairs) return 0;
-    uint64_t cap = (rows * avg_row * 2 + 1023) & ~1023ull;
-    if (cap < 4096) cap = 4096;
-    if (cap > kSweepMaxCap) cap = kSweepMaxCap;
-    if (const char* e = getenv("CSVB200_MAT_CAP")) {
-        const long v = atol(e);
-        if (v >= 64 && v <= (long)kSweepMaxCap) cap = (uint64_t)v & ~15ull;
-    }
-    *cap_bytes = (uint32_t)cap;
-    return rows;
-}
-
-size_t materialize_multi_scratch_bytes(uint32_t nrec, uint32_t ncols, uint32_t rows_per_tile)
-{
-    const size_t per = rows_per_tile ? rows_per_tile : (uint32_t)kMultiThreads;
-    const size_t tiles = ((size_t)nrec + per - 1) / per + 1;
+    const size_t tiles = ((size_t)nrec + kMultiThreads - 1) / kMultiThreads + 1;
     return 128 + tiles * ncols * sizeof(uint64_t);
-}
-
-template <bool kOffsets, bool kWrite>
-static cudaError_t sweep_launch(const MaterializeMultiParams& p, cudaStream_t stream)
-{
-    static std::mutex mu;                                   // one attribute cache per instantiation and device
-    static bool done[64] = {};
-    constexpr size_t kMax = kSweepMaxCap + 16 + kSweepMaxCap + 16 * (kMatMaxCols + 1) +
-                            (kSweepMaxSlotWords + 2 * (kSweepMaxPairs + 128)) * sizeof(uint32_t);
-    int dev = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e != cudaSuccess) return e;
-    {
-        std::lock_guard<std::mutex> lock(mu);
-        if (dev >= 64 || !done[dev]) {
-            e = cudaFuncSetAttribute(materialize_sweep_kernel<kOffsets, kWrite>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMax);
-            if (e != cudaSuccess) return e;
-            if (dev < 64) done[dev] = true;
-        }
-    }
-    materialize_sweep_kernel<kOffsets, kWrite><<<p.tiles, kSweepThreads, sweep_smem_bytes(p, kWrite), stream>>>(p);
-    return cudaGetLastError();
-}
-
-// one launch: offsets, values, or both in one pass
-cudaError_t launch_materialize_sweep(const MaterializeMultiParams& p, bool offsets, bool write, cudaStream_t stream)
-{
-    if (p.tiles == 0 || p.ncols == 0 || !(offsets || write)) return cudaSuccess;
-    if (offsets && write) return sweep_launch<true, true>(p, stream);
-    return offsets ? sweep_launch<true, false>(p, stream) : sweep_launch<false, true>(p, stream);
 }
 
 cudaError_t launch_materialize_multi_offsets(const MaterializeMultiParams& p, cudaStream_t stream)

@@ -601,48 +601,45 @@ def test_tape_chunks_vs_oracle(ctx):
         idx.free()
 
 
-@pytest.mark.parametrize("sweep", ["0", "1", "32:1024", "64"])
 @pytest.mark.parametrize("flags", [0, 1, 2, 3])
-def test_materialize_columns_row_sweep_and_per_row_paths(ctx, flags, sweep, monkeypatch):
-    """Both forms of csvb200_materialize_columns on the same requests: the row sweep (tiles of R records staged through
-    shared memory; forced here, also with 32- and 64-row tiles and a 1 KiB staging area) and the per-row kernels, against the oracle.  Cases: every escape
-    shape of _column_cases, a 40 KB quoted field (its tile does not fit the staging area: per-value path inside the
-    sweep), a column listed twice (per-row kernels: the sweep unquotes in place), CRLF rows, a sub-range, clipping by out_cap in the device form."""
+def test_materialize_columns_vs_oracle(ctx, flags):
+    """csvb200_materialize_columns: several columns of the same records in one sweep per pass; every column equals what
+    the oracle's scalar definition and the single-column call give.  Cases: every escape shape of _column_cases, alone
+    and behind a 40 KB quoted field, one column, a column listed more than once, an out-of-range field, empty ranges, a
+    range that runs past the last record, 17 columns = more columns than warps, clipping by out_cap in the device form,
+    CRLF rows and a wide quoted file."""
     import torch
-    monkeypatch.setenv("CSVB200_MAT_SWEEP", sweep.split(":")[0])
-    if ":" in sweep:
-        monkeypatch.setenv("CSVB200_MAT_CAP", sweep.split(":")[1])   # 1 KiB staged per tile: many tiles take the per-value path
+    dev = torch.device("cuda", ctx.device)
     big = b'"' + b'ab""cd, \n' * 4000 + b'"'
     head, rest = _column_cases().split(b"\n", 1)
-    raw = head + b"\n" + b"77, " + big + b" ,tail\n" + b"78,x,y\n" * 40 + rest
-    idx = ctx.index_build(raw, cs.BUILD_KEEP_BYTES)
-    rc, jump = idx.tape_init(3, False)
-    host = idx.to_host()
-    for fields, first, nrec in (([0, 1, 2], 0, rc - 1), ([2, 0], 17, 1000), ([1, 1, 1, 1], 0, 60), ([1, 7, 2, 2], rc - 5, 20),
-                                ([0, 1], 5, 0), ([2, 1, 0] * 5 + [1, 2], 1024, 1100)):
-        got = idx.materialize_columns(fields, first, nrec, flags)
-        for f, (offs, out) in zip(fields, got):
-            w_offs, w_out = O.materialize_column(raw, host, rc, 3, False, f, first, nrec, flags)
-            assert (offs == w_offs).all(), (fields, f, first, nrec)
-            assert out.tobytes() == w_out, (fields, f, first, nrec)
-    # device form, destination too small for the last values: whole values are clipped, nothing past out_cap is written
-    dev = torch.device("cuda", ctx.device)
-    fields, nrec = [1, 2], rc - 1
-    want = [O.materialize_column(raw, host, rc, 3, False, f, 0, nrec, flags) for f in fields]
-    caps = [len(w[1]) // 2 + 3 for w in want]
-    d_off = [torch.zeros(nrec + 1, dtype=torch.int64, device=dev) for _ in fields]
-    d_out = [torch.full((len(w[1]) + 64,), 0xEE, dtype=torch.uint8, device=dev) for w in want]
-    torch.cuda.synchronize()
-    idx.materialize_columns_device(fields, 0, nrec, flags, [t.data_ptr() for t in d_off], [t.data_ptr() for t in d_out], caps)
-    idx.sync()
-    torch.cuda.synchronize()
-    for (w_offs, w_out), cap, o, v in zip(want, caps, d_off, d_out):
-        assert (o.cpu().numpy().view(np.uint64) == w_offs).all()
-        keep = int(w_offs[w_offs <= cap].max())
-        got = v.cpu().numpy()
-        assert got[:keep].tobytes() == w_out[:keep]
-        assert (got[keep:] == 0xEE).all()
-    idx.free()
+    for raw in (_column_cases(), head + b"\n" + b"77, " + big + b" ,tail\n" + b"78,x,y\n" * 40 + rest):
+        idx = ctx.index_build(raw, cs.BUILD_KEEP_BYTES)
+        rc, jump = idx.tape_init(3, False)
+        host = idx.to_host()
+        for fields, first, nrec in (([0, 1, 2], 0, rc - 1), ([2, 0], 17, 1000), ([1], 3, 700), ([1, 1, 1, 1], 0, 60),
+                                    ([1, 7, 2, 2], rc - 5, 20), ([0, 1], 5, 0), ([2, 1, 0] * 5 + [1, 2], 1024, 1100)):
+            got = idx.materialize_columns(fields, first, nrec, flags)
+            for f, (offs, out) in zip(fields, got):
+                w_offs, w_out = O.materialize_column(raw, host, rc, 3, False, f, first, nrec, flags)
+                assert (offs == w_offs).all(), (fields, f, first, nrec)
+                assert out.tobytes() == w_out, (fields, f, first, nrec)
+        # device form, destination too small for the last values: whole values are clipped, nothing past out_cap is written
+        fields, nrec = [1, 2], rc - 1
+        want = [O.materialize_column(raw, host, rc, 3, False, f, 0, nrec, flags) for f in fields]
+        caps = [len(w[1]) // 2 + 3 for w in want]
+        d_off = [torch.zeros(nrec + 1, dtype=torch.int64, device=dev) for _ in fields]
+        d_out = [torch.full((len(w[1]) + 64,), 0xEE, dtype=torch.uint8, device=dev) for w in want]
+        torch.cuda.synchronize()
+        idx.materialize_columns_device(fields, 0, nrec, flags, [t.data_ptr() for t in d_off], [t.data_ptr() for t in d_out], caps)
+        idx.sync()
+        torch.cuda.synchronize()
+        for (w_offs, w_out), cap, o, v in zip(want, caps, d_off, d_out):
+            assert (o.cpu().numpy().view(np.uint64) == w_offs).all()
+            keep = int(w_offs[w_offs <= cap].max())
+            got = v.cpu().numpy()
+            assert got[:keep].tobytes() == w_out[:keep]
+            assert (got[keep:] == 0xEE).all()
+        idx.free()
     # CRLF rows (row_size = field_cnt + 1) and a wide quoted file against the single-column kernels
     raw = golden_bytes("sample_rx.csv")
     idx = ctx.index_build(raw, cs.BUILD_KEEP_BYTES)
@@ -660,6 +657,39 @@ def test_materialize_columns_row_sweep_and_per_row_paths(ctx, flags, sweep, monk
     for f in (0, 1, 7, 15):
         offs, out = idx.materialize_column(f, 0, rc - 1, flags)
         assert (got[f][0] == offs).all() and got[f][1].tobytes() == out.tobytes()
+    idx.free()
+
+
+def test_materialize_device_forms_reject_null_destinations(ctx):
+    """Both device forms check every column's destinations before they launch anything: a null offsets array, or a
+    capacity above 0 with no value buffer, is CSVB200_ERR_INVALID_ARG (ValueError).  The index stays usable."""
+    import torch
+    raw = _column_cases()
+    idx = ctx.index_build(raw, cs.BUILD_KEEP_BYTES)
+    rc, _ = idx.tape_init(3, False)
+    host = idx.to_host()
+    fields, nrec, flags = [1, 2], rc - 1, cs.FIELD_UNQUOTE | cs.FIELD_TRIM
+    want = [O.materialize_column(raw, host, rc, 3, False, f, 0, nrec, flags) for f in fields]
+    dev = torch.device("cuda", ctx.device)
+    d_off = [torch.zeros(nrec + 1, dtype=torch.int64, device=dev) for _ in fields]
+    d_out = [torch.zeros(len(w[1]), dtype=torch.uint8, device=dev) for w in want]
+    p_off, p_out, caps = [t.data_ptr() for t in d_off], [t.data_ptr() for t in d_out], [len(w[1]) for w in want]
+    torch.cuda.synchronize()
+    with pytest.raises(ValueError):
+        idx.materialize_columns_device(fields, 0, nrec, flags, [p_off[0], 0])
+    with pytest.raises(ValueError):
+        idx.materialize_columns_device(fields, 0, nrec, flags, p_off, [p_out[0], 0], caps)
+    with pytest.raises(ValueError):
+        idx.materialize_columns_device(fields, 0, nrec, flags, p_off, None, caps)
+    with pytest.raises(ValueError):
+        idx.materialize_column_device(fields[0], 0, nrec, flags, 0, p_out[0], caps[0])
+    with pytest.raises(ValueError):
+        idx.materialize_column_device(fields[0], 0, nrec, flags, p_off[0], 0, caps[0])
+    idx.materialize_columns_device(fields, 0, nrec, flags, p_off, p_out, caps)
+    torch.cuda.synchronize()
+    for (w_offs, w_out), o, v in zip(want, d_off, d_out):
+        assert (o.cpu().numpy().view(np.uint64) == w_offs).all()
+        assert v.cpu().numpy().tobytes() == w_out
     idx.free()
 
 
@@ -1500,34 +1530,6 @@ def test_multi_distributed_index_lookups_two_gpus():
     m = cs.Multi(list(range(min(torch.cuda.device_count(), 8))))
     _check_multi_lookups(m, nfields=256, size=64 << 20)
     m.close()
-
-
-@pytest.mark.parametrize("flags", [0, 3])
-def test_materialize_columns_one_sweep_vs_oracle(ctx, flags):
-    """csvb200_materialize_columns: several columns of the same records in one sweep per pass; every column equals what
-    the single-column call and the oracle's scalar definition give (incl. an out-of-range field, empty ranges, a range
-    that runs past the last record, 17 columns = more columns than warps)."""
-    raw = _column_cases()
-    idx = ctx.index_build(raw, cs.BUILD_KEEP_BYTES)
-    rc, jump = idx.tape_init(3, False)
-    host = idx.to_host()
-    for fields, first, nrec in (([0, 1, 2], 0, rc - 1), ([2, 0], 17, 1000), ([1], 3, 700), ([1, 7, 2, 2], rc - 5, 20),
-                                ([0, 1], 5, 0), ([2, 1, 0] * 5 + [1, 2], 1024, 1100)):
-        got = idx.materialize_columns(fields, first, nrec, flags)
-        for f, (offs, out) in zip(fields, got):
-            w_offs, w_out = O.materialize_column(raw, host, rc, 3, False, f, first, nrec, flags)
-            assert (offs == w_offs).all(), (fields, f, first, nrec)
-            assert out.tobytes() == w_out, (fields, f, first, nrec)
-    idx.free()
-    # a wide quoted file: all 16 columns at once against the single-column kernel
-    q, _ = gen.quoted(3 << 20, seed=43)
-    idx = ctx.index_build(q, cs.BUILD_KEEP_BYTES)
-    rc, _ = idx.tape_init(16, True)
-    got = idx.materialize_columns(list(range(16)), 0, rc - 1, flags)
-    for f in (0, 1, 7, 15):
-        offs, out = idx.materialize_column(f, 0, rc - 1, flags)
-        assert (got[f][0] == offs).all() and got[f][1].tobytes() == out.tobytes()
-    idx.free()
 
 
 def test_bench_dump_outputs_vs_oracle():

@@ -53,8 +53,7 @@ def main():
         return e0.elapsed_time(e1) / reps
     ms_off = timed(lambda: idx.materialize_columns_device(cols, 0, nrec, 3, p_offs))
     ms_both = timed(lambda: idx.materialize_columns_device(cols, 0, nrec, 3, p_offs, p_outs, totals))
-    print(json.dumps({"workload": wl, "bytes": n, "records": nrec, "columns": cols, "sweep_env": os.environ.get("CSVB200_MAT_SWEEP"),
-                      "ms_offsets": ms_off, "ms_offsets_plus_write": ms_both, "value_bytes": sum(totals)}))
+    print(json.dumps({"workload": wl, "bytes": n, "records": nrec, "columns": cols, "ms_offsets": ms_off, "ms_offsets_plus_write": ms_both, "value_bytes": sum(totals)}))
     idx.free()
     ctx.close()
 

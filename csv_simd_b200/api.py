@@ -462,6 +462,27 @@ class MultiIndex:
         self._check(self._lib.csvb200_multi_seek_records(self._h, rec.ctypes.data, rec.size, out.ctypes.data))
         return out
 
+    def materialize_columns(self, fields, first_record: int, nrec: int, flags: int = FIELD_RAW):
+        """csvb200_multi_materialize_columns: as StructureIndex.materialize_columns, each device materialising the records
+        it holds -> [(offsets, values)] per requested field."""
+        f = np.ascontiguousarray(fields, dtype=np.uint32)
+        k = int(f.size)
+        offs = [np.zeros(nrec + 1, dtype=np.uint64) for _ in range(k)]
+        p_off = (C.c_void_p * k)(*[o.ctypes.data for o in offs])
+        lens = (C.c_size_t * k)()
+        caps = (C.c_size_t * k)()
+        rc = self._lib.csvb200_multi_materialize_columns(self._h, f.ctypes.data, k, first_record, nrec, flags, p_off, None,
+                                                         caps, lens)
+        if rc not in (0, 9):      # CSVB200_ERR_CAPACITY sizes the outputs
+            self._check(rc)
+        vals = [np.empty(int(lens[c]), dtype=np.uint8) for c in range(k)]
+        if any(v.size for v in vals):
+            p_out = (C.c_void_p * k)(*[v.ctypes.data if v.size else None for v in vals])
+            caps = (C.c_size_t * k)(*[v.size for v in vals])
+            self._check(self._lib.csvb200_multi_materialize_columns(self._h, f.ctypes.data, k, first_record, nrec, flags,
+                                                                    p_off, p_out, caps, lens))
+        return list(zip(offs, vals))
+
     def seek_fields_device(self, k: int, d_rec: int, d_fld: int, nq: int, d_out: int):
         self._check(self._lib.csvb200_multi_seek_fields_device(self._h, k, C.c_void_p(d_rec), C.c_void_p(d_fld), nq,
                                                                C.c_void_p(d_out)))

@@ -10,7 +10,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libcsvb200.so")
 SOURCES = ["api.cu", "index_build.cu", "index_build_tma.cu", "lookup.cu", "tape.cu", "materialize.cu", "stream.cu", "validate.cu", "exchange.cu"]
-HEADERS = ["internal.h", "ctx.h", "slice_pool.h", "bitslice.cuh", "utf8slice.cuh", "index_common.cuh", os.path.join("..", "..", "include", "csvb200.h")]
+HEADERS = ["internal.h", "ctx.h", "slice_pool.h", "record_split.h", "bitslice.cuh", "utf8slice.cuh", "index_common.cuh", os.path.join("..", "..", "include", "csvb200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -1752,19 +1752,19 @@ int csvb200_gather_fields(csvb200_index* idx, const uint32_t* rec, const uint32_
 }
 
 // enqueue lengths + scan (+ write when d_out != nullptr) of one column on the context's stream
-static int materialize_enqueue(csvb200_index* idx, uint32_t field_idx, uint32_t first_record, uint32_t nrec, uint32_t flags,
-                               uint64_t* d_offsets, uint8_t* d_out, size_t out_cap, bool offsets_pass, bool write_pass)
+static int materialize_enqueue(csvb200_ctx* ctx, const MatSource& src, uint32_t field_idx, uint32_t first_record, uint32_t nrec,
+                               uint32_t flags, uint64_t* d_offsets, uint8_t* d_out, size_t out_cap, uint64_t offset_base,
+                               bool offsets_pass, bool write_pass)
 {
-    csvb200_ctx* ctx = idx->ctx;
     MaterializeParams p{};
-    p.index = idx->d_index;
-    p.index_len = idx->len;
-    p.bytes = idx->d_bytes_owned ? idx->d_bytes_owned : idx->src;
-    p.n = idx->n;
-    p.pos_bias = idx->pos_bias;
-    p.record_cnt = idx->record_cnt;
-    p.field_cnt = idx->field_cnt;
-    p.row_size = (uint32_t)idx->jump;
+    p.index = src.index;
+    p.index_len = src.index_len;
+    p.bytes = src.bytes;
+    p.n = src.n;
+    p.pos_bias = src.pos_bias;
+    p.record_cnt = src.record_cnt;
+    p.field_cnt = src.field_cnt;
+    p.row_size = src.row_size;
     p.field_idx = field_idx;
     p.first_record = first_record;
     p.nrec = nrec;
@@ -1772,6 +1772,7 @@ static int materialize_enqueue(csvb200_index* idx, uint32_t field_idx, uint32_t 
     p.offsets = d_offsets;
     p.out = d_out;
     p.out_cap = out_cap;
+    p.offset_base = offset_base;
     if (offsets_pass) {
         const size_t sbytes = materialize_scratch_bytes(nrec);
         int rc = ensure_scratch(ctx, sbytes);
@@ -1800,24 +1801,34 @@ static int materialize_prepare(csvb200_index* idx, uint32_t flags)
     return CSVB200_OK;
 }
 
-// several columns, one sweep per pass (materialize.cu: a thread owns a row and walks its requested fields)
-static int materialize_multi_enqueue(csvb200_index* idx, const uint32_t* fields, uint32_t ncols, uint32_t first_record,
-                                     uint32_t nrec, uint32_t flags, uint64_t* const* d_offsets, uint8_t* const* d_outs,
-                                     const size_t* out_caps, bool offsets_pass, bool write_pass)
+static MatSource source_of(const csvb200_index* idx)
 {
-    csvb200_ctx* ctx = idx->ctx;
+    return MatSource{idx->d_index, idx->len, idx->d_bytes_owned ? idx->d_bytes_owned : idx->src, idx->n, idx->pos_bias,
+                     idx->record_cnt, idx->field_cnt, (uint32_t)idx->jump};
+}
+
+}  // extern "C"
+
+namespace csvb200 {
+
+// several columns, one sweep per pass (materialize.cu: a thread owns a row and walks its requested fields)
+int materialize_multi_enqueue(csvb200_ctx* ctx, const MatSource& src, const uint32_t* fields, uint32_t ncols,
+                              uint32_t first_record, uint32_t nrec, uint32_t flags, uint64_t* const* d_offsets,
+                              uint8_t* const* d_outs, const size_t* out_caps, const uint64_t* offset_base, bool offsets_pass,
+                              bool write_pass)
+{
     if (ncols == 1)   // one column: the single-column kernels (1024-record tiles) are the faster form
-        return materialize_enqueue(idx, fields[0], first_record, nrec, flags, d_offsets[0], d_outs ? d_outs[0] : nullptr,
-                                   out_caps ? out_caps[0] : 0, offsets_pass, write_pass);
+        return materialize_enqueue(ctx, src, fields[0], first_record, nrec, flags, d_offsets[0], d_outs ? d_outs[0] : nullptr,
+                                   out_caps ? out_caps[0] : 0, offset_base ? offset_base[0] : 0, offsets_pass, write_pass);
     MaterializeMultiParams p{};
-    p.index = idx->d_index;
-    p.index_len = idx->len;
-    p.bytes = idx->d_bytes_owned ? idx->d_bytes_owned : idx->src;
-    p.n = idx->n;
-    p.pos_bias = idx->pos_bias;
-    p.record_cnt = idx->record_cnt;
-    p.field_cnt = idx->field_cnt;
-    p.row_size = (uint32_t)idx->jump;
+    p.index = src.index;
+    p.index_len = src.index_len;
+    p.bytes = src.bytes;
+    p.n = src.n;
+    p.pos_bias = src.pos_bias;
+    p.record_cnt = src.record_cnt;
+    p.field_cnt = src.field_cnt;
+    p.row_size = src.row_size;
     p.first_record = first_record;
     p.nrec = nrec;
     p.flags = flags;
@@ -1828,6 +1839,7 @@ static int materialize_multi_enqueue(csvb200_index* idx, const uint32_t* fields,
         p.offsets[c] = d_offsets[c];
         p.out[c] = d_outs ? d_outs[c] : nullptr;
         p.out_cap[c] = out_caps ? out_caps[c] : 0;
+        p.offset_base[c] = offset_base ? offset_base[c] : 0;
     }
     if (offsets_pass) {
         const size_t sbytes = materialize_multi_scratch_bytes(nrec, ncols);
@@ -1848,6 +1860,10 @@ static int materialize_multi_enqueue(csvb200_index* idx, const uint32_t* fields,
     return CSVB200_OK;
 }
 
+}  // namespace csvb200
+
+extern "C" {
+
 int csvb200_materialize_columns_device(csvb200_index* idx, const uint32_t* fields, uint32_t ncols, uint32_t first_record,
                                        uint32_t nrec, uint32_t flags, uint64_t* const* d_offsets, uint8_t* const* d_outs,
                                        const size_t* out_caps)
@@ -1859,8 +1875,8 @@ int csvb200_materialize_columns_device(csvb200_index* idx, const uint32_t* field
     for (uint32_t c = 0; c < ncols; ++c)
         if (!d_offsets[c] || (out_caps && out_caps[c] && (!d_outs || !d_outs[c])))
             return fail(idx->ctx, CSVB200_ERR_INVALID_ARG, "null argument");
-    return materialize_multi_enqueue(idx, fields, ncols, first_record, nrec, flags, d_offsets, d_outs, out_caps, true,
-                                     d_outs != nullptr);
+    return materialize_multi_enqueue(idx->ctx, source_of(idx), fields, ncols, first_record, nrec, flags, d_offsets, d_outs,
+                                     out_caps, nullptr, true, d_outs != nullptr);
 }
 
 int csvb200_materialize_columns(csvb200_index* idx, const uint32_t* fields, uint32_t ncols, uint32_t first_record,
@@ -1881,7 +1897,8 @@ int csvb200_materialize_columns(csvb200_index* idx, const uint32_t* fields, uint
         CU_TRY(ctx, d_off[c].alloc(((size_t)nrec + 1) * sizeof(uint64_t), ctx->stream));
         p_off[c] = d_off[c].as<uint64_t>();
     }
-    rc = materialize_multi_enqueue(idx, fields, ncols, first_record, nrec, flags, p_off.data(), nullptr, nullptr, true, false);
+    rc = materialize_multi_enqueue(ctx, source_of(idx), fields, ncols, first_record, nrec, flags, p_off.data(), nullptr, nullptr,
+                                   nullptr, true, false);
     if (rc) return rc;
     for (uint32_t c = 0; c < ncols; ++c)
         CU_TRY(ctx, cudaMemcpyAsync(out_offsets[c], p_off[c], ((size_t)nrec + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1902,7 +1919,8 @@ int csvb200_materialize_columns(csvb200_index* idx, const uint32_t* fields, uint
         p_out[c] = d_out[c].as<uint8_t>();
         caps[c] = out_lens[c];
     }
-    rc = materialize_multi_enqueue(idx, fields, ncols, first_record, nrec, flags, p_off.data(), p_out.data(), caps.data(), false, true);
+    rc = materialize_multi_enqueue(ctx, source_of(idx), fields, ncols, first_record, nrec, flags, p_off.data(), p_out.data(),
+                                   caps.data(), nullptr, false, true);
     if (rc) return rc;
     for (uint32_t c = 0; c < ncols; ++c)
         if (out_lens[c]) CU_TRY(ctx, cudaMemcpyAsync(outs[c], p_out[c], out_lens[c], cudaMemcpyDeviceToHost, ctx->stream));

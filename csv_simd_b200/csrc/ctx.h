@@ -218,6 +218,21 @@ struct DevBuf {
 // place, a pageable one goes through the context's two pinned bounce buffers and its host threads
 int download(csvb200_ctx* ctx, uint64_t* dst, const uint64_t* d_src, size_t count);
 int ensure_bounce(csvb200_ctx* ctx);
+// What the materialisation launches read: the index addressed by global slot (index[s] for s < index_len), the bytes
+// the positions point into (bytes[0] is global byte pos_bias, n of them) and the tape metadata.
+struct MatSource {
+    const uint64_t* index;
+    uint64_t index_len;
+    const uint8_t* bytes;
+    uint64_t n, pos_bias;
+    uint32_t record_cnt, field_cnt, row_size;
+};
+// Enqueues the offsets pass (lengths + scan into d_offsets, offset_base[c] added to column c's; offset_base may be null)
+// and / or the write pass of `ncols` columns on the context's stream; one column goes to the single-column kernels.
+int materialize_multi_enqueue(csvb200_ctx* ctx, const MatSource& src, const uint32_t* fields, uint32_t ncols,
+                              uint32_t first_record, uint32_t nrec, uint32_t flags, uint64_t* const* d_offsets,
+                              uint8_t* const* d_outs, const size_t* out_caps, const uint64_t* offset_base, bool offsets_pass,
+                              bool write_pass);
 // host-side wait for all ranks' rows of one build (exchange.cu)
 int exchange_wait_all(csvb200_exchange* ex, uint64_t epoch, uint64_t* counts, uint32_t* carries);
 

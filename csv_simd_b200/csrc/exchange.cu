@@ -17,6 +17,7 @@
 #include <vector>
 
 #include "ctx.h"
+#include "record_split.h"
 #include "slice_pool.h"
 
 using namespace csvb200;
@@ -220,6 +221,7 @@ struct csvb200_multi_index {
     std::vector<csvb200_index*> seg;      // segment k on device k (global byte positions)
     std::vector<uint8_t*> d_bytes;        // device copies of the shards (kept: csvb200_index_free does not own them)
     std::vector<uint64_t> base;           // base[k] = global slot of seg[k][0]; base[G] = total length
+    std::vector<size_t> cuts;             // byte shard k = global bytes [cuts[k], cuts[k + 1]), held in d_bytes[k]
     SegmentTable table{};                 // the same, as the kernels take it
     bool tape_ready = false;
     uint32_t field_cnt = 0, record_cnt = 0;
@@ -427,6 +429,7 @@ int csvb200_multi_index_build(csvb200_multi* m, const uint8_t* host_bytes, size_
         return rc;
     }
     mi->m = m;
+    mi->cuts = cuts;
     mi->table.nseg = (uint32_t)G;
     for (int k = 0; k < G; ++k) {
         mi->seg.push_back(work[k].idx);
@@ -644,3 +647,213 @@ int csvb200_multi_index_build_to_host(csvb200_multi* m, const uint8_t* host_byte
 }
 
 }  // extern "C"
+
+// ---------------------------------------------------------------------------------------------------------------
+// column materialisation over the distributed index: every device materialises the records whose bytes it holds
+// ---------------------------------------------------------------------------------------------------------------
+namespace {
+
+// An index pointer to hand the kernels so that index[s] addresses global slot s, given the array that starts at slot
+// first_slot.  The pointer itself points before the array; that is safe because the kernels read index[s] only for the
+// slots of the records they are given, and a piece is only given records whose slots all lie in [first_slot, end).
+const uint64_t* by_global_slot(const uint64_t* first, uint64_t first_slot)
+{
+    return reinterpret_cast<const uint64_t*>(reinterpret_cast<uintptr_t>(first) - first_slot * sizeof(uint64_t));
+}
+
+// one piece of a request (record_split.h) and what its device made of it
+struct MatPiece {
+    RecordPiece r{};
+    uint64_t pos = 0;             // window position of its first record
+    int k = 0;                    // the device that runs it
+    MatSource src{};
+    DevBuf row_slots, row_bytes;  // boundary record: its index slots and byte span, staged on device k
+    DevBuf d_off[kMatMaxCols], d_out[kMatMaxCols];
+    uint64_t total[kMatMaxCols] = {}, start[kMatMaxCols] = {};
+};
+
+// Copies the slots and the byte span of boundary record p->r.first to device p->k, from whichever devices hold them.
+int stage_boundary_row(csvb200_multi_index* mi, MatPiece* p)
+{
+    csvb200_ctx* ctx = mi->m->ctx[p->k];
+    const int dev = ctx->device;
+    const uint64_t lo = (uint64_t)(uint32_t)(p->r.first + 1u) * mi->jump, hi = lo + mi->jump;
+    CU_TRY(ctx, p->row_slots.alloc((hi - lo + 1) * sizeof(uint64_t), ctx->stream));
+    uint64_t* slots = p->row_slots.as<uint64_t>();
+    for (uint32_t j = p->r.seg_lo; j <= p->r.seg_hi; ++j) {
+        const uint64_t a = std::max(lo, mi->base[j]), b = std::min(hi + 1, mi->base[j + 1]);
+        if (a < b)
+            CU_TRY(ctx, cudaMemcpyPeerAsync(slots + (a - lo), dev, mi->table.ptr[j] + (a - mi->base[j]), mi->m->ctx[j]->device,
+                                            (b - a) * sizeof(uint64_t), ctx->stream));
+    }
+    uint64_t ends[2];
+    CU_TRY(ctx, cudaMemcpyAsync(&ends[0], slots, sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    CU_TRY(ctx, cudaMemcpyAsync(&ends[1], slots + (hi - lo), sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    // every value of the row lies in (index[lo], index[hi]); the staged bytes start at index[lo] itself, so no position
+    // the kernels compute from the row's slots falls below the span
+    const uint64_t p0 = ends[0], p1 = std::max(ends[0], ends[1]);
+    CU_TRY(ctx, p->row_bytes.alloc(((p1 - p0 + 15) & ~uint64_t(15)) + 16, ctx->stream));
+    for (size_t j = 0; j + 1 < mi->cuts.size(); ++j) {
+        const uint64_t a = std::max<uint64_t>(p0, mi->cuts[j]), b = std::min<uint64_t>(p1, mi->cuts[j + 1]);
+        if (a < b)
+            CU_TRY(ctx, cudaMemcpyPeerAsync(p->row_bytes.as<uint8_t>() + (a - p0), dev, mi->d_bytes[j] + (a - mi->cuts[j]),
+                                            mi->m->ctx[j]->device, b - a, ctx->stream));
+    }
+    p->src.index = by_global_slot(slots, lo);
+    p->src.index_len = hi + 1;
+    p->src.bytes = p->row_bytes.as<uint8_t>();
+    p->src.n = p1 - p0;
+    p->src.pos_bias = p0;
+    return CSVB200_OK;
+}
+
+}  // namespace
+
+extern "C" int csvb200_multi_materialize_columns(csvb200_multi_index* mi, const uint32_t* fields, uint32_t ncols,
+                                                 uint32_t first_record, uint32_t nrec, uint32_t flags,
+                                                 uint64_t* const* out_offsets, uint8_t* const* outs, const size_t* out_caps,
+                                                 size_t* out_lens)
+{
+    if (!mi) return CSVB200_ERR_INVALID_ARG;
+    csvb200_multi* m = mi->m;
+    if (!mi->tape_ready) return mfail(m, CSVB200_ERR_INVALID_STATE, "csvb200_multi_tape_init has not been called");
+    if (flags & ~(CSVB200_FIELD_UNQUOTE | CSVB200_FIELD_TRIM)) return mfail(m, CSVB200_ERR_INVALID_ARG, "unknown field flags");
+    if (!fields || !out_offsets || !out_lens || ncols == 0 || ncols > kMatMaxCols)
+        return mfail(m, CSVB200_ERR_INVALID_ARG, "1 <= ncols <= 32 and non-null arrays");
+    for (uint32_t c = 0; c < ncols; ++c)
+        if (!out_offsets[c]) return mfail(m, CSVB200_ERR_INVALID_ARG, "null argument");
+    // the kernels compute slots in u32, as the reference does; past 2^32 slots that would address the wrong segment
+    if (mi->base.back() > (1ull << 32)) return mfail(m, CSVB200_ERR_INVALID_ARG, "index of more than 2^32 entries");
+    const int G = (int)mi->seg.size();
+    const std::vector<RecordPiece> split =
+        split_records(mi->base.data(), (uint32_t)G, mi->jump, mi->record_cnt, first_record, nrec);
+    std::vector<MatPiece> pieces(split.size());
+    for (size_t i = 0, pos = 0; i < split.size(); pos += split[i].count, ++i) {
+        MatPiece& p = pieces[i];
+        p.r = split[i];
+        p.pos = pos;
+        // interior records read segment k and shard k in place; dead records read nothing, any device will do
+        p.k = p.r.seg_lo < (uint32_t)G ? (int)p.r.seg_lo : G - 1;
+        p.src = MatSource{by_global_slot(mi->table.ptr[p.k], mi->base[p.k]), mi->base[p.k + 1], mi->d_bytes[p.k],
+                          mi->cuts[p.k + 1] - mi->cuts[p.k], mi->cuts[p.k], mi->record_cnt, mi->field_cnt, (uint32_t)mi->jump};
+    }
+    std::vector<int> rcs(G, CSVB200_OK);
+    auto first_error = [&]() -> int {
+        for (int k = 0; k < G; ++k)
+            if (rcs[k]) return mfail(m, rcs[k], "device " + std::to_string(k) + ": " + csvb200_last_error(m->ctx[k]));
+        return CSVB200_OK;
+    };
+    // offsets pass: every piece's value lengths, scanned on its device; only the column totals come back
+    run_phase(m, [&](int k) {
+        csvb200_ctx* ctx = m->ctx[k];
+        rcs[k] = [&]() -> int {
+            CU_TRY(ctx, cudaSetDevice(ctx->device));
+            for (MatPiece& p : pieces) {
+                if (p.k != k) continue;
+                if (!p.r.interior() && p.r.seg_lo < (uint32_t)G) {
+                    int rc = stage_boundary_row(mi, &p);
+                    if (rc) return rc;
+                }
+                uint64_t* d_off[kMatMaxCols];
+                for (uint32_t c = 0; c < ncols; ++c) {
+                    CU_TRY(ctx, p.d_off[c].alloc(((size_t)p.r.count + 1) * sizeof(uint64_t), ctx->stream));
+                    d_off[c] = p.d_off[c].as<uint64_t>();
+                }
+                int rc = materialize_multi_enqueue(ctx, p.src, fields, ncols, p.r.first, p.r.count, flags, d_off, nullptr,
+                                                   nullptr, nullptr, true, false);
+                if (rc) return rc;
+                for (uint32_t c = 0; c < ncols; ++c)
+                    CU_TRY(ctx, cudaMemcpyAsync(&p.total[c], d_off[c] + p.r.count, sizeof(uint64_t), cudaMemcpyDeviceToHost,
+                                                ctx->stream));
+            }
+            CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+            return CSVB200_OK;
+        }();
+    });
+    int rc = first_error();
+    bool small = false, any = false, write = false;
+    if (!rc) {
+        for (uint32_t c = 0; c < ncols; ++c) {
+            uint64_t at = 0;
+            for (MatPiece& p : pieces) {
+                p.start[c] = at;
+                at += p.total[c];
+            }
+            out_lens[c] = (size_t)at;
+            if (at > (out_caps ? out_caps[c] : 0)) small = true;
+            if (at) any = true;
+        }
+        write = !small && any && outs;
+        for (uint32_t c = 0; write && c < ncols; ++c)
+            if (out_lens[c] && !outs[c]) write = false;
+        if (nrec == 0)
+            for (uint32_t c = 0; c < ncols; ++c) out_offsets[c][0] = 0;
+        // write pass: values into device buffers by the offsets of the first pass, then the offsets pass again with
+        // every column's start added, and both straight to their place in the caller's arrays.  The offsets come down
+        // even when the values do not (CSVB200_ERR_CAPACITY, the sizing call).
+        run_phase(m, [&](int k) {
+            csvb200_ctx* ctx = m->ctx[k];
+            rcs[k] = [&]() -> int {
+                CU_TRY(ctx, cudaSetDevice(ctx->device));
+                for (size_t i = 0; i < pieces.size(); ++i) {
+                    MatPiece& p = pieces[i];
+                    if (p.k != k) continue;
+                    uint64_t* d_off[kMatMaxCols];
+                    uint8_t* d_out[kMatMaxCols];
+                    size_t caps[kMatMaxCols];
+                    bool values = false;
+                    for (uint32_t c = 0; c < ncols; ++c) {
+                        d_off[c] = p.d_off[c].as<uint64_t>();
+                        d_out[c] = nullptr;
+                        caps[c] = write ? (size_t)p.total[c] : 0;
+                        if (caps[c]) {
+                            CU_TRY(ctx, p.d_out[c].alloc(caps[c], ctx->stream));
+                            d_out[c] = p.d_out[c].as<uint8_t>();
+                            values = true;
+                        }
+                    }
+                    int rc = CSVB200_OK;
+                    if (values)
+                        rc = materialize_multi_enqueue(ctx, p.src, fields, ncols, p.r.first, p.r.count, flags, d_off, d_out,
+                                                       caps, nullptr, false, true);
+                    if (!rc)
+                        rc = materialize_multi_enqueue(ctx, p.src, fields, ncols, p.r.first, p.r.count, flags, d_off, nullptr,
+                                                       nullptr, p.start, true, false);
+                    if (rc) return rc;
+                    // adjacent pieces share one offset: each brings its own records' offsets, the last piece the end too
+                    const size_t n_off = (size_t)p.r.count + (i + 1 == pieces.size() ? 1 : 0);
+                    for (uint32_t c = 0; c < ncols; ++c) {
+                        CU_TRY(ctx, cudaMemcpyAsync(out_offsets[c] + p.pos, d_off[c], n_off * sizeof(uint64_t),
+                                                    cudaMemcpyDeviceToHost, ctx->stream));
+                        if (caps[c])
+                            CU_TRY(ctx, cudaMemcpyAsync(outs[c] + p.start[c], d_out[c], caps[c], cudaMemcpyDeviceToHost,
+                                                        ctx->stream));
+                    }
+                }
+                CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+                return CSVB200_OK;
+            }();
+        });
+        rc = first_error();
+    }
+    // every buffer goes back to the pool of the device it came from, on that device's stream
+    run_phase(m, [&](int k) {
+        cudaSetDevice(m->ctx[k]->device);
+        for (MatPiece& p : pieces) {
+            if (p.k != k) continue;
+            p.row_slots.reset();
+            p.row_bytes.reset();
+            for (uint32_t c = 0; c < ncols; ++c) {
+                p.d_off[c].reset();
+                p.d_out[c].reset();
+            }
+        }
+    });
+    cudaGetLastError();
+    if (rc) return rc;
+    if (small) return mfail(m, CSVB200_ERR_CAPACITY, "materialize destination too small");
+    if (!any) return CSVB200_OK;
+    if (!write) return mfail(m, CSVB200_ERR_INVALID_ARG, "null argument");
+    return CSVB200_OK;
+}

@@ -204,6 +204,7 @@ struct MaterializeParams {
     uint64_t out_cap;
     uint64_t* tile_desc;     // look-back descriptors (zeroed), materialize_scratch_bytes(nrec) - 128 bytes
     uint32_t* ticket;        // zeroed
+    uint64_t offset_base;    // added to every offset the offsets pass writes (0: offsets start at 0)
 };
 size_t materialize_scratch_bytes(uint32_t nrec);   // [128 B ticket cell][descriptors]
 
@@ -229,6 +230,7 @@ struct MaterializeMultiParams {
     uint64_t* tile_desc;              // [ncols][tiles] look-back descriptors (zeroed)
     uint32_t* ticket;                 // zeroed
     uint32_t tiles;
+    uint64_t offset_base[kMatMaxCols];   // per column, added to every offset the offsets pass writes
 };
 size_t materialize_multi_scratch_bytes(uint32_t nrec, uint32_t ncols);
 cudaError_t launch_materialize_multi_offsets(const MaterializeMultiParams& p, cudaStream_t stream);

@@ -304,7 +304,7 @@ __global__ void __launch_bounds__(kMatThreads) materialize_offsets_kernel(const 
     }
     if (tid == 0) s_prefix = lookback(p.tile_desc, tile, total);
     __syncthreads();
-    uint64_t off = s_prefix + wbase + (inc - tsum);
+    uint64_t off = p.offset_base + s_prefix + wbase + (inc - tsum);
 #pragma unroll
     for (int k = 0; k < kMatItems; ++k) {
         if (i0 + k < p.nrec) p.offsets[i0 + k] = off;
@@ -414,7 +414,7 @@ __global__ void __launch_bounds__(kMultiThreads) materialize_multi_offsets_kerne
     // one chain per column, thread c walks column c's: all the chains of the tile advance together in one warp
     // (a warp per chain with 128-descriptor hops measured slower here: 0.404 against 0.362 ms for 8 columns, 0.697
     // against 0.513 ms for 16 -- with 256-row tiles the walks are short and the chains queue up)
-    if (tid < p.ncols) s_base[tid] = lookback(p.tile_desc + (uint64_t)tid * p.tiles, tile, s_total[tid]);
+    if (tid < p.ncols) s_base[tid] = p.offset_base[tid] + lookback(p.tile_desc + (uint64_t)tid * p.tiles, tile, s_total[tid]);
     __syncthreads();
     for (uint32_t c = 0; c < p.ncols; ++c) {
         const uint64_t off = s_base[c] + s_len[c * kMultiThreads + tid];

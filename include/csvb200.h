@@ -281,6 +281,16 @@ int csvb200_multi_seek_records(csvb200_multi_index* mi, const uint32_t* rec, siz
 int csvb200_multi_seek_fields_device(csvb200_multi_index* mi, int k, const uint32_t* d_rec, const uint32_t* d_fld, size_t nq,
                                      csvb200_range* d_out);
 void* csvb200_multi_stream(csvb200_multi* m, int k);
+/* csvb200_materialize_columns over the distributed index, with the same results byte for byte and the same status
+ * codes, into host arrays; before csvb200_multi_tape_init it is CSVB200_ERR_INVALID_STATE.  Every device materialises
+ * the records whose index slots all lie in its segment, from its own shard of the bytes.  A record whose slots run
+ * over a cut (at most one per cut) has its slots and bytes copied to one device and goes through the same kernels
+ * there.  Offsets and values go straight from every device to their place in the caller's arrays.  An index of more
+ * than 2^32 entries is CSVB200_ERR_INVALID_ARG: the kernels address slots in u32, as the reference does. */
+int csvb200_multi_materialize_columns(csvb200_multi_index* mi, const uint32_t* fields, uint32_t ncols,
+                                      uint32_t first_record, uint32_t nrec, uint32_t flags,
+                                      uint64_t* const* out_offsets, uint8_t* const* outs,
+                                      const size_t* out_caps, size_t* out_lens);
 
 typedef struct csvb200_multi_stats {
     double seconds, upload_seconds, download_seconds;

@@ -534,6 +534,10 @@ class StructureIndex:
 
     @property
     def device_ptr(self) -> int:
+        """csvb200_index_device_ptr: the entries as u64 device memory, valid until free().  An index built by
+        index_build / index_build_device of at most 4 GiB holds 4-byte entries; the first call converts it in place
+        to u64 entries, once (one kernel, 12 bytes of device traffic per entry), and every later call returns the
+        same pointer."""
         return int(self._lib.csvb200_index_device_ptr(self._h) or 0)
 
     def to_host(self, out: np.ndarray | None = None) -> np.ndarray:

@@ -201,7 +201,16 @@ struct ReserveAll {
     }
 };
 
-// enqueue one build of idx->src[0..n) into idx->d_index (capacity idx->cap)
+// The storage decision, made here only: a build gets 4-byte entries (a compact index) when it is one piece -- one of the
+// two non-shard entry points, so no shard offset, exchange or carry from elsewhere -- of at most 4 GiB, whose largest
+// position n - 1 fits in 32 bits, and the context was not created with CSVB200_INDEX_ENTRY_BYTES=8.  The entries are then
+// the absolute positions themselves: widening one is a zero-extension.  Every other index holds u64 entries.
+uint32_t entry_bytes_for(const csvb200_ctx* ctx, size_t n, bool one_piece)
+{
+    return one_piece && ctx->compact_index && (uint64_t)n <= (1ull << 32) ? 4u : 8u;
+}
+
+// enqueue one build of idx->src[0..n) into idx->d_entries (capacity idx->cap)
 // redo = the conditional second launch of a speculative shard build (runs only if the carry prediction was wrong)
 int enqueue_build(csvb200_index* idx, bool timed, bool redo = false)
 {
@@ -210,7 +219,7 @@ int enqueue_build(csvb200_index* idx, bool timed, bool redo = false)
     const uint64_t num_tiles = (n + kTileBytes - 1) / kTileBytes;
     // an empty shard still runs one (empty) tile when its carry / result live on the device
     if (num_tiles == 0 && !(idx->d_shard_par || idx->d_result2 || idx->speculative)) {
-        if (idx->out_base == 1 && idx->cap > 0) CU_TRY(ctx, cudaMemsetAsync(idx->d_index, 0, 8, ctx->stream));  // sentinel alone
+        if (idx->out_base == 1 && idx->cap > 0) CU_TRY(ctx, cudaMemsetAsync(idx->d_entries, 0, idx->entry_bytes, ctx->stream));  // sentinel alone
         uint64_t* h_cell = ctx->h_cells + idx->cell * kCellWords;
         h_cell[0] = 0;
         h_cell[1] = idx->carry_parity;
@@ -218,7 +227,8 @@ int enqueue_build(csvb200_index* idx, bool timed, bool redo = false)
         BuildParams p{};
         p.in = idx->src;
         p.n = n;
-        p.index = idx->d_index;
+        p.index = idx->d_entries;
+        p.entry_bytes = idx->entry_bytes;
         p.cap = idx->cap;
         p.out_base = idx->out_base;
         p.pos_bias = idx->pos_bias;
@@ -326,7 +336,8 @@ int new_index(csvb200_ctx* ctx, csvb200_index** out)
 int build_device_common(csvb200_ctx* ctx, const void* dev_bytes, size_t n, uint32_t carry_parity, uint64_t pos_bias,
                         int emit_sentinel, csvb200_index** out, const uint32_t* d_shard_par = nullptr,
                         uint32_t shard_rank = 0, uint64_t* d_result2 = nullptr, bool speculative = false,
-                        uint64_t predict_window = 0, csvb200_exchange* ex = nullptr, bool validate = false)
+                        uint64_t predict_window = 0, csvb200_exchange* ex = nullptr, bool validate = false,
+                        bool one_piece = false)
 {
     if (!ctx || !out || (n && !dev_bytes)) return fail(ctx, CSVB200_ERR_INVALID_ARG, "null argument");
     if ((reinterpret_cast<uintptr_t>(dev_bytes) & 15u) != 0)
@@ -358,9 +369,10 @@ int build_device_common(csvb200_ctx* ctx, const void* dev_bytes, size_t n, uint3
         idx->speculative = true;
         idx->predict_window = predict_window ? predict_window : kDefaultPredictWindow;
     }
+    idx->entry_bytes = entry_bytes_for(ctx, n, one_piece && pos_bias == 0 && !ex && !speculative && !d_shard_par && !d_result2);
     idx->cap = initial_cap(ctx, n);
-    const size_t idx_bytes = idx->cap * sizeof(uint64_t);
-    cudaError_t e = pool_malloc((void**)&idx->d_index, idx_bytes, ctx->stream);
+    const size_t idx_bytes = idx->cap * idx->entry_bytes;
+    cudaError_t e = pool_malloc(&idx->d_entries, idx_bytes, ctx->stream);
     if (e != cudaSuccess) {
         cudaGetLastError();
         csvb200_index_free(idx);
@@ -507,6 +519,7 @@ int csvb200_ctx_create(int device, csvb200_ctx** out)
     }
     if (const char* t = std::getenv("CSVB200_TUNE")) ctx->tune = (uint32_t)std::atoi(t);
     ctx->dbg_timeline = std::getenv("CSVB200_DBG_TIMELINE") != nullptr;
+    if (const char* b = std::getenv("CSVB200_INDEX_ENTRY_BYTES")) ctx->compact_index = std::strcmp(b, "8") != 0;
     auto bail = [&](cudaError_t) {
         cudaGetLastError();
         csvb200_ctx_destroy(ctx);
@@ -659,7 +672,7 @@ int csvb200_index_build_device(csvb200_ctx* ctx, const void* dev_bytes, size_t n
     if (ctx && (flags & CSVB200_BUILD_STRICT_MIN64) && n < 64)
         return fail(ctx, CSVB200_ERR_INPUT_TOO_SMALL, "n < 64: the reference panics on this input");
     return build_device_common(ctx, dev_bytes, n, 0u, 0ull, 1, out, nullptr, 0, nullptr, false, 0, nullptr,
-                               (flags & CSVB200_BUILD_VALIDATE) != 0);
+                               (flags & CSVB200_BUILD_VALIDATE) != 0, true);
 }
 
 int csvb200_index_validation(csvb200_index* idx, int* is_ascii, uint64_t* newlines_outside_quotes)
@@ -802,7 +815,7 @@ int csvb200_index_build(csvb200_ctx* ctx, const uint8_t* host_bytes, size_t n, u
     int rc = upload(ctx, d_bytes.as<uint8_t>(), host_bytes, n);
     csvb200_index* idx = nullptr;
     if (!rc) rc = build_device_common(ctx, d_bytes.p, n, 0u, 0ull, 1, &idx, nullptr, 0, nullptr, false, 0, nullptr,
-                                      (flags & CSVB200_BUILD_VALIDATE) != 0);
+                                      (flags & CSVB200_BUILD_VALIDATE) != 0, true);
     if (!rc) rc = csvb200_index_sync(idx);  // resolves a capacity overflow while the bytes are still here
     if (rc) {
         if (idx) csvb200_index_free(idx);
@@ -1301,7 +1314,7 @@ int csvb200_index_wrap_device(csvb200_ctx* ctx, const uint64_t* d_entries, size_
     csvb200_index* idx = nullptr;
     int rc = new_index(ctx, &idx);
     if (rc) return rc;
-    idx->d_index = const_cast<uint64_t*>(d_entries);
+    idx->d_entries = const_cast<uint64_t*>(d_entries);
     idx->borrowed = true;
     idx->cap = idx->len = len;
     idx->n = input_bytes;
@@ -1337,10 +1350,10 @@ int csvb200_index_sync(csvb200_index* idx)
         }
         // capacity overflow (denser than the reserve heuristic): rebuild with the exact size
         if (!idx->src) return fail(ctx, CSVB200_ERR_INVALID_STATE, "index overflow and input no longer available");
-        CU_TRY(ctx, cudaFreeAsync(idx->d_index, ctx->stream));
-        idx->d_index = nullptr;
+        CU_TRY(ctx, cudaFreeAsync(idx->d_entries, ctx->stream));
+        idx->d_entries = nullptr;
         idx->cap = len + 2;
-        CU_TRY(ctx, pool_malloc((void**)&idx->d_index, idx->cap * sizeof(uint64_t), ctx->stream));
+        CU_TRY(ctx, pool_malloc(&idx->d_entries, idx->cap * idx->entry_bytes, ctx->stream));
         int rc = enqueue_build(idx, true);
         if (rc) return rc;
     }
@@ -1359,11 +1372,32 @@ int csvb200_index_end_parity(csvb200_index* idx)
     return idx->end_parity;
 }
 
+// A compact index turns into an ordinary u64 one, in place and once: whoever asks for raw u64 device memory gets an
+// index whose every later consumer takes the u64 path.
+static int widen_in_place(csvb200_index* idx)
+{
+    csvb200_ctx* ctx = idx->ctx;
+    CU_TRY(ctx, cudaSetDevice(ctx->device));
+    DevBuf wide;
+    CU_TRY(ctx, wide.alloc(idx->len * sizeof(uint64_t), ctx->stream));
+    CU_TRY(ctx, launch_widen_entries(static_cast<const uint32_t*>(idx->d_entries), idx->len, wide.as<uint64_t>(), ctx->stream));
+    ctx->launches += 1;
+    CU_TRY(ctx, cudaFreeAsync(idx->d_entries, ctx->stream));
+    idx->d_entries = wide.release();
+    idx->entry_bytes = 8;
+    idx->cap = idx->len;
+    CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    return CSVB200_OK;
+}
+
 const uint64_t* csvb200_index_device_ptr(csvb200_index* idx)
 {
     if (!idx || csvb200_index_sync(idx) != CSVB200_OK) return nullptr;
-    return idx->d_index;
+    if (idx->entry_bytes == 4 && widen_in_place(idx) != CSVB200_OK) return nullptr;
+    return static_cast<const uint64_t*>(idx->d_entries);
 }
+
+constexpr size_t kWidenChunk = 4u << 20;   // entries per widened chunk of a compact index on its way out (32 MiB as u64)
 
 int csvb200_index_copy_out(csvb200_index* idx, uint64_t* dst, size_t dst_cap)
 {
@@ -1372,8 +1406,39 @@ int csvb200_index_copy_out(csvb200_index* idx, uint64_t* dst, size_t dst_cap)
     if (rc) return rc;
     csvb200_ctx* ctx = idx->ctx;
     if (idx->len > dst_cap) return fail(ctx, CSVB200_ERR_CAPACITY, "destination index buffer too small");
-    CU_TRY(ctx, cudaMemcpyAsync(dst, idx->d_index, idx->len * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
-    CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    if (idx->entry_bytes == 8) {
+        CU_TRY(ctx, cudaMemcpyAsync(dst, idx->d_entries, idx->len * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
+        CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+        return CSVB200_OK;
+    }
+    // compact index: widened on the device, chunk by chunk, into two pooled buffers; the context's stream widens chunk
+    // k + 1 while its copy stream brings chunk k home (widening on the host would cost more than the copy, DESIGN 6)
+    CU_TRY(ctx, cudaSetDevice(ctx->device));
+    const size_t chunk = std::min(kWidenChunk, idx->len);
+    DevBuf wide;
+    CU_TRY(ctx, wide.alloc(2 * chunk * sizeof(uint64_t), ctx->stream));
+    cudaEvent_t widened = nullptr, copied[2] = {nullptr, nullptr};
+    cudaError_t e = cudaEventCreateWithFlags(&widened, cudaEventDisableTiming);
+    for (int b = 0; b < 2 && e == cudaSuccess; ++b) e = cudaEventCreateWithFlags(&copied[b], cudaEventDisableTiming);
+    const uint32_t* src = static_cast<const uint32_t*>(idx->d_entries);
+    for (size_t off = 0, k = 0; off < idx->len && e == cudaSuccess; off += chunk, ++k) {
+        const size_t len = std::min(chunk, idx->len - off);
+        uint64_t* buf = wide.as<uint64_t>() + (k & 1) * chunk;
+        if (k >= 2) e = cudaStreamWaitEvent(ctx->stream, copied[k & 1], 0);   // the copy of chunk k - 2 has left buf
+        if (e == cudaSuccess) e = launch_widen_entries(src + off, len, buf, ctx->stream);
+        if (e == cudaSuccess) ctx->launches += 1;
+        if (e == cudaSuccess) e = cudaEventRecord(widened, ctx->stream);
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->copy_stream, widened, 0);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(dst + off, buf, len * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->copy_stream);
+        if (e == cudaSuccess) e = cudaEventRecord(copied[k & 1], ctx->copy_stream);
+    }
+    // the buffers go back to the pool on ctx->stream: it must not run ahead of the last copy
+    const cudaError_t s = cudaStreamSynchronize(ctx->copy_stream);
+    if (e == cudaSuccess) e = s;
+    if (widened) cudaEventDestroy(widened);
+    for (cudaEvent_t ev : copied)
+        if (ev) cudaEventDestroy(ev);
+    CU_TRY(ctx, e);
     return CSVB200_OK;
 }
 
@@ -1382,7 +1447,7 @@ void csvb200_index_free(csvb200_index* idx)
     if (!idx) return;
     csvb200_ctx* ctx = idx->ctx;
     cudaSetDevice(ctx->device);
-    if (idx->d_index && !idx->borrowed) cudaFreeAsync(idx->d_index, ctx->stream);
+    if (idx->d_entries && !idx->borrowed) cudaFreeAsync(idx->d_entries, ctx->stream);
     if (idx->d_bytes_owned) cudaFreeAsync(idx->d_bytes_owned, ctx->stream);
     if (idx->d_nonascii) cudaFreeAsync(idx->d_nonascii, ctx->stream);
     if (idx->done) cudaEventDestroy(idx->done);
@@ -1431,7 +1496,8 @@ int csvb200_tape_validate(csvb200_index* idx, uint32_t field_cnt, int crlf, csvb
     uint64_t* h_cell = ctx->h_cells + cell * kCellWords;
     CU_TRY(ctx, cudaMemsetAsync(d_cell, 0xff, sizeof(uint64_t), ctx->stream));
     TapeValidateParams p{};
-    p.index = idx->d_index;
+    p.index = idx->d_entries;
+    p.entry_bytes = idx->entry_bytes;
     p.index_len = idx->len;
     p.bytes = bytes;
     p.n = idx->n;
@@ -1453,8 +1519,10 @@ int csvb200_tape_validate(csvb200_index* idx, uint32_t field_cnt, int crlf, csvb
     out->first_bad_pos = UINT64_MAX;
     if (out->first_bad_slot != UINT64_MAX) {
         out->first_bad_record = (out->first_bad_slot - 1) / j;
-        CU_TRY(ctx, cudaMemcpyAsync(&out->first_bad_pos, idx->d_index + out->first_bad_slot, sizeof(uint64_t),
-                                    cudaMemcpyDeviceToHost, ctx->stream));
+        out->first_bad_pos = 0;   // a u32 entry lands in the low half (little-endian host)
+        CU_TRY(ctx, cudaMemcpyAsync(&out->first_bad_pos,
+                                    static_cast<const uint8_t*>(idx->d_entries) + out->first_bad_slot * idx->entry_bytes,
+                                    idx->entry_bytes, cudaMemcpyDeviceToHost, ctx->stream));
         CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     } else if (out->problem != 0) {
         out->first_bad_record = (idx->len - 1) / j;      // the file ends inside this record
@@ -1499,7 +1567,8 @@ int csvb200_tape_chunks(csvb200_index* idx, uint8_t num, csvb200_chunk* out, siz
     CU_TRY(ctx, d_slots.alloc(slots.size() * 8, ctx->stream));
     CU_TRY(ctx, d_vals.alloc(slots.size() * 8, ctx->stream));
     CU_TRY(ctx, cudaMemcpyAsync(d_slots.p, slots.data(), slots.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
-    CU_TRY(ctx, launch_gather_slots(idx->d_index, idx->len, d_slots.as<uint64_t>(), slots.size(), d_vals.as<uint64_t>(), ctx->stream));
+    CU_TRY(ctx, launch_gather_slots(idx->d_entries, idx->entry_bytes, idx->len, d_slots.as<uint64_t>(), slots.size(),
+                                    d_vals.as<uint64_t>(), ctx->stream));
     ctx->launches += 1;
     CU_TRY(ctx, cudaMemcpyAsync(vals.data(), d_vals.p, slots.size() * 8, cudaMemcpyDeviceToHost, ctx->stream));
     CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
@@ -1515,7 +1584,8 @@ static int seek_device(csvb200_index* idx, const uint32_t* d_rec, const uint32_t
 {
     csvb200_ctx* ctx = idx->ctx;
     LookupParams p{};
-    p.index = idx->d_index;
+    p.index = idx->d_entries;
+    p.entry_bytes = idx->entry_bytes;
     p.index_len = idx->len;
     p.record_cnt = idx->record_cnt;
     p.field_cnt = idx->field_cnt;
@@ -1758,6 +1828,7 @@ static int materialize_enqueue(csvb200_ctx* ctx, const MatSource& src, uint32_t 
 {
     MaterializeParams p{};
     p.index = src.index;
+    p.entry_bytes = src.entry_bytes;
     p.index_len = src.index_len;
     p.bytes = src.bytes;
     p.n = src.n;
@@ -1803,8 +1874,8 @@ static int materialize_prepare(csvb200_index* idx, uint32_t flags)
 
 static MatSource source_of(const csvb200_index* idx)
 {
-    return MatSource{idx->d_index, idx->len, idx->d_bytes_owned ? idx->d_bytes_owned : idx->src, idx->n, idx->pos_bias,
-                     idx->record_cnt, idx->field_cnt, (uint32_t)idx->jump};
+    return MatSource{idx->d_entries, idx->len, idx->d_bytes_owned ? idx->d_bytes_owned : idx->src, idx->n, idx->pos_bias,
+                     idx->record_cnt, idx->field_cnt, (uint32_t)idx->jump, idx->entry_bytes};
 }
 
 }  // extern "C"
@@ -1822,6 +1893,7 @@ int materialize_multi_enqueue(csvb200_ctx* ctx, const MatSource& src, const uint
                                    out_caps ? out_caps[0] : 0, offset_base ? offset_base[0] : 0, offsets_pass, write_pass);
     MaterializeMultiParams p{};
     p.index = src.index;
+    p.entry_bytes = src.entry_bytes;
     p.index_len = src.index_len;
     p.bytes = src.bytes;
     p.n = src.n;
@@ -2063,8 +2135,8 @@ int csvb200_index_load(csvb200_ctx* ctx, const char* path, csvb200_index** out)
     int rc = new_index(ctx, &idx);
     if (rc) return rc;
     idx->cap = host.size();
-    cudaError_t e = pool_malloc((void**)&idx->d_index, idx->cap * sizeof(uint64_t), ctx->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(idx->d_index, host.data(), host.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream);
+    cudaError_t e = pool_malloc(&idx->d_entries, idx->cap * sizeof(uint64_t), ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(idx->d_entries, host.data(), host.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     if (e != cudaSuccess) {
         cudaGetLastError();

@@ -55,6 +55,7 @@ struct csvb200_ctx {
     uint8_t* h_small_in = nullptr;             // pinned, device-mapped staging of the small-input fast path (build_to_host_small)
     uint64_t* h_small_out = nullptr;
     bool dbg_timeline = false;                 // CSVB200_DBG_TIMELINE: device-resident builds run the instrumented kernel
+    bool compact_index = true;                 // CSVB200_INDEX_ENTRY_BYTES=8 clears it: every index keeps u64 entries
     uint64_t* d_dbg = nullptr;                 // ... and leave 8 words per super-tile here
     size_t dbg_words = 0;
     int io_threads = 0;                        // slices per pool; 0 = default_io_threads() (csvb200_multi_create divides them over its devices)
@@ -93,7 +94,10 @@ struct csvb200_exchange {
 
 struct csvb200_index {
     csvb200_ctx* ctx = nullptr;
-    uint64_t* d_index = nullptr;
+    // the entries: u64, or the u32 absolute positions of a compact index (one-piece device-resident builds of at most
+    // 4 GiB, see compact_entries in api.cu); cap and len count entries, not bytes
+    void* d_entries = nullptr;
+    uint32_t entry_bytes = 8;
     size_t cap = 0;
     size_t len = 0;
     int end_parity = 0;
@@ -124,7 +128,7 @@ struct csvb200_index {
     size_t carry_cell = SIZE_MAX;
     uint64_t predict_window = 0;
     uint8_t* d_bytes_owned = nullptr;
-    bool borrowed = false;                  // d_index belongs to the caller (csvb200_index_wrap_device): never freed here
+    bool borrowed = false;                  // d_entries belongs to the caller (csvb200_index_wrap_device): never freed here
     // Tape metadata (TapeCore::init)
     bool tape_ready = false;
     uint32_t field_cnt = 0, record_cnt = 0;
@@ -221,11 +225,12 @@ int ensure_bounce(csvb200_ctx* ctx);
 // What the materialisation launches read: the index addressed by global slot (index[s] for s < index_len), the bytes
 // the positions point into (bytes[0] is global byte pos_bias, n of them) and the tape metadata.
 struct MatSource {
-    const uint64_t* index;
+    const void* index;
     uint64_t index_len;
     const uint8_t* bytes;
     uint64_t n, pos_bias;
     uint32_t record_cnt, field_cnt, row_size;
+    uint32_t entry_bytes = 8;   // 4: the u32 entries of a compact index (one-GPU indexes only)
 };
 // Enqueues the offsets pass (lengths + scan into d_offsets, offset_base[c] added to column c's; offset_base may be null)
 // and / or the write pass of `ncols` columns on the context's stream; one column goes to the single-column kernels.

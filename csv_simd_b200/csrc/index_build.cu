@@ -1,6 +1,6 @@
 // index_build.cu -- fused single-pass CSV structural index build for sm_100a.
 //
-// Replaces, in ONE kernel and one pass over the input (traffic = N + 8E):
+// Replaces, in ONE kernel and one pass over the input (traffic = N + 8E; N + 4E for a compact index):
 //   reader::read            src/reader.rs:150-306      (64-byte block loop, tail padding, carries)
 //   SimdInput::structure    src/avx/stage1.rs:193-407  (classify, bit-pack, clmul prefix-XOR, carry, mask)
 //   Stage1::crush_set_bits  src/stage1.rs:162-296      (tzcnt/blsr extraction into the growing Vec<usize>)
@@ -51,6 +51,8 @@ struct __align__(1024) Smem {
     uint64_t base;
 };
 
+// E: the entry type, u64 or the u32 of a compact index (positions below 2^32: the sums are exact in 32 bits)
+template <class E>
 __global__ void __launch_bounds__(kThreads, 3) index_build_kernel(const BuildParams p)
 {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -222,7 +224,7 @@ __global__ void __launch_bounds__(kThreads, 3) index_build_kernel(const BuildPar
             if (tile == p.num_tiles - 1) {
                 write_result(p, cend, pend);
             }
-            if (tile == 0u && p.write_sentinel && p.cap > 0) p.index[0] = 0ull;
+            if (tile == 0u && p.write_sentinel && p.cap > 0) static_cast<E*>(p.index)[0] = 0u;
             if (p.total_out != nullptr && (o0 | o1) != 0u) atomicAdd(p.total_out, (unsigned long long)(o0 + o1));
             if (p.validate) {
                 const uint32_t nl = pin ? nl_b : nl_a;
@@ -262,18 +264,18 @@ __global__ void __launch_bounds__(kThreads, 3) index_build_kernel(const BuildPar
     }
     __syncthreads();
     {
-        const uint64_t tile_pos = p.pos_bias + tile_off;
-        if (head && tid == 0 && cnt > 0 && g0 < p.cap) p.index[g0] = tile_pos + sm.stage[1];
+        const E tile_pos = (E)(p.pos_bias + tile_off);
+        if (head && tid == 0 && cnt > 0 && g0 < p.cap) static_cast<E*>(p.index)[g0] = tile_pos + sm.stage[1];
         // staging index j = i + head is even for every pair, and g = g0 - head + j is even too
         const uint32_t end = cnt + head;
         const uint64_t gbase = g0 - head;
-        uint64_t* out = p.index + gbase;
+        E* out = static_cast<E*>(p.index) + gbase;
         if (gbase + end <= p.cap) {
             // common case: the whole run fits; full 16-byte stores except possibly the last entry
             const uint32_t end2 = end & ~1u;
             for (uint32_t j = 2u * head + 2u * tid; j < end2; j += 2u * kThreads) {
                 const uint32_t pr = *reinterpret_cast<const uint32_t*>(&sm.stage[j]);
-                stg_128(out + j, tile_pos + (pr & 0xffffu), tile_pos + (pr >> 16));
+                stg_pair(out + j, tile_pos + (E)(pr & 0xffffu), tile_pos + (E)(pr >> 16));
             }
             if ((end & 1u) && tid == 0 && end > 2u * head) out[end - 1] = tile_pos + sm.stage[end - 1];
         } else {
@@ -484,22 +486,27 @@ __global__ void class_bytes_kernel(const uint8_t* __restrict__ in, uint64_t n, u
 cudaError_t launch_index_build(const BuildParams& p, cudaStream_t stream)
 {
     if (p.num_tiles == 0) return cudaSuccess;
+    const int compact = p.entry_bytes == 4 ? 1 : 0;
     // the opt-in to > 48 KiB of dynamic shared memory is per (kernel, device): cached per device ordinal
     static std::mutex mu;
-    static bool configured[64] = {};
+    static bool configured[2][64] = {};   // [compact]
     int dev = 0;
     cudaError_t e = cudaGetDevice(&dev);
     if (e != cudaSuccess) return e;
     if (dev < 0 || dev >= 64) return cudaErrorInvalidDevice;
     {
         std::lock_guard<std::mutex> lock(mu);
-        if (!configured[dev]) {
-            e = cudaFuncSetAttribute(index_build_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
+        if (!configured[compact][dev]) {
+            e = cudaFuncSetAttribute(compact ? index_build_kernel<uint32_t> : index_build_kernel<uint64_t>,
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
             if (e != cudaSuccess) return e;
-            configured[dev] = true;
+            configured[compact][dev] = true;
         }
     }
-    index_build_kernel<<<p.num_tiles, kThreads, sizeof(Smem), stream>>>(p);
+    if (compact)
+        index_build_kernel<uint32_t><<<p.num_tiles, kThreads, sizeof(Smem), stream>>>(p);
+    else
+        index_build_kernel<uint64_t><<<p.num_tiles, kThreads, sizeof(Smem), stream>>>(p);
     return cudaGetLastError();
 }
 

@@ -177,12 +177,14 @@ template <class S>
 __device__ __forceinline__ void worker_barrier() { asm volatile("bar.sync 1, %0;" ::"n"(S::kWorkerThreads) : "memory"); }
 
 // streams staged entries [j0, j1) (staging indices, j0 even) of a run whose staging index 0 maps to
-// global slot gbase; positions are tile_pos + 16-bit offset
-template <class S>
+// global slot gbase; positions are tile_pos + 16-bit offset, stored as E (u64, or u32 for a compact index, whose
+// positions are below 2^32: the sums are exact in 32 bits)
+template <class S, class E>
 __device__ __forceinline__ void copy_out_range(const BuildParams& p, const uint16_t* stg, uint32_t local0, uint32_t j0,
-                                               uint32_t j1, uint64_t gbase, uint64_t tile_pos, uint32_t tid)
+                                               uint32_t j1, uint64_t gbase, uint64_t tile_pos_, uint32_t tid)
 {
-    uint64_t* out = p.index + gbase;
+    E* out = static_cast<E*>(p.index) + gbase;
+    const E tile_pos = (E)tile_pos_;
     if (gbase + j1 <= p.cap) {
         const uint32_t j1e = j1 & ~1u;
         // (Splitting tile_pos into a shared high word and one 32-bit add per entry halves this loop's instructions
@@ -190,7 +192,7 @@ __device__ __forceinline__ void copy_out_range(const BuildParams& p, const uint1
         //  collide with the TMA reads; the paced version interleaves better with them.)
         for (uint32_t j = j0 + 2u * tid; j < j1e; j += 2u * S::kWorkerThreads) {
             const uint32_t pr = *reinterpret_cast<const uint32_t*>(&stg[j - local0]);
-            stg_128(out + j, tile_pos + (pr & 0xffffu), tile_pos + (pr >> 16));
+            stg_pair(out + j, tile_pos + (E)(pr & 0xffffu), tile_pos + (E)(pr >> 16));
         }
         if ((j1 & 1u) && tid == 0 && j1 > j0) out[j1 - 1] = tile_pos + stg[j1 - 1 - local0];
     } else {
@@ -214,7 +216,7 @@ struct SuperRegs {
 // Ordered compaction of one sub-tile: expand the masks into 16-bit offsets in shared memory at the
 // scanned slots, then stream the run out as 16-byte stores.  `seq` numbers the sub-tile compactions
 // of this CTA (it alternates the staging buffer when there are two).
-template <class S>
+template <class S, class E>
 __device__ __forceinline__ void compact_sub(SmemTma<S>& sm, const BuildParams& p, const TileRegs& t, const PrefixInfo<S::kSub, S::kWorkers>& pi,
                                             int sub, uint32_t super_tile, uint32_t seq, uint32_t tid, uint32_t warp)
 {
@@ -271,8 +273,8 @@ __device__ __forceinline__ void compact_sub(SmemTma<S>& sm, const BuildParams& p
             if (c & 1u) *dst++ = (uint16_t)(rel0 + (uint32_t)__ffs((int)m) - 1u);
         }
         worker_barrier<S>();
-        if (head && tid == 0 && cnt > 0 && g0 < p.cap) p.index[g0] = tile_pos + stg[1];
-        copy_out_range<S>(p, stg, 0u, 2u * head, end, gbase, tile_pos, tid);
+        if (head && tid == 0 && cnt > 0 && g0 < p.cap) static_cast<E*>(p.index)[g0] = (E)tile_pos + stg[1];
+        copy_out_range<S, E>(p, stg, 0u, 2u * head, end, gbase, tile_pos, tid);
         // no trailing barrier: see above
     } else {
         // dense sub-tile (more than kStageCap entries): several staging rounds
@@ -290,8 +292,8 @@ __device__ __forceinline__ void compact_sub(SmemTma<S>& sm, const BuildParams& p
             }
             worker_barrier<S>();
             const uint32_t r1 = min(end, r0 + kCap);
-            if (r0 == 0 && head && tid == 0 && cnt > 0 && g0 < p.cap) p.index[g0] = tile_pos + stg[1];
-            copy_out_range<S>(p, stg, r0, r0 == 0 ? 2u * head : r0, r1, gbase, tile_pos, tid);
+            if (r0 == 0 && head && tid == 0 && cnt > 0 && g0 < p.cap) static_cast<E*>(p.index)[g0] = (E)tile_pos + stg[1];
+            copy_out_range<S, E>(p, stg, r0, r0 == 0 ? 2u * head : r0, r1, gbase, tile_pos, tid);
             worker_barrier<S>();
         }
     }
@@ -312,7 +314,7 @@ __device__ __forceinline__ uint64_t dbg_globaltimer()
 
 // compaction of the `it`-th super-tile this CTA processed; every warp arrives on the producer's `go` barrier after the
 // first sub-tile's compaction (see the producer)
-template <class S, bool kDbg = false>
+template <class S, class E, bool kDbg = false>
 __device__ __forceinline__ void compact_super(SmemTma<S>& sm, const BuildParams& p, const SuperRegs<S::kSub>& t, uint32_t it,
                                               uint32_t tid, uint32_t warp)
 {
@@ -323,15 +325,16 @@ __device__ __forceinline__ void compact_super(SmemTma<S>& sm, const BuildParams&
     const PrefixInfo<S::kSub, S::kWorkers>& pi = sm.pref[pb];
 #pragma unroll
     for (int sub = 0; sub < S::kSub; ++sub) {
-        compact_sub<S>(sm, p, t.sub[sub], pi, sub, t.tile, it * S::kSub + sub, tid, warp);
+        compact_sub<S, E>(sm, p, t.sub[sub], pi, sub, t.tile, it * S::kSub + sub, tid, warp);
         if (sub == 0 && (tid & 31u) == 0u) mbar_arrive(&sm.go);
     }
 }
 
 // kVal: CSVB200_BUILD_VALIDATE by-products; kEx: the cross-GPU exchange in the epilogue of the last CTA.  Both are
 // compile-time so that the plain build keeps the register allocation it was tuned with (with the exchange code merely
-// present the 64-register shape measured 0.401 instead of 0.391 ms on cfg2).
-template <class S, bool kVal, bool kEx, bool kDbg = false>
+// present the 64-register shape measured 0.401 instead of 0.391 ms on cfg2).  E: the entry type, u64 or the u32 of a
+// compact index.
+template <class S, bool kVal, bool kEx, bool kDbg = false, class E = uint64_t>
 __global__ void __launch_bounds__(S::kThreadsAll, S::kMinBlocks)
 index_build_tma_kernel(const BuildParams p, const __grid_constant__ CUtensorMap tmap)
 {
@@ -481,7 +484,7 @@ index_build_tma_kernel(const BuildParams p, const __grid_constant__ CUtensorMap 
                     pi.cnt[sub] = (uint32_t)(b1 - b0);
                 }
                 if (tile == p.num_tiles - 1) write_result(p, cend, pend);
-                if (tile == 0u && p.write_sentinel && p.cap > 0) p.index[0] = 0ull;
+                if (tile == 0u && p.write_sentinel && p.cap > 0) static_cast<E*>(p.index)[0] = 0u;
                 cta_total += (uint64_t)(o0 + o1);
                 if (kVal) {
                     cta_nl += pin ? nl_b : nl_a;
@@ -620,13 +623,13 @@ index_build_tma_kernel(const BuildParams p, const __grid_constant__ CUtensorMap 
                 // no skew: the tile just classified is compacted at once (the other CTAs of the SM cover the look-back);
                 // nothing outlives an iteration, which frees the registers the pending masks take
                 if (cur.tile == kInvalidTile) break;
-                compact_super<S, kDbg>(sm, p, cur, it, tid, warp);
+                compact_super<S, E, kDbg>(sm, p, cur, it, tid, warp);
                 continue;
             }
             // ---- ordered compaction of the super-tile classified kSkew iterations ago: its look-back has
             //      had kSkew classify phases to complete ----
             if (pend[0].tile != kInvalidTile)
-                compact_super<S, kDbg>(sm, p, pend[0], it - kSkew, tid, warp);
+                compact_super<S, E, kDbg>(sm, p, pend[0], it - kSkew, tid, warp);
             else if (lane == 0u)
                 mbar_arrive(&sm.go);   // nothing to compact yet: the producer may draw the next ticket at once
             if (cur.tile == kInvalidTile) {
@@ -634,7 +637,7 @@ index_build_tma_kernel(const BuildParams p, const __grid_constant__ CUtensorMap 
                 // `go` complete phases nobody waits for)
 #pragma unroll
                 for (int k = 1; k < kSkew; ++k)
-                    if (pend[k].tile != kInvalidTile) compact_super<S, kDbg>(sm, p, pend[k], it - kSkew + k, tid, warp);
+                    if (pend[k].tile != kInvalidTile) compact_super<S, E, kDbg>(sm, p, pend[k], it - kSkew + k, tid, warp);
                 break;
             }
 #pragma unroll
@@ -675,7 +678,7 @@ struct ShapeState {
     int grid_cap[kMaxDevices] = {};
 };
 
-template <class S, bool kVal = false, bool kEx = false, bool kDbg = false>
+template <class S, bool kVal = false, bool kEx = false, bool kDbg = false, class E = uint64_t>
 cudaError_t launch_shape(const BuildParams& p_in, cudaStream_t stream)
 {
     static ShapeState state;
@@ -702,14 +705,14 @@ cudaError_t launch_shape(const BuildParams& p_in, cudaStream_t stream)
     {
         std::lock_guard<std::mutex> lock(state.mu);
         if (state.grid_cap[dev] == 0) {
-            e = cudaFuncSetAttribute(index_build_tma_kernel<S, kVal, kEx, kDbg>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+            e = cudaFuncSetAttribute(index_build_tma_kernel<S, kVal, kEx, kDbg, E>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                      (int)sizeof(SmemTma<S>));
             if (e != cudaSuccess) return e;
-            cudaFuncSetAttribute(index_build_tma_kernel<S, kVal, kEx, kDbg>, cudaFuncAttributePreferredSharedMemoryCarveout,
+            cudaFuncSetAttribute(index_build_tma_kernel<S, kVal, kEx, kDbg, E>, cudaFuncAttributePreferredSharedMemoryCarveout,
                                  cudaSharedmemCarveoutMaxShared);
             int sms = 148, per_sm = 0;
             cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-            e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, index_build_tma_kernel<S, kVal, kEx, kDbg>, S::kThreadsAll,
+            e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, index_build_tma_kernel<S, kVal, kEx, kDbg, E>, S::kThreadsAll,
                                                               sizeof(SmemTma<S>));
             if (e != cudaSuccess) return e;
             if (per_sm < 1) return cudaErrorLaunchOutOfResources;
@@ -728,7 +731,7 @@ cudaError_t launch_shape(const BuildParams& p_in, cudaStream_t stream)
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = p.pdl_wait ? 1u : 0u;
-    return cudaLaunchKernelEx(&cfg, index_build_tma_kernel<S, kVal, kEx, kDbg>, p, tmap);
+    return cudaLaunchKernelEx(&cfg, index_build_tma_kernel<S, kVal, kEx, kDbg, E>, p, tmap);
 }
 
 }  // namespace
@@ -737,6 +740,12 @@ uint64_t build_flag_tile_bytes(bool use_tma) { return use_tma ? (uint64_t)ShapeB
 
 cudaError_t launch_index_build_tma(const BuildParams& p, cudaStream_t stream)
 {
+    if (p.entry_bytes == 4) {   // compact index: device-resident one-piece builds only, never the exchange
+        if (p.ex.peers) return cudaErrorInvalidValue;
+        if (p.validate) return launch_shape<ShapeB, true, false, false, uint32_t>(p, stream);
+        if (p.dbg) return launch_shape<ShapeB, false, false, true, uint32_t>(p, stream);
+        return launch_shape<ShapeB, false, false, false, uint32_t>(p, stream);
+    }
     if (p.validate) return p.ex.peers ? launch_shape<ShapeB, true, true>(p, stream) : launch_shape<ShapeB, true, false>(p, stream);
     if (p.ex.peers) return launch_shape<ShapeB, false, true>(p, stream);
     if (p.dbg) return launch_shape<ShapeB, false, false, true>(p, stream);   // timeline instrumentation (tools/timeline.py)

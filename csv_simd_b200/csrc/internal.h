@@ -60,8 +60,8 @@ struct ExchangeArgs {
 struct BuildParams {
     const uint8_t* in;       // 16-byte aligned device pointer to the shard's bytes
     uint64_t n;              // bytes
-    uint64_t* index;         // output entries (u64, == Rust usize); 16-byte aligned
-    uint64_t cap;            // number of u64 slots available at `index`
+    void* index;             // output entries, entry_bytes each; 16-byte aligned
+    uint64_t cap;            // number of entry slots available at `index`
     uint64_t out_base;       // slot of the first entry produced by the virtual predecessor (1 after the sentinel)
     uint64_t pos_bias;       // added to every emitted byte position (global offset of the shard)
     const uint64_t* carry;   // optional device cell {entries so far, parity}; overrides the two below
@@ -105,6 +105,9 @@ struct BuildParams {
     unsigned long long* nl_out;
     uint32_t* hi_out;
     uint32_t* nonascii_bitmap;
+    // 8: u64 entries (== Rust usize); 4: u32 entries of a compact index (the absolute positions of a build with
+    // pos_bias == 0 and n <= 2^32).  0 reads as 8.
+    uint32_t entry_bytes;
 };
 
 // one tile per CTA, plain loads: small inputs and cross-check of the TMA kernel
@@ -135,11 +138,12 @@ cudaError_t launch_class_bytes(const uint8_t* in, uint64_t n, uint8_t* out, cuda
 
 // K4 batched lookups. ranges[2*i] = start, ranges[2*i+1] = end; (UINT64_MAX, UINT64_MAX) = None.
 struct LookupParams {
-    const uint64_t* index;
+    const void* index;       // entry_bytes per entry (8, or 4 for a compact index); the sharded form reads u64 only
     uint64_t index_len;
     uint32_t record_cnt;
     uint32_t field_cnt;
     uint32_t row_size;       // jump: field_cnt (+1 for CRLF)
+    uint32_t entry_bytes;    // (fills the hole before `rec`: the sharded kernel's parameter layout stays as it was)
     const uint32_t* rec;
     const uint32_t* fld;     // nullptr => seek_record
     uint64_t nq;
@@ -165,7 +169,7 @@ cudaError_t launch_range_lengths(const uint64_t* ranges, uint64_t nq, uint64_t* 
 
 // K5 tape validation (tape.cu): first index slot whose separator class does not fit its place in the record
 struct TapeValidateParams {
-    const uint64_t* index;
+    const void* index;       // entry_bytes per entry
     uint64_t index_len;
     const uint8_t* bytes;    // the shard the index positions refer to
     uint64_t n;
@@ -173,11 +177,14 @@ struct TapeValidateParams {
     uint64_t jump;
     int crlf;
     uint64_t* first_bad_slot;   // device word, preset to UINT64_MAX; atomicMin
+    uint32_t entry_bytes;
 };
 cudaError_t launch_tape_validate(const TapeValidateParams& p, cudaStream_t stream);
-// out[i] = index[slots[i]] (UINT64_MAX when the slot is past the end)
-cudaError_t launch_gather_slots(const uint64_t* index, uint64_t index_len, const uint64_t* slots, uint64_t n,
-                                uint64_t* out, cudaStream_t stream);
+// out[i] = index[slots[i]] (UINT64_MAX when the slot is past the end); entry_bytes per index entry
+cudaError_t launch_gather_slots(const void* index, uint32_t entry_bytes, uint64_t index_len, const uint64_t* slots,
+                                uint64_t n, uint64_t* out, cudaStream_t stream);
+// out[i] = in[i] for i < n: the u32 entries of a compact index as u64 (in and out 16-byte aligned)
+cudaError_t launch_widen_entries(const uint32_t* in, uint64_t n, uint64_t* out, cudaStream_t stream);
 
 // K7 ASCII / UTF-8 validation (validate.cu): result[0] (preset UINT64_MAX) <- start of the first ill-formed
 // sequence, result[1] (preset 0) <- 1 when any byte is >= 0x80
@@ -191,7 +198,7 @@ uint64_t build_flag_tile_bytes(bool use_tma);
 
 // K6 column materialisation (materialize.cu)
 struct MaterializeParams {
-    const uint64_t* index;
+    const void* index;       // entry_bytes per entry
     uint64_t index_len;
     const uint8_t* bytes;
     uint64_t n;
@@ -205,6 +212,7 @@ struct MaterializeParams {
     uint64_t* tile_desc;     // look-back descriptors (zeroed), materialize_scratch_bytes(nrec) - 128 bytes
     uint32_t* ticket;        // zeroed
     uint64_t offset_base;    // added to every offset the offsets pass writes (0: offsets start at 0)
+    uint32_t entry_bytes;
 };
 size_t materialize_scratch_bytes(uint32_t nrec);   // [128 B ticket cell][descriptors]
 
@@ -214,7 +222,7 @@ size_t materialize_scratch_bytes(uint32_t nrec);   // [128 B ticket cell][descri
 constexpr uint32_t kMatMaxCols = 32;
 constexpr int kMultiThreads = 256;   // threads per CTA of the multi-column kernels = records per tile
 struct MaterializeMultiParams {
-    const uint64_t* index;
+    const void* index;                // entry_bytes per entry
     uint64_t index_len;
     const uint8_t* bytes;
     uint64_t n;
@@ -231,11 +239,28 @@ struct MaterializeMultiParams {
     uint32_t* ticket;                 // zeroed
     uint32_t tiles;
     uint64_t offset_base[kMatMaxCols];   // per column, added to every offset the offsets pass writes
+    uint32_t entry_bytes;
 };
 size_t materialize_multi_scratch_bytes(uint32_t nrec, uint32_t ncols);
 cudaError_t launch_materialize_multi_offsets(const MaterializeMultiParams& p, cudaStream_t stream);
 cudaError_t launch_materialize_multi_write(const MaterializeMultiParams& p, cudaStream_t stream);
 cudaError_t launch_materialize_offsets(const MaterializeParams& p, cudaStream_t stream);
 cudaError_t launch_materialize_write(const MaterializeParams& p, cudaStream_t stream);
+
+#ifdef __CUDACC__
+// One index entry, read through the non-coherent path: a u64 entry, or a u32 entry of a compact index zero-extended.
+__device__ __forceinline__ uint64_t ldg_entry(const uint64_t* p)
+{
+    uint64_t v;
+    asm volatile("ld.global.nc.u64 %0, [%1];" : "=l"(v) : "l"(p));
+    return v;
+}
+__device__ __forceinline__ uint64_t ldg_entry(const uint32_t* p)
+{
+    uint32_t v;
+    asm volatile("ld.global.nc.u32 %0, [%1];" : "=r"(v) : "l"(p));
+    return v;
+}
+#endif
 
 }  // namespace csvb200

@@ -19,15 +19,11 @@ namespace csvb200 {
 
 namespace {
 
-__device__ __forceinline__ uint64_t ldg_u64(const uint64_t* p)
-{
-    uint64_t v;
-    asm volatile("ld.global.nc.u64 %0, [%1];" : "=l"(v) : "l"(p));
-    return v;
-}
-
+// E: the entry type, u64 or the u32 of a compact index
+template <class E>
 __global__ void __launch_bounds__(256) seek_kernel(const LookupParams p)
 {
+    const E* __restrict__ index = static_cast<const E*>(p.index);
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
     for (uint64_t q = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; q < p.nq; q += stride) {
         const uint32_t r = p.rec[q];
@@ -46,8 +42,8 @@ __global__ void __launch_bounds__(256) seek_kernel(const LookupParams p)
         }
         if (live) {
             if (e_slot < p.index_len) {
-                start = ldg_u64(p.index + s) + 1;
-                end = ldg_u64(p.index + e_slot);
+                start = ldg_entry(index + s) + 1;
+                end = ldg_entry(index + e_slot);
             } else {
                 atomicAdd(p.oob, 1u);
             }
@@ -64,7 +60,7 @@ __device__ __forceinline__ uint64_t sharded_entry(const SegmentTable& seg, uint6
 #pragma unroll
     for (uint32_t j = 1; j < kExMaxWorld; ++j)
         if (j < seg.nseg && s >= seg.base[j]) k = j;
-    return ldg_u64(seg.ptr[k] + (s - seg.base[k]));
+    return ldg_entry(seg.ptr[k] + (s - seg.base[k]));
 }
 
 __global__ void __launch_bounds__(256) seek_sharded_kernel(const LookupParams p, const SegmentTable seg)
@@ -139,7 +135,10 @@ cudaError_t launch_seek(const LookupParams& p, cudaStream_t stream)
     uint64_t blocks = (p.nq + 255) / 256;
     const uint64_t max_blocks = (uint64_t)sms * 32;
     if (blocks > max_blocks) blocks = max_blocks;
-    seek_kernel<<<(unsigned)blocks, 256, 0, stream>>>(p);
+    if (p.entry_bytes == 4)
+        seek_kernel<uint32_t><<<(unsigned)blocks, 256, 0, stream>>>(p);
+    else
+        seek_kernel<uint64_t><<<(unsigned)blocks, 256, 0, stream>>>(p);
     return cudaGetLastError();
 }
 

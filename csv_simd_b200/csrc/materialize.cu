@@ -20,12 +20,6 @@ constexpr int kMatItems = 4;
 constexpr int kMatTile = kMatThreads * kMatItems;
 constexpr uint64_t kMatAgg = 1ull << 62, kMatPrefix = 2ull << 62, kMatMask = (1ull << 62) - 1;
 
-__device__ __forceinline__ uint64_t ldg_u64(const uint64_t* p)
-{
-    uint64_t v;
-    asm volatile("ld.global.nc.u64 %0, [%1];" : "=l"(v) : "l"(p));
-    return v;
-}
 __device__ __forceinline__ uint64_t ld_relaxed(const uint64_t* p)
 {
     uint64_t v;
@@ -59,37 +53,42 @@ __device__ __forceinline__ uint64_t lookback(uint64_t* desc, uint32_t tile, uint
     return prefix;
 }
 
-// what the per-value helpers need of either parameter block
+// what the per-value helpers need of either parameter block; E: the entry type, u64 or the u32 of a compact index
+template <class E>
 struct FieldView {
-    const uint64_t* index;
+    const E* index;
     uint64_t index_len;
     const uint8_t* bytes;
     uint64_t n, pos_bias;
     uint32_t record_cnt, field_cnt, row_size, field_idx, flags;
 };
-__device__ __forceinline__ FieldView view_of(const MaterializeParams& p)
+template <class E>
+__device__ __forceinline__ FieldView<E> view_of(const MaterializeParams& p)
 {
-    return FieldView{p.index, p.index_len, p.bytes, p.n, p.pos_bias, p.record_cnt, p.field_cnt, p.row_size, p.field_idx, p.flags};
+    return FieldView<E>{static_cast<const E*>(p.index), p.index_len, p.bytes, p.n, p.pos_bias, p.record_cnt, p.field_cnt, p.row_size, p.field_idx, p.flags};
 }
-__device__ __forceinline__ FieldView view_of(const MaterializeMultiParams& p, uint32_t c)
+template <class E>
+__device__ __forceinline__ FieldView<E> view_of(const MaterializeMultiParams& p, uint32_t c)
 {
-    return FieldView{p.index, p.index_len, p.bytes, p.n, p.pos_bias, p.record_cnt, p.field_cnt, p.row_size, p.field_idx[c], p.flags};
+    return FieldView<E>{static_cast<const E*>(p.index), p.index_len, p.bytes, p.n, p.pos_bias, p.record_cnt, p.field_cnt, p.row_size, p.field_idx[c], p.flags};
 }
 
 // seek_field (src/record_source.rs:104-140) as byte offsets relative to p.bytes; false = Ok(None) or a
 // slot the reference would panic on
-__device__ __forceinline__ bool field_range(const FieldView& p, uint32_t r, uint64_t& a, uint64_t& b)
+template <class E>
+__device__ __forceinline__ bool field_range(const FieldView<E>& p, uint32_t r, uint64_t& a, uint64_t& b)
 {
     if ((uint32_t)(r + 1u) >= p.record_cnt || p.field_idx >= p.field_cnt) return false;
     const uint32_t s = (uint32_t)(r + 1u) * p.row_size + p.field_idx;   // u32 arithmetic, as the reference
     if ((uint64_t)s + 1 >= p.index_len) return false;
-    a = ldg_u64(p.index + s) + 1 - p.pos_bias;
-    b = ldg_u64(p.index + s + 1) - p.pos_bias;
+    a = ldg_entry(p.index + s) + 1 - p.pos_bias;
+    b = ldg_entry(p.index + s + 1) - p.pos_bias;
     return a <= b && b <= p.n;
 }
 
 // trims [a, b) in place and reports whether the value is a quoted field to unquote
-__device__ __forceinline__ bool trim_and_test(const FieldView& p, uint64_t& a, uint64_t& b)
+template <class E>
+__device__ __forceinline__ bool trim_and_test(const FieldView<E>& p, uint64_t& a, uint64_t& b)
 {
     const uint8_t* x = p.bytes;
     if (p.flags & 2u) {
@@ -167,7 +166,8 @@ struct Unquoter {
 };
 
 // length of the value made of the raw slice [a, b)
-__device__ __forceinline__ uint64_t value_len_range(const FieldView& p, uint64_t a, uint64_t b)
+template <class E>
+__device__ __forceinline__ uint64_t value_len_range(const FieldView<E>& p, uint64_t a, uint64_t b)
 {
     if (!trim_and_test(p, a, b)) return b - a;
     uint64_t o = 0;
@@ -178,7 +178,8 @@ __device__ __forceinline__ uint64_t value_len_range(const FieldView& p, uint64_t
     return o;
 }
 
-__device__ __forceinline__ uint64_t value_len(const FieldView& p, uint32_t r)
+template <class E>
+__device__ __forceinline__ uint64_t value_len(const FieldView<E>& p, uint32_t r)
 {
     uint64_t a, b;
     if (!field_range(p, r, a, b)) return 0;
@@ -187,8 +188,8 @@ __device__ __forceinline__ uint64_t value_len(const FieldView& p, uint32_t r)
 
 // put(byte) for every byte of the value made of the raw slice [a, b); x is the caller's restrict-qualified copy of
 // p.bytes (without it every byte load has to wait for the previous byte store)
-template <class Put>
-__device__ __forceinline__ void emit_value(const FieldView& p, const uint8_t* __restrict__ x, uint64_t a, uint64_t b, Put put)
+template <class E, class Put>
+__device__ __forceinline__ void emit_value(const FieldView<E>& p, const uint8_t* __restrict__ x, uint64_t a, uint64_t b, Put put)
 {
     if (!trim_and_test(p, a, b)) {
         if (b - a < 16) {   // short raw values: a handful of byte loads beat 16 predicated steps per chunk
@@ -225,8 +226,8 @@ struct RangeBatch {
     uint32_t ok, plain, quoted;   // quoted bit k: not padded, both ends are quotes: the value is the unquoted [a + 1, b - 1)
 };
 // item(k, rec, fld) -> does item k exist, and which (record, field) it is
-template <int kB, class Item>
-__device__ __forceinline__ void range_batch_load(const FieldView& p, Item item, RangeBatch<kB>& rb)
+template <int kB, class E, class Item>
+__device__ __forceinline__ void range_batch_load(const FieldView<E>& p, Item item, RangeBatch<kB>& rb)
 {
     rb.ok = rb.plain = rb.quoted = 0;
 #pragma unroll
@@ -237,8 +238,8 @@ __device__ __forceinline__ void range_batch_load(const FieldView& p, Item item, 
         if ((uint32_t)(r + 1u) >= p.record_cnt || f >= p.field_cnt) continue;
         const uint32_t s = (uint32_t)(r + 1u) * p.row_size + f;   // u32 arithmetic, as the reference
         if ((uint64_t)s + 1 >= p.index_len) continue;
-        rb.a[k] = ldg_u64(p.index + s);
-        rb.b[k] = ldg_u64(p.index + s + 1);
+        rb.a[k] = ldg_entry(p.index + s);
+        rb.b[k] = ldg_entry(p.index + s + 1);
         rb.ok |= 1u << k;
     }
 #pragma unroll
@@ -271,6 +272,7 @@ __device__ __forceinline__ void range_batch_load(const FieldView& p, Item item, 
     }
 }
 
+template <class E>
 __global__ void __launch_bounds__(kMatThreads) materialize_offsets_kernel(const MaterializeParams p)
 {
     __shared__ uint64_t s_warp[kMatThreads / 32];
@@ -284,7 +286,7 @@ __global__ void __launch_bounds__(kMatThreads) materialize_offsets_kernel(const 
     uint64_t len[kMatItems], tsum = 0;
 #pragma unroll
     for (int k = 0; k < kMatItems; ++k) {
-        len[k] = i0 + k < p.nrec ? value_len(view_of(p), p.first_record + (uint32_t)(i0 + k)) : 0;
+        len[k] = i0 + k < p.nrec ? value_len(view_of<E>(p), p.first_record + (uint32_t)(i0 + k)) : 0;
         tsum += len[k];
     }
     // block exclusive scan of the thread sums
@@ -313,6 +315,7 @@ __global__ void __launch_bounds__(kMatThreads) materialize_offsets_kernel(const 
     if (i0 < p.nrec && i0 + kMatItems >= p.nrec) p.offsets[p.nrec] = off;   // the thread owning the last record
 }
 
+template <class E>
 __global__ void __launch_bounds__(kMatThreads) materialize_write_kernel(const MaterializeParams p)
 {
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
@@ -320,7 +323,7 @@ __global__ void __launch_bounds__(kMatThreads) materialize_write_kernel(const Ma
     // (the compiler must assume out aliases bytes), which serialises the copy into load -> store round trips
     const uint8_t* __restrict__ x = p.bytes;
     uint8_t* __restrict__ out = p.out;
-    const FieldView fv = view_of(p);
+    const FieldView<E> fv = view_of<E>(p);
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < p.nrec; i += stride) {
         uint64_t a, b;
         if (!field_range(fv, p.first_record + (uint32_t)i, a, b)) continue;
@@ -339,9 +342,10 @@ __global__ void __launch_bounds__(kMatThreads) materialize_write_kernel(const Ma
 // A row sweep (tiles of 32-128 records staged through shared memory) was built, measured against these kernels and
 // removed: it won on quoted columns and lost on unquoted ones (DESIGN 4.8, profiles/r02_mat_sweep_ab.jsonl).
 using ColBatch = RangeBatch<kColBatch>;
+template <class E>
 __device__ __forceinline__ void col_batch_load(const MaterializeMultiParams& p, uint32_t r, uint32_t c0, bool row_live, ColBatch& cb)
 {
-    range_batch_load(view_of(p, 0), [&](int k, uint32_t& rec, uint32_t& fld) {
+    range_batch_load(view_of<E>(p, 0), [&](int k, uint32_t& rec, uint32_t& fld) {
         const uint32_t c = c0 + (uint32_t)k;
         if (!row_live || c >= p.ncols) return false;
         rec = r;
@@ -350,7 +354,7 @@ __device__ __forceinline__ void col_batch_load(const MaterializeMultiParams& p, 
     }, cb);
 }
 
-template <bool kBatched>   // separate kernels: the batched form needs 64 registers, the plain one 32
+template <bool kBatched, class E>   // separate kernels: the batched form needs 64 registers, the plain one 32
 __global__ void __launch_bounds__(kMultiThreads) materialize_multi_offsets_kernel(const MaterializeMultiParams p)
 {
     extern __shared__ uint32_t s_len[];                    // [ncols][256] lengths, then exclusive prefixes in place
@@ -364,10 +368,10 @@ __global__ void __launch_bounds__(kMultiThreads) materialize_multi_offsets_kerne
     // fewer than kColBatchMin columns: one value after the other (the batches cost registers: 4 columns 1.86 -> 2.01 ms
     // unquoted, 3.01 -> 3.29 ms quoted, where 8 / 16 unquoted columns go 3.43 -> 2.96 ms and 6.83 -> 4.74 ms)
     for (uint32_t c = 0; !kBatched && c < p.ncols; ++c)
-        s_len[c * kMultiThreads + tid] = i < p.nrec ? (uint32_t)value_len(view_of(p, c), p.first_record + (uint32_t)i) : 0u;
+        s_len[c * kMultiThreads + tid] = i < p.nrec ? (uint32_t)value_len(view_of<E>(p, c), p.first_record + (uint32_t)i) : 0u;
     for (uint32_t c0 = 0; kBatched && c0 < p.ncols; c0 += kColBatch) {
         ColBatch cb;
-        col_batch_load(p, p.first_record + (uint32_t)i, c0, i < p.nrec, cb);
+        col_batch_load<E>(p, p.first_record + (uint32_t)i, c0, i < p.nrec, cb);
 #pragma unroll
         for (int k = 0; k < kColBatch; ++k) {
             const uint32_t c = c0 + (uint32_t)k;
@@ -383,7 +387,7 @@ __global__ void __launch_bounds__(kMultiThreads) materialize_multi_offsets_kerne
                 u.finish();
                 len = o;
             } else if (cb.ok >> k & 1u)
-                len = (uint32_t)value_len_range(view_of(p, c), cb.a[k], cb.b[k]);          // padded: trim first
+                len = (uint32_t)value_len_range(view_of<E>(p, c), cb.a[k], cb.b[k]);          // padded: trim first
             s_len[c * kMultiThreads + tid] = len;
         }
     }
@@ -423,14 +427,14 @@ __global__ void __launch_bounds__(kMultiThreads) materialize_multi_offsets_kerne
     }
 }
 
-template <bool kBatched>
+template <bool kBatched, class E>
 __global__ void __launch_bounds__(kMultiThreads) materialize_multi_write_kernel(const MaterializeMultiParams p)
 {
     const uint8_t* __restrict__ x = p.bytes;
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= p.nrec) return;
     for (uint32_t c = 0; !kBatched && c < p.ncols; ++c) {
-        const FieldView fv = view_of(p, c);
+        const FieldView<E> fv = view_of<E>(p, c);
         uint8_t* __restrict__ out = p.out[c];
         uint64_t a, b;
         if (!field_range(fv, p.first_record + (uint32_t)i, a, b)) continue;
@@ -440,7 +444,7 @@ __global__ void __launch_bounds__(kMultiThreads) materialize_multi_write_kernel(
     }
     for (uint32_t c0 = 0; kBatched && c0 < p.ncols; c0 += kColBatch) {
         ColBatch cb;
-        col_batch_load(p, p.first_record + (uint32_t)i, c0, true, cb);
+        col_batch_load<E>(p, p.first_record + (uint32_t)i, c0, true, cb);
         uint64_t o[kColBatch], o_end[kColBatch];
 #pragma unroll
         for (int k = 0; k < kColBatch; ++k) {
@@ -473,7 +477,7 @@ __global__ void __launch_bounds__(kMultiThreads) materialize_multi_write_kernel(
                 u.finish();
                 continue;
             }
-            emit_value(view_of(p, c), x, a, b, put);   // padded: trim first
+            emit_value(view_of<E>(p, c), x, a, b, put);   // padded: trim first
         }
     }
 }
@@ -490,10 +494,15 @@ cudaError_t launch_materialize_multi_offsets(const MaterializeMultiParams& p, cu
 {
     if (p.tiles == 0 || p.ncols == 0) return cudaSuccess;
     const size_t smem = (size_t)p.ncols * kMultiThreads * sizeof(uint32_t);
-    if (p.ncols >= kColBatchMin)
-        materialize_multi_offsets_kernel<true><<<p.tiles, kMultiThreads, smem, stream>>>(p);
+    const bool batched = p.ncols >= kColBatchMin, compact = p.entry_bytes == 4;
+    if (batched && compact)
+        materialize_multi_offsets_kernel<true, uint32_t><<<p.tiles, kMultiThreads, smem, stream>>>(p);
+    else if (batched)
+        materialize_multi_offsets_kernel<true, uint64_t><<<p.tiles, kMultiThreads, smem, stream>>>(p);
+    else if (compact)
+        materialize_multi_offsets_kernel<false, uint32_t><<<p.tiles, kMultiThreads, smem, stream>>>(p);
     else
-        materialize_multi_offsets_kernel<false><<<p.tiles, kMultiThreads, smem, stream>>>(p);
+        materialize_multi_offsets_kernel<false, uint64_t><<<p.tiles, kMultiThreads, smem, stream>>>(p);
     return cudaGetLastError();
 }
 
@@ -501,10 +510,15 @@ cudaError_t launch_materialize_multi_write(const MaterializeMultiParams& p, cuda
 {
     if (p.nrec == 0 || p.ncols == 0) return cudaSuccess;
     const unsigned blocks = (p.nrec + kMultiThreads - 1) / kMultiThreads;
-    if (p.ncols >= kColBatchMin)
-        materialize_multi_write_kernel<true><<<blocks, kMultiThreads, 0, stream>>>(p);
+    const bool batched = p.ncols >= kColBatchMin, compact = p.entry_bytes == 4;
+    if (batched && compact)
+        materialize_multi_write_kernel<true, uint32_t><<<blocks, kMultiThreads, 0, stream>>>(p);
+    else if (batched)
+        materialize_multi_write_kernel<true, uint64_t><<<blocks, kMultiThreads, 0, stream>>>(p);
+    else if (compact)
+        materialize_multi_write_kernel<false, uint32_t><<<blocks, kMultiThreads, 0, stream>>>(p);
     else
-        materialize_multi_write_kernel<false><<<blocks, kMultiThreads, 0, stream>>>(p);
+        materialize_multi_write_kernel<false, uint64_t><<<blocks, kMultiThreads, 0, stream>>>(p);
     return cudaGetLastError();
 }
 
@@ -514,7 +528,10 @@ cudaError_t launch_materialize_offsets(const MaterializeParams& p, cudaStream_t 
 {
     const uint32_t tiles = (p.nrec + kMatTile - 1) / kMatTile;
     if (tiles == 0) return cudaSuccess;
-    materialize_offsets_kernel<<<tiles, kMatThreads, 0, stream>>>(p);
+    if (p.entry_bytes == 4)
+        materialize_offsets_kernel<uint32_t><<<tiles, kMatThreads, 0, stream>>>(p);
+    else
+        materialize_offsets_kernel<uint64_t><<<tiles, kMatThreads, 0, stream>>>(p);
     return cudaGetLastError();
 }
 
@@ -527,7 +544,10 @@ cudaError_t launch_materialize_write(const MaterializeParams& p, cudaStream_t st
     uint64_t blocks = ((uint64_t)p.nrec + kMatThreads - 1) / kMatThreads;
     const uint64_t max_blocks = (uint64_t)sms * 16;
     if (blocks > max_blocks) blocks = max_blocks;
-    materialize_write_kernel<<<(unsigned)blocks, kMatThreads, 0, stream>>>(p);
+    if (p.entry_bytes == 4)
+        materialize_write_kernel<uint32_t><<<(unsigned)blocks, kMatThreads, 0, stream>>>(p);
+    else
+        materialize_write_kernel<uint64_t><<<(unsigned)blocks, kMatThreads, 0, stream>>>(p);
     return cudaGetLastError();
 }
 

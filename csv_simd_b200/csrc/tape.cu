@@ -8,25 +8,20 @@
 //   LF files   (jump = field_cnt)     : ',' for k < jump-1, CR or LF for k = jump-1
 //   CRLF files (jump = field_cnt + 1) : ',' for k < jump-2, CR for k = jump-2, LF right after it for k = jump-1
 // and reports the FIRST slot that is not (atomicMin), i.e. the first bad record.  HBM-bound: reads the
-// index once (8E bytes) and one byte per entry of the input (every 32-byte sector of a dense file: N).
+// index once (8E bytes, 4E for a compact index) and one byte per entry of the input (every 32-byte sector of a dense
+// file: N).
 #include "internal.h"
 
 namespace csvb200 {
 
 namespace {
 
-__device__ __forceinline__ uint64_t ldg_u64(const uint64_t* p)
-{
-    uint64_t v;
-    asm volatile("ld.global.nc.u64 %0, [%1];" : "=l"(v) : "l"(p));
-    return v;
-}
-
 // One row of 32 slots per warp step.  Everything that does not depend on the slot is hoisted: CRLF / LF is a
 // template parameter, k = (s - 1) % jump lives in 32 bits and advances by 32 % jump, and the only 64-bit
 // work left per slot is the position arithmetic (the first version spent ~100 instructions per slot row on
-// 64-bit modulo / select chains and was issue-bound at 0.55 of the HBM peak).
-template <bool kCrlf>
+// 64-bit modulo / select chains and was issue-bound at 0.55 of the HBM peak).  E: the entry type, u64 or the u32 of a
+// compact index.
+template <bool kCrlf, class E>
 __global__ void __launch_bounds__(256) tape_validate_kernel(const TapeValidateParams p)
 {
     const uint32_t lane = threadIdx.x & 31u;
@@ -36,7 +31,7 @@ __global__ void __launch_bounds__(256) tape_validate_kernel(const TapeValidatePa
     const uint32_t nl0 = jump - (kCrlf ? 2u : 1u);    // first line-end slot of a row (k >= nl0 is CR / LF territory)
     const uint64_t last = p.index_len - 1;            // slots are 1 .. last; i = s - 1 in [0, last)
     const uint32_t step = 32u % jump;                 // k advances by 32 slots per warp row
-    const uint64_t* __restrict__ index = p.index + 1; // index[i] here is slot s = i + 1
+    const E* __restrict__ index = static_cast<const E*>(p.index) + 1;   // index[i] here is slot s = i + 1
     uint64_t bad = UINT64_MAX;                        // smallest failing i
     constexpr int kUnroll = 4;
     constexpr uint64_t kRun = 32 * 16;
@@ -49,7 +44,7 @@ __global__ void __launch_bounds__(256) tape_validate_kernel(const TapeValidatePa
 #pragma unroll
             for (int u = 0; u < kUnroll; ++u) {
                 const uint64_t iu = i + 32ull * u;
-                pos[u] = iu < run_end ? ldg_u64(index + iu) : UINT64_MAX;   // UINT64_MAX - bias >= n: treated as skipped below
+                pos[u] = iu < run_end ? ldg_entry(index + iu) : UINT64_MAX;   // UINT64_MAX - bias >= n: treated as skipped below
                 kk[u] = k;
                 k += step;
                 k = k >= jump ? k - jump : k;
@@ -72,7 +67,7 @@ __global__ void __launch_bounds__(256) tape_validate_kernel(const TapeValidatePa
                 } else if (kk[u] == nl0) {
                     ok = b == 0x0Du;
                 } else {
-                    ok = b == 0x0Au && ldg_u64(index + iu - 1) + 1 == pos[u];   // the LF directly after its CR
+                    ok = b == 0x0Au && ldg_entry(index + iu - 1) + 1 == pos[u];   // the LF directly after its CR
                 }
                 if (!ok && iu < bad) bad = iu;
             }
@@ -88,20 +83,54 @@ __global__ void __launch_bounds__(256) tape_validate_kernel(const TapeValidatePa
         atomicMin(reinterpret_cast<unsigned long long*>(p.first_bad_slot), (unsigned long long)(bad + 1));
 }
 
-__global__ void gather_slots_kernel(const uint64_t* __restrict__ index, uint64_t index_len,
+template <class E>
+__global__ void gather_slots_kernel(const E* __restrict__ index, uint64_t index_len,
                                     const uint64_t* __restrict__ slots, uint64_t n, uint64_t* __restrict__ out)
 {
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) out[i] = slots[i] < index_len ? index[slots[i]] : UINT64_MAX;
+    if (i < n) out[i] = slots[i] < index_len ? (uint64_t)index[slots[i]] : UINT64_MAX;
+}
+
+// four entries per thread and trip: one 16-byte load, two 16-byte stores (12 bytes of traffic per entry)
+__global__ void __launch_bounds__(256) widen_entries_kernel(const uint32_t* __restrict__ in, uint64_t n,
+                                                            uint64_t* __restrict__ out)
+{
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const uint64_t n4 = n / 4;
+    for (uint64_t i = t; i < n4; i += stride) {
+        const uint4 v = reinterpret_cast<const uint4*>(in)[i];
+        reinterpret_cast<ulonglong2*>(out)[2 * i] = make_ulonglong2(v.x, v.y);
+        reinterpret_cast<ulonglong2*>(out)[2 * i + 1] = make_ulonglong2(v.z, v.w);
+    }
+    for (uint64_t i = 4 * n4 + t; i < n; i += stride) out[i] = in[i];
 }
 
 }  // namespace
 
-cudaError_t launch_gather_slots(const uint64_t* index, uint64_t index_len, const uint64_t* slots, uint64_t n,
-                                uint64_t* out, cudaStream_t stream)
+cudaError_t launch_gather_slots(const void* index, uint32_t entry_bytes, uint64_t index_len, const uint64_t* slots,
+                                uint64_t n, uint64_t* out, cudaStream_t stream)
 {
     if (n == 0) return cudaSuccess;
-    gather_slots_kernel<<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(index, index_len, slots, n, out);
+    const unsigned blocks = (unsigned)((n + 127) / 128);
+    if (entry_bytes == 4)
+        gather_slots_kernel<<<blocks, 128, 0, stream>>>(static_cast<const uint32_t*>(index), index_len, slots, n, out);
+    else
+        gather_slots_kernel<<<blocks, 128, 0, stream>>>(static_cast<const uint64_t*>(index), index_len, slots, n, out);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_widen_entries(const uint32_t* in, uint64_t n, uint64_t* out, cudaStream_t stream)
+{
+    if (n == 0) return cudaSuccess;
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    uint64_t blocks = (n / 4 + 255) / 256;
+    const uint64_t max_blocks = (uint64_t)sms * 8;
+    if (blocks > max_blocks) blocks = max_blocks;
+    if (blocks == 0) blocks = 1;
+    widen_entries_kernel<<<(unsigned)blocks, 256, 0, stream>>>(in, n, out);
     return cudaGetLastError();
 }
 
@@ -116,10 +145,15 @@ cudaError_t launch_tape_validate(const TapeValidateParams& p, cudaStream_t strea
     if (blocks > max_blocks) blocks = max_blocks;
     if (blocks == 0) blocks = 1;
     if (p.jump > 0xffffffffull) return cudaErrorInvalidValue;
-    if (p.crlf)
-        tape_validate_kernel<true><<<(unsigned)blocks, 256, 0, stream>>>(p);
+    const bool compact = p.entry_bytes == 4;
+    if (p.crlf && compact)
+        tape_validate_kernel<true, uint32_t><<<(unsigned)blocks, 256, 0, stream>>>(p);
+    else if (p.crlf)
+        tape_validate_kernel<true, uint64_t><<<(unsigned)blocks, 256, 0, stream>>>(p);
+    else if (compact)
+        tape_validate_kernel<false, uint32_t><<<(unsigned)blocks, 256, 0, stream>>>(p);
     else
-        tape_validate_kernel<false><<<(unsigned)blocks, 256, 0, stream>>>(p);
+        tape_validate_kernel<false, uint64_t><<<(unsigned)blocks, 256, 0, stream>>>(p);
     return cudaGetLastError();
 }
 

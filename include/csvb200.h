@@ -310,6 +310,12 @@ int csvb200_index_wrap_device(csvb200_ctx* ctx, const uint64_t* d_entries, size_
 int csvb200_index_sync(csvb200_index* idx);
 size_t csvb200_index_len(csvb200_index* idx);          /* entries incl. the sentinel if emitted */
 int csvb200_index_end_parity(csvb200_index* idx);      /* quote parity after the last byte */
+/* The entries as u64 device memory, valid until csvb200_index_free.  An index built by csvb200_index_build or
+ * csvb200_index_build_device over at most 4 GiB of input is stored with 4-byte entries (the positions fit in 32 bits;
+ * every other call of this header reads them natively and csvb200_index_copy_out widens them on the way out).  The
+ * first call of this function converts such an index in place, once: one extra kernel and 12 bytes of device traffic
+ * per entry, and it synchronises the context's stream.  From then on it is an ordinary 8-byte index and every call
+ * returns the same pointer.  CSVB200_INDEX_ENTRY_BYTES=8 at context creation keeps 8-byte entries throughout. */
 const uint64_t* csvb200_index_device_ptr(csvb200_index* idx);
 int csvb200_index_copy_out(csvb200_index* idx, uint64_t* dst, size_t dst_cap); /* fills a caller Vec<usize> */
 void csvb200_index_free(csvb200_index* idx);

@@ -119,6 +119,9 @@ SIGNATURES = {
     "csvb200_multi_stream": (C.c_void_p, [C.c_void_p, C.c_int]),
     "csvb200_multi_materialize_columns": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32,
                                                     vpp, vpp, szp, szp]),
+    "csvb200_multi_tape_validate": (C.c_int, [C.c_void_p, C.c_uint32, C.c_int, C.POINTER(TapeReport)]),
+    "csvb200_multi_validate_utf8": (C.c_int, [C.c_void_p, u64p, C.POINTER(C.c_int)]),
+    "csvb200_multi_tape_chunks": (C.c_int, [C.c_void_p, C.c_uint8, C.POINTER(Chunk), C.c_size_t, szp]),
     "csvb200_index_wrap_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.c_void_p, vpp]),
     "csvb200_index_sync": (C.c_int, [C.c_void_p]),
     "csvb200_index_len": (C.c_size_t, [C.c_void_p]),

@@ -483,6 +483,26 @@ class MultiIndex:
                                                                     p_off, p_out, caps, lens))
         return list(zip(offs, vals))
 
+    def tape_validate(self, field_cnt: int, crlf: bool) -> dict:
+        """csvb200_multi_tape_validate: as StructureIndex.tape_validate, every device checking its own segment."""
+        rep = _lib.TapeReport()
+        self._check(self._lib.csvb200_multi_tape_validate(self._h, field_cnt, int(crlf), C.byref(rep)))
+        return {k: int(getattr(rep, k)) for k, _ in _lib.TapeReport._fields_}
+
+    def tape_chunks(self, num: int):
+        """csvb200_multi_tape_chunks: as StructureIndex.tape_chunks, the byte ranges read from the owning segments."""
+        arr = (_lib.Chunk * 256)()
+        n = C.c_size_t()
+        self._check(self._lib.csvb200_multi_tape_chunks(self._h, num & 0xFF, arr, 256, C.byref(n)))
+        return [{k: int(getattr(arr[i], k)) for k, _ in _lib.Chunk._fields_} for i in range(n.value)]
+
+    def validate_utf8(self):
+        """csvb200_multi_validate_utf8: as Context.validate_utf8 on the whole input, every device judging its own shard
+        -> (valid_up_to or None when well-formed UTF-8, is_ascii)."""
+        v, asc = C.c_uint64(), C.c_int()
+        self._check(self._lib.csvb200_multi_validate_utf8(self._h, C.byref(v), C.byref(asc)))
+        return (None if v.value == 0xFFFFFFFFFFFFFFFF else v.value), bool(asc.value)
+
     def seek_fields_device(self, k: int, d_rec: int, d_fld: int, nq: int, d_out: int):
         self._check(self._lib.csvb200_multi_seek_fields_device(self._h, k, C.c_void_p(d_rec), C.c_void_p(d_fld), nq,
                                                                C.c_void_p(d_out)))

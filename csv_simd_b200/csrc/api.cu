@@ -1531,6 +1531,42 @@ int csvb200_tape_validate(csvb200_index* idx, uint32_t field_cnt, int crlf, csvb
     return CSVB200_OK;
 }
 
+}  // extern "C"
+
+namespace csvb200 {
+
+int tape_chunk_slots(uint32_t record_cnt, uint64_t jump, uint8_t num, csvb200_chunk* out, size_t out_cap, size_t* n_out)
+{
+    // boundaries(record_cnt, num) (src/tape.rs:385-428); None -> StructureError::InvalidState (:99-100)
+    const uint32_t task = record_cnt;
+    if (task == 0 || num == 0) return CSVB200_ERR_INVALID_STATE;
+    const size_t nchunks = task < num ? 1 : num;
+    *n_out = nchunks;
+    if (!out || out_cap < nchunks) return CSVB200_ERR_CAPACITY;
+    const uint32_t job = task < num ? task : task / num, rem = task < num ? 0 : task % num;
+    uint64_t acc = 0;
+    for (size_t i = 0; i < nchunks; ++i) {
+        const uint32_t len = job + (i < rem ? 1u : 0u);
+        out[i].id = (uint8_t)i;
+        out[i].start = acc * jump;                            // KeyToPos(boundary.start * jump) (:104-106)
+        out[i].end = (acc + len) * jump;                      // (:107-110)
+        out[i].record_cnt = len;
+        acc += len;
+    }
+    out[0].start = jump;                                      // chunk 0 skips the header row (:117-123)
+    out[0].record_cnt -= 1;
+    return CSVB200_OK;
+}
+
+const char* tape_chunk_error(int code)
+{
+    return code == CSVB200_ERR_CAPACITY ? "chunk array too small" : csvb200_status_string(code);
+}
+
+}  // namespace csvb200
+
+extern "C" {
+
 int csvb200_tape_chunks(csvb200_index* idx, uint8_t num, csvb200_chunk* out, size_t out_cap, size_t* n_out)
 {
     if (!idx || !n_out) return CSVB200_ERR_INVALID_ARG;
@@ -1538,24 +1574,9 @@ int csvb200_tape_chunks(csvb200_index* idx, uint8_t num, csvb200_chunk* out, siz
     if (rc) return rc;
     csvb200_ctx* ctx = idx->ctx;
     if (!idx->tape_ready) return fail(ctx, CSVB200_ERR_INVALID_STATE, "csvb200_tape_init has not been called");
-    // boundaries(record_cnt, num) (src/tape.rs:385-428); None -> StructureError::InvalidState (:99-100)
-    const uint32_t task = idx->record_cnt;
-    if (task == 0 || num == 0) return fail(ctx, CSVB200_ERR_INVALID_STATE, csvb200_status_string(CSVB200_ERR_INVALID_STATE));
-    const size_t nchunks = task < num ? 1 : num;
-    *n_out = nchunks;
-    if (!out || out_cap < nchunks) return fail(ctx, CSVB200_ERR_CAPACITY, "chunk array too small");
-    const uint32_t job = task < num ? task : task / num, rem = task < num ? 0 : task % num;
-    uint64_t acc = 0;
-    for (size_t i = 0; i < nchunks; ++i) {
-        const uint32_t len = job + (i < rem ? 1u : 0u);
-        out[i].id = (uint8_t)i;
-        out[i].start = acc * idx->jump;                       // KeyToPos(boundary.start * jump) (:104-106)
-        out[i].end = (acc + len) * idx->jump;                 // (:107-110)
-        out[i].record_cnt = len;
-        acc += len;
-    }
-    out[0].start = idx->jump;                                 // chunk 0 skips the header row (:117-123)
-    out[0].record_cnt -= 1;
+    rc = tape_chunk_slots(idx->record_cnt, idx->jump, num, out, out_cap, n_out);
+    if (rc) return fail(ctx, rc, tape_chunk_error(rc));
+    const size_t nchunks = *n_out;
     // byte ranges the chunks delimit: two index entries per chunk, fetched in one small gather
     CU_TRY(ctx, cudaSetDevice(ctx->device));
     std::vector<uint64_t> slots(2 * nchunks), vals(2 * nchunks, UINT64_MAX);

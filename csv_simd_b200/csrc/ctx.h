@@ -238,6 +238,11 @@ int materialize_multi_enqueue(csvb200_ctx* ctx, const MatSource& src, const uint
                               uint32_t first_record, uint32_t nrec, uint32_t flags, uint64_t* const* d_offsets,
                               uint8_t* const* d_outs, const size_t* out_caps, const uint64_t* offset_base, bool offsets_pass,
                               bool write_pass);
+// The slots of Tape::chunks(num) (src/tape.rs:95-140) over boundaries(record_cnt, num): every field of out[0 .. *n_out)
+// but byte_start / byte_end.  CSVB200_ERR_INVALID_STATE when record_cnt or num is 0, CSVB200_ERR_CAPACITY (with *n_out
+// set) when out_cap is short; tape_chunk_error gives the message the chunk calls report with either.
+int tape_chunk_slots(uint32_t record_cnt, uint64_t jump, uint8_t num, csvb200_chunk* out, size_t out_cap, size_t* n_out);
+const char* tape_chunk_error(int code);
 // host-side wait for all ranks' rows of one build (exchange.cu)
 int exchange_wait_all(csvb200_exchange* ex, uint64_t epoch, uint64_t* counts, uint32_t* carries);
 

@@ -19,6 +19,7 @@
 #include "ctx.h"
 #include "record_split.h"
 #include "slice_pool.h"
+#include "utf8_halo.h"
 
 using namespace csvb200;
 
@@ -857,3 +858,212 @@ extern "C" int csvb200_multi_materialize_columns(csvb200_multi_index* mi, const 
     if (!write) return mfail(m, CSVB200_ERR_INVALID_ARG, "null argument");
     return CSVB200_OK;
 }
+
+// ---------------------------------------------------------------------------------------------------------------
+// tape validation, UTF-8 validation and chunks over the distributed index: every device checks its own segment and
+// shard in place with the one-GPU kernels, and the host joins the answers across the cuts
+// ---------------------------------------------------------------------------------------------------------------
+namespace {
+
+// the entry of global slot s (< the index length), copied from the device whose segment holds it
+int read_entry(csvb200_multi_index* mi, uint64_t s, uint64_t* out)
+{
+    const uint32_t j = segment_of(mi->base.data(), (uint32_t)mi->seg.size(), s);
+    csvb200_ctx* ctx = mi->m->ctx[j];
+    CU_TRY(ctx, cudaSetDevice(ctx->device));
+    CU_TRY(ctx, cudaMemcpyAsync(out, mi->table.ptr[j] + (s - mi->base[j]), sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    return CSVB200_OK;
+}
+
+int first_device_error(csvb200_multi* m, const std::vector<int>& rcs)
+{
+    for (size_t k = 0; k < rcs.size(); ++k)
+        if (rcs[k]) return mfail(m, rcs[k], "device " + std::to_string(k) + ": " + csvb200_last_error(m->ctx[k]));
+    return CSVB200_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int csvb200_multi_tape_validate(csvb200_multi_index* mi, uint32_t field_cnt, int crlf, csvb200_tape_report* out)
+{
+    if (!mi || !out) return CSVB200_ERR_INVALID_ARG;
+    csvb200_multi* m = mi->m;
+    const uint64_t len = mi->base.back();
+    const uint64_t j = crlf ? (uint64_t)field_cnt + 1 : (uint64_t)field_cnt;   // src/tape.rs:318-321
+    if (j == 0 || len == 0) return mfail(m, CSVB200_ERR_INVALID_ARG, "field_cnt must be >= 1");
+    const int G = (int)mi->seg.size();
+    // device k checks the global slots [max(1, base[k]), base[k + 1]) of its segment against its shard.  The LF slot of a
+    // CRLF file compares its entry with the one before it, which for a segment's first slot lives in the nearest lower
+    // non-empty segment (slot 0 for segment 0): read here, one entry per segment, and handed to the kernel.
+    std::vector<uint64_t> prev(G, 0);
+    for (int k = 0; k < G && crlf; ++k) {
+        const uint64_t first = std::max<uint64_t>(1, mi->base[k]);
+        if (first < mi->base[k + 1]) {
+            int rc = read_entry(mi, first - 1, &prev[k]);
+            if (rc) return mfail(m, rc, csvb200_last_error(m->ctx[segment_of(mi->base.data(), (uint32_t)G, first - 1)]));
+        }
+    }
+    std::vector<int> rcs(G, CSVB200_OK);
+    std::vector<uint64_t> bad(G, UINT64_MAX);
+    run_phase(m, [&](int k) {
+        csvb200_ctx* ctx = m->ctx[k];
+        rcs[k] = [&]() -> int {
+            const uint64_t first = std::max<uint64_t>(1, mi->base[k]);
+            if (first >= mi->base[k + 1]) return CSVB200_OK;
+            CU_TRY(ctx, cudaSetDevice(ctx->device));
+            CellLease lease(ctx, 1);
+            if (!lease.ok()) return fail(ctx, CSVB200_ERR_OOM, "no free result cell (4095 live index objects)");
+            uint64_t* d_cell = ctx->d_cells + lease.first * kCellWords;
+            uint64_t* h_cell = ctx->h_cells + lease.first * kCellWords;
+            CU_TRY(ctx, cudaMemsetAsync(d_cell, 0xff, sizeof(uint64_t), ctx->stream));
+            TapeValidateParams p{};
+            p.index = by_global_slot(mi->table.ptr[k], mi->base[k]);
+            p.entry_bytes = 8;
+            p.index_len = mi->base[k + 1];
+            p.bytes = mi->d_bytes[k];
+            p.n = mi->cuts[k + 1] - mi->cuts[k];
+            p.pos_bias = mi->cuts[k];
+            p.jump = j;
+            p.crlf = crlf ? 1 : 0;
+            p.first_bad_slot = d_cell;
+            p.first_slot = first;
+            p.prev_entry = prev[k];
+            CU_TRY(ctx, launch_tape_validate_segment(p, ctx->stream));
+            ctx->launches += 1;
+            CU_TRY(ctx, cudaMemcpyAsync(h_cell, d_cell, sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
+            CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+            bad[k] = h_cell[0];
+            return CSVB200_OK;
+        }();
+    });
+    int rc = first_device_error(m, rcs);
+    if (rc) return rc;
+    std::memset(out, 0, sizeof(*out));
+    out->index_len = len;
+    out->jump = j;
+    out->record_cnt = (uint32_t)((len - 1) / j);   // src/tape.rs:323-325
+    out->problem = (len - 1) % j;                  // src/tape.rs:327
+    out->first_bad_slot = *std::min_element(bad.begin(), bad.end());
+    out->first_bad_record = UINT64_MAX;
+    out->first_bad_pos = UINT64_MAX;
+    if (out->first_bad_slot != UINT64_MAX) {
+        out->first_bad_record = (out->first_bad_slot - 1) / j;
+        rc = read_entry(mi, out->first_bad_slot, &out->first_bad_pos);
+        if (rc) return mfail(m, rc, csvb200_last_error(m->ctx[segment_of(mi->base.data(), (uint32_t)G, out->first_bad_slot)]));
+    } else if (out->problem != 0) {
+        out->first_bad_record = (len - 1) / j;     // the file ends inside this record
+    }
+    out->ok = out->first_bad_slot == UINT64_MAX && out->problem == 0;
+    return CSVB200_OK;
+}
+
+int csvb200_multi_validate_utf8(csvb200_multi_index* mi, uint64_t* valid_up_to, int* is_ascii)
+{
+    if (!mi) return CSVB200_ERR_INVALID_ARG;
+    csvb200_multi* m = mi->m;
+    const int G = (int)mi->seg.size();
+    // the first and last (up to) 3 bytes of every shard, from which the host assembles every shard's halo
+    std::vector<uint8_t> first3(3 * G, 0), last3(3 * G, 0);
+    std::vector<int> rcs(G, CSVB200_OK);
+    run_phase(m, [&](int k) {
+        csvb200_ctx* ctx = m->ctx[k];
+        rcs[k] = [&]() -> int {
+            const size_t n = mi->cuts[k + 1] - mi->cuts[k], c = std::min<size_t>(3, n);
+            if (c == 0) return CSVB200_OK;
+            uint8_t tail[3];
+            CU_TRY(ctx, cudaSetDevice(ctx->device));
+            CU_TRY(ctx, cudaMemcpyAsync(&first3[3 * k], mi->d_bytes[k], c, cudaMemcpyDeviceToHost, ctx->stream));
+            CU_TRY(ctx, cudaMemcpyAsync(tail, mi->d_bytes[k] + n - c, c, cudaMemcpyDeviceToHost, ctx->stream));
+            CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+            for (size_t i = 0; i < c; ++i) last3[3 * k + i] = tail[c - 1 - i];
+            return CSVB200_OK;
+        }();
+    });
+    int rc = first_device_error(m, rcs);
+    if (rc) return rc;
+    std::vector<uint64_t> bad(G, UINT64_MAX), high(G, 0);
+    run_phase(m, [&](int k) {
+        csvb200_ctx* ctx = m->ctx[k];
+        rcs[k] = [&]() -> int {
+            const uint64_t n = mi->cuts[k + 1] - mi->cuts[k];
+            if (n == 0) return CSVB200_OK;
+            const Utf8Halo halo = utf8_halo(mi->cuts.data(), (uint32_t)G, (uint32_t)k,
+                                            reinterpret_cast<const uint8_t(*)[3]>(first3.data()),
+                                            reinterpret_cast<const uint8_t(*)[3]>(last3.data()));
+            CU_TRY(ctx, cudaSetDevice(ctx->device));
+            CellLease lease(ctx, 1);
+            if (!lease.ok()) return fail(ctx, CSVB200_ERR_OOM, "no free result cell (4095 live index objects)");
+            uint64_t* d_cell = ctx->d_cells + lease.first * kCellWords;
+            uint64_t* h_cell = ctx->h_cells + lease.first * kCellWords;
+            CU_TRY(ctx, cudaMemsetAsync(d_cell, 0xff, sizeof(uint64_t), ctx->stream));
+            CU_TRY(ctx, cudaMemsetAsync(d_cell + 1, 0, sizeof(uint64_t), ctx->stream));
+            CU_TRY(ctx, launch_utf8_validate_segment(mi->d_bytes[k], n, mi->cuts[k], halo, d_cell, ctx->stream));
+            ctx->launches += 1;
+            CU_TRY(ctx, cudaMemcpyAsync(h_cell, d_cell, 2 * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
+            CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+            bad[k] = h_cell[0];
+            high[k] = h_cell[1];
+            return CSVB200_OK;
+        }();
+    });
+    rc = first_device_error(m, rcs);
+    if (rc) return rc;
+    if (valid_up_to) *valid_up_to = *std::min_element(bad.begin(), bad.end());
+    if (is_ascii) *is_ascii = *std::max_element(high.begin(), high.end()) ? 0 : 1;
+    return CSVB200_OK;
+}
+
+int csvb200_multi_tape_chunks(csvb200_multi_index* mi, uint8_t num, csvb200_chunk* out, size_t out_cap, size_t* n_out)
+{
+    if (!mi || !n_out) return CSVB200_ERR_INVALID_ARG;
+    csvb200_multi* m = mi->m;
+    if (!mi->tape_ready) return mfail(m, CSVB200_ERR_INVALID_STATE, "csvb200_multi_tape_init has not been called");
+    int rc = tape_chunk_slots(mi->record_cnt, mi->jump, num, out, out_cap, n_out);
+    if (rc) return mfail(m, rc, tape_chunk_error(rc));
+    // the byte ranges: two entries per chunk, each gathered on the device whose segment holds it
+    const int G = (int)mi->seg.size();
+    const size_t nvals = 2 * *n_out;
+    std::vector<uint64_t> slots(nvals), vals(nvals, UINT64_MAX);
+    std::vector<uint32_t> owner(nvals);
+    for (size_t i = 0; i < *n_out; ++i) {
+        slots[2 * i] = out[i].start;
+        slots[2 * i + 1] = out[i].end;
+    }
+    for (size_t i = 0; i < nvals; ++i) owner[i] = segment_of(mi->base.data(), (uint32_t)G, slots[i]);
+    std::vector<int> rcs(G, CSVB200_OK);
+    run_phase(m, [&](int k) {
+        csvb200_ctx* ctx = m->ctx[k];
+        rcs[k] = [&]() -> int {
+            std::vector<uint64_t> local, got;
+            for (size_t i = 0; i < nvals; ++i)
+                if (owner[i] == (uint32_t)k) local.push_back(slots[i] - mi->base[k]);
+            if (local.empty()) return CSVB200_OK;
+            got.resize(local.size());
+            CU_TRY(ctx, cudaSetDevice(ctx->device));
+            DevBuf d_slots, d_vals;
+            CU_TRY(ctx, d_slots.alloc(local.size() * 8, ctx->stream));
+            CU_TRY(ctx, d_vals.alloc(local.size() * 8, ctx->stream));
+            CU_TRY(ctx, cudaMemcpyAsync(d_slots.p, local.data(), local.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
+            CU_TRY(ctx, launch_gather_slots(mi->table.ptr[k], 8, mi->base[k + 1] - mi->base[k], d_slots.as<uint64_t>(),
+                                            local.size(), d_vals.as<uint64_t>(), ctx->stream));
+            ctx->launches += 1;
+            CU_TRY(ctx, cudaMemcpyAsync(got.data(), d_vals.p, got.size() * 8, cudaMemcpyDeviceToHost, ctx->stream));
+            CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+            for (size_t i = 0, q = 0; i < nvals; ++i)
+                if (owner[i] == (uint32_t)k) vals[i] = got[q++];
+            return CSVB200_OK;
+        }();
+    });
+    rc = first_device_error(m, rcs);
+    if (rc) return rc;
+    for (size_t i = 0; i < *n_out; ++i) {
+        out[i].byte_start = vals[2 * i] == UINT64_MAX ? UINT64_MAX : vals[2 * i] + 1;
+        out[i].byte_end = vals[2 * i + 1] == UINT64_MAX ? UINT64_MAX : vals[2 * i + 1] + 1;
+    }
+    return CSVB200_OK;
+}
+
+}  // extern "C"

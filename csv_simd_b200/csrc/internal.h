@@ -178,8 +178,14 @@ struct TapeValidateParams {
     int crlf;
     uint64_t* first_bad_slot;   // device word, preset to UINT64_MAX; atomicMin
     uint32_t entry_bytes;
+    // segment form only: `index` addresses GLOBAL slots (index[s] for s in [first_slot, index_len), u64 entries), the
+    // slots checked are [first_slot, index_len) with first_slot >= 1, and prev_entry is the entry of slot first_slot - 1,
+    // which the kernel never reads from `index` (it lives in a lower segment, on another device)
+    uint64_t first_slot;
+    uint64_t prev_entry;
 };
 cudaError_t launch_tape_validate(const TapeValidateParams& p, cudaStream_t stream);
+cudaError_t launch_tape_validate_segment(const TapeValidateParams& p, cudaStream_t stream);
 // out[i] = index[slots[i]] (UINT64_MAX when the slot is past the end); entry_bytes per index entry
 cudaError_t launch_gather_slots(const void* index, uint32_t entry_bytes, uint64_t index_len, const uint64_t* slots,
                                 uint64_t n, uint64_t* out, cudaStream_t stream);
@@ -189,6 +195,12 @@ cudaError_t launch_widen_entries(const uint32_t* in, uint64_t n, uint64_t* out, 
 // K7 ASCII / UTF-8 validation (validate.cu): result[0] (preset UINT64_MAX) <- start of the first ill-formed
 // sequence, result[1] (preset 0) <- 1 when any byte is >= 0x80
 cudaError_t launch_utf8_validate(const uint8_t* in, uint64_t n, uint64_t* result, cudaStream_t stream);
+// the same over one shard of a distributed input: in[0] is global byte pos_bias, the halo holds the bytes around the
+// shard (utf8_halo.h); result[0] gets the global start of the first ill-formed sequence LED inside the shard, result[1]
+// is set when a byte of the shard itself is >= 0x80
+struct Utf8Halo;
+cudaError_t launch_utf8_validate_segment(const uint8_t* in, uint64_t n, uint64_t pos_bias, const Utf8Halo& halo,
+                                         uint64_t* result, cudaStream_t stream);
 // the same over the tiles (tile_bytes each) whose bit is set in `bitmap` only: the build kernel flags the tiles that
 // hold a byte >= 0x80, every other tile is ASCII and leads (and owes) no multi-byte sequence
 cudaError_t launch_utf8_validate_flagged(const uint8_t* in, uint64_t n, const uint32_t* bitmap, uint64_t tile_bytes,

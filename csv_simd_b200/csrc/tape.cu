@@ -20,8 +20,9 @@ namespace {
 // template parameter, k = (s - 1) % jump lives in 32 bits and advances by 32 % jump, and the only 64-bit
 // work left per slot is the position arithmetic (the first version spent ~100 instructions per slot row on
 // 64-bit modulo / select chains and was issue-bound at 0.55 of the HBM peak).  E: the entry type, u64 or the u32 of a
-// compact index.
-template <bool kCrlf, class E>
+// compact index.  kSeg: the segment form (one segment of a distributed index, see TapeValidateParams) -- its own
+// instantiations, so the one-GPU ones compile to the code they always had.
+template <bool kCrlf, class E, bool kSeg>
 __global__ void __launch_bounds__(256) tape_validate_kernel(const TapeValidateParams p)
 {
     const uint32_t lane = threadIdx.x & 31u;
@@ -30,12 +31,13 @@ __global__ void __launch_bounds__(256) tape_validate_kernel(const TapeValidatePa
     const uint32_t jump = (uint32_t)p.jump;
     const uint32_t nl0 = jump - (kCrlf ? 2u : 1u);    // first line-end slot of a row (k >= nl0 is CR / LF territory)
     const uint64_t last = p.index_len - 1;            // slots are 1 .. last; i = s - 1 in [0, last)
+    const uint64_t i_first = kSeg ? p.first_slot - 1 : 0;   // the segment form starts at its own first slot
     const uint32_t step = 32u % jump;                 // k advances by 32 slots per warp row
     const E* __restrict__ index = static_cast<const E*>(p.index) + 1;   // index[i] here is slot s = i + 1
     uint64_t bad = UINT64_MAX;                        // smallest failing i
     constexpr int kUnroll = 4;
     constexpr uint64_t kRun = 32 * 16;
-    for (uint64_t run = warp0 * kRun; run < last; run += warps * kRun) {
+    for (uint64_t run = i_first + warp0 * kRun; run < last; run += warps * kRun) {
         const uint64_t run_end = run + kRun < last ? run + kRun : last;
         uint32_t k = (uint32_t)((run + lane) % jump);
         for (uint64_t i = run + lane; i < run_end; i += 32 * kUnroll) {
@@ -67,7 +69,8 @@ __global__ void __launch_bounds__(256) tape_validate_kernel(const TapeValidatePa
                 } else if (kk[u] == nl0) {
                     ok = b == 0x0Du;
                 } else {
-                    ok = b == 0x0Au && ldg_entry(index + iu - 1) + 1 == pos[u];   // the LF directly after its CR
+                    // the LF directly after its CR; a segment's first slot finds its CR's entry in prev_entry
+                    ok = b == 0x0Au && (kSeg && iu == i_first ? p.prev_entry : ldg_entry(index + iu - 1)) + 1 == pos[u];
                 }
                 if (!ok && iu < bad) bad = iu;
             }
@@ -134,26 +137,46 @@ cudaError_t launch_widen_entries(const uint32_t* in, uint64_t n, uint64_t* out, 
     return cudaGetLastError();
 }
 
-cudaError_t launch_tape_validate(const TapeValidateParams& p, cudaStream_t stream)
+// blocks for `slots` slots: 8 warps per block, one run each, at most 8 blocks per SM
+static unsigned tape_validate_blocks(uint64_t slots)
 {
-    if (p.index_len <= 1 || p.jump == 0) return cudaSuccess;
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    uint64_t blocks = (p.index_len + 32 * 16 * 8 - 1) / (32 * 16 * 8);   // 8 warps per block, one run each
+    uint64_t blocks = (slots + 32 * 16 * 8 - 1) / (32 * 16 * 8);
     const uint64_t max_blocks = (uint64_t)sms * 8;
     if (blocks > max_blocks) blocks = max_blocks;
     if (blocks == 0) blocks = 1;
+    return (unsigned)blocks;
+}
+
+cudaError_t launch_tape_validate(const TapeValidateParams& p, cudaStream_t stream)
+{
+    if (p.index_len <= 1 || p.jump == 0) return cudaSuccess;
+    const unsigned blocks = tape_validate_blocks(p.index_len);
     if (p.jump > 0xffffffffull) return cudaErrorInvalidValue;
     const bool compact = p.entry_bytes == 4;
     if (p.crlf && compact)
-        tape_validate_kernel<true, uint32_t><<<(unsigned)blocks, 256, 0, stream>>>(p);
+        tape_validate_kernel<true, uint32_t, false><<<blocks, 256, 0, stream>>>(p);
     else if (p.crlf)
-        tape_validate_kernel<true, uint64_t><<<(unsigned)blocks, 256, 0, stream>>>(p);
+        tape_validate_kernel<true, uint64_t, false><<<blocks, 256, 0, stream>>>(p);
     else if (compact)
-        tape_validate_kernel<false, uint32_t><<<(unsigned)blocks, 256, 0, stream>>>(p);
+        tape_validate_kernel<false, uint32_t, false><<<blocks, 256, 0, stream>>>(p);
     else
-        tape_validate_kernel<false, uint64_t><<<(unsigned)blocks, 256, 0, stream>>>(p);
+        tape_validate_kernel<false, uint64_t, false><<<blocks, 256, 0, stream>>>(p);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_tape_validate_segment(const TapeValidateParams& p, cudaStream_t stream)
+{
+    if (p.first_slot == 0 || p.first_slot >= p.index_len || p.jump == 0) return cudaSuccess;
+    if (p.jump > 0xffffffffull) return cudaErrorInvalidValue;
+    if (p.entry_bytes == 4) return cudaErrorInvalidValue;   // the segments of a distributed index hold u64 entries
+    const unsigned blocks = tape_validate_blocks(p.index_len - p.first_slot);
+    if (p.crlf)
+        tape_validate_kernel<true, uint64_t, true><<<blocks, 256, 0, stream>>>(p);
+    else
+        tape_validate_kernel<false, uint64_t, true><<<blocks, 256, 0, stream>>>(p);
     return cudaGetLastError();
 }
 

@@ -12,6 +12,7 @@
 // look-ahead, 3 of look-behind) and the answer is an atomicMin.  32-byte groups that are pure ASCII (the
 // common case in CSV) cost two 128-bit loads and a mask test.
 #include "internal.h"
+#include "utf8_halo.h"
 #include "utf8slice.cuh"
 
 namespace csvb200 {
@@ -54,8 +55,42 @@ __device__ __forceinline__ uint64_t judge_group(const uint8_t* __restrict__ in, 
     return r == kUtf8None ? UINT64_MAX : i0 + r;
 }
 
-__global__ void __launch_bounds__(256) utf8_validate_kernel(const uint8_t* __restrict__ in, uint64_t n,
-                                                            uint64_t* __restrict__ result)   // {valid_up_to, non-ascii flag}
+// The same for one shard of a distributed input, global bytes [pos_bias, pos_bias + n), given its halo (utf8_halo.h).
+// Only sequences LED inside the shard are judged: the after-halo is look-ahead only, since a lead there has its own
+// look-ahead cut off by the halo's end and is judged by the device that holds it.  In the shard's last group the
+// after-halo bytes take the places of the zero fill past n.  Returns the global start or UINT64_MAX.
+__device__ __forceinline__ uint64_t judge_group_seg(const uint8_t* __restrict__ in, uint64_t n, uint64_t i0, const uint32_t w_in[8],
+                                                    const Utf8Halo& h, uint64_t pos_bias)
+{
+    uint32_t w[8];
+#pragma unroll
+    for (int k = 0; k < 8; ++k) w[k] = w_in[k];
+    if (i0 + 32 > n) {
+        const uint32_t a = h.after_len ? h.after & (0xffffffu >> (8 * (3 - h.after_len))) : 0u;
+        const int at = 8 * (int)(n - i0);                              // bit position of byte n inside the group
+#pragma unroll
+        for (int k = 0; k < 8; ++k) {
+            const int sh = at - 32 * k;
+            if (sh >= 0 && sh < 32) w[k] |= a << sh;
+            else if (sh < 0 && sh > -24) w[k] |= a >> -sh;
+        }
+    }
+    const uint32_t b1 = i0 ? in[i0 - 1] : h.before & 0xffu, b2 = i0 ? in[i0 - 2] : (h.before >> 8) & 0xffu,
+                   b3 = i0 ? in[i0 - 3] : h.before >> 16;             // i0 is 0 or >= 32
+    uint32_t nx[3];
+#pragma unroll
+    for (int d = 0; d < 3; ++d) {
+        const uint64_t q = i0 + 32 + d;
+        nx[d] = q < n ? (uint32_t)in[q] : q - n < h.after_len ? (h.after >> (8 * (q - n))) & 0xffu : 0x100u;
+    }
+    const uint32_t r = utf8_check32(w, utf8_owed(b1, b2, b3), nx[0], nx[1], nx[2]);
+    return r == kUtf8None || i0 + r >= n ? UINT64_MAX : pos_bias + i0 + r;
+}
+
+// kSeg: the shard form (utf8_validate_segment_kernel); the one-GPU kernel instantiates the code it always had
+template <bool kSeg>
+__device__ __forceinline__ void utf8_validate_body(const uint8_t* __restrict__ in, uint64_t n, uint64_t* __restrict__ result,
+                                                   const Utf8Halo& h, uint64_t pos_bias)
 {
     const uint64_t ngroups = (n + 31) / 32;
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
@@ -74,14 +109,16 @@ __global__ void __launch_bounds__(256) utf8_validate_kernel(const uint8_t* __res
             oa |= wa[k];
             ob |= has_b ? wb[k] : 0u;
         }
-        if (oa & 0x80808080u) {            // pure-ASCII groups (the common case in CSV) lead no multi-byte sequence
+        // pure-ASCII groups (the common case in CSV) lead no multi-byte sequence; the zero fill past n keeps a shard's
+        // after-halo out of oa / ob
+        if (oa & 0x80808080u) {
             nonascii = 1u;
-            const uint64_t r = judge_group(in, n, ia, wa);
+            const uint64_t r = kSeg ? judge_group_seg(in, n, ia, wa, h, pos_bias) : judge_group(in, n, ia, wa);
             bad = r < bad ? r : bad;
         }
         if (ob & 0x80808080u) {
             nonascii = 1u;
-            const uint64_t r = judge_group(in, n, ib, wb);
+            const uint64_t r = kSeg ? judge_group_seg(in, n, ib, wb, h, pos_bias) : judge_group(in, n, ib, wb);
             bad = r < bad ? r : bad;
         }
     }
@@ -95,6 +132,19 @@ __global__ void __launch_bounds__(256) utf8_validate_kernel(const uint8_t* __res
         if (bad != UINT64_MAX) atomicMin(reinterpret_cast<unsigned long long*>(result), (unsigned long long)bad);
         if (any) atomicOr(reinterpret_cast<unsigned long long*>(result + 1), 1ull);
     }
+}
+
+__global__ void __launch_bounds__(256) utf8_validate_kernel(const uint8_t* __restrict__ in, uint64_t n,
+                                                            uint64_t* __restrict__ result)   // {valid_up_to, non-ascii flag}
+{
+    utf8_validate_body<false>(in, n, result, Utf8Halo{0u, 0u, 0u}, 0);
+}
+
+__global__ void __launch_bounds__(256) utf8_validate_segment_kernel(const uint8_t* __restrict__ in, uint64_t n,
+                                                                    uint64_t pos_bias, const Utf8Halo halo,
+                                                                    uint64_t* __restrict__ result)
+{
+    utf8_validate_body<true>(in, n, result, halo, pos_bias);
 }
 
 // Only the tiles the build kernel flagged (a byte >= 0x80 somewhere inside): one CTA per flagged tile at a time.
@@ -148,16 +198,30 @@ cudaError_t launch_utf8_validate_flagged(const uint8_t* in, uint64_t n, const ui
     return cudaGetLastError();
 }
 
-cudaError_t launch_utf8_validate(const uint8_t* in, uint64_t n, uint64_t* result, cudaStream_t stream)
+// two 32-byte groups per thread and sweep, at most 8 blocks per SM
+static unsigned utf8_validate_blocks(uint64_t n)
 {
-    if (n == 0) return cudaSuccess;
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     uint64_t blocks = ((n + 31) / 32 + 511) / 512;
     const uint64_t max_blocks = (uint64_t)sms * 8;
     if (blocks > max_blocks) blocks = max_blocks;
-    utf8_validate_kernel<<<(unsigned)blocks, 256, 0, stream>>>(in, n, result);
+    return (unsigned)blocks;
+}
+
+cudaError_t launch_utf8_validate(const uint8_t* in, uint64_t n, uint64_t* result, cudaStream_t stream)
+{
+    if (n == 0) return cudaSuccess;
+    utf8_validate_kernel<<<utf8_validate_blocks(n), 256, 0, stream>>>(in, n, result);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_utf8_validate_segment(const uint8_t* in, uint64_t n, uint64_t pos_bias, const Utf8Halo& halo,
+                                         uint64_t* result, cudaStream_t stream)
+{
+    if (n == 0) return cudaSuccess;
+    utf8_validate_segment_kernel<<<utf8_validate_blocks(n), 256, 0, stream>>>(in, n, pos_bias, halo, result);
     return cudaGetLastError();
 }
 

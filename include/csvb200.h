@@ -291,6 +291,15 @@ int csvb200_multi_materialize_columns(csvb200_multi_index* mi, const uint32_t* f
                                       uint32_t first_record, uint32_t nrec, uint32_t flags,
                                       uint64_t* const* out_offsets, uint8_t* const* outs,
                                       const size_t* out_caps, size_t* out_lens);
+/* csvb200_tape_validate, csvb200_validate_utf8 (over the whole input) and csvb200_tape_chunks over the distributed
+ * index, with the same results field for field and the same status codes as the one-GPU calls on an index of the same
+ * bytes.  Every device checks its own segment against its own shard of the bytes, in place: nothing is uploaded again
+ * or gathered.  The tape check needs no csvb200_multi_tape_init; the chunks do (else CSVB200_ERR_INVALID_STATE). */
+struct csvb200_tape_report;
+struct csvb200_chunk;
+int csvb200_multi_tape_validate(csvb200_multi_index* mi, uint32_t field_cnt, int crlf, struct csvb200_tape_report* out);
+int csvb200_multi_validate_utf8(csvb200_multi_index* mi, uint64_t* valid_up_to, int* is_ascii);
+int csvb200_multi_tape_chunks(csvb200_multi_index* mi, uint8_t num, struct csvb200_chunk* out, size_t out_cap, size_t* n_out);
 
 typedef struct csvb200_multi_stats {
     double seconds, upload_seconds, download_seconds;

@@ -140,6 +140,14 @@ SIGNATURES = {
     "csvb200_seek_records_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "csvb200_gather_fields": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p,
                                         C.c_size_t]),
+    "csvb200_seek_values": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint32, C.c_void_p, C.c_void_p,
+                                      C.c_size_t, szp, C.c_void_p]),
+    "csvb200_seek_values_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint32, C.c_void_p,
+                                             C.c_void_p, C.c_size_t, C.c_void_p]),
+    "csvb200_multi_seek_values": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint32, C.c_void_p,
+                                            C.c_void_p, C.c_size_t, szp, C.c_void_p]),
+    "csvb200_multi_seek_values_device": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint32,
+                                                   C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "csvb200_materialize_column": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p,
                                              C.c_void_p, C.c_size_t, szp]),
     "csvb200_materialize_column_device": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32,

@@ -50,6 +50,32 @@ def _as_u8(data) -> np.ndarray:
     return np.frombuffer(data, dtype=np.uint8)
 
 
+def _values_call(call, rec, fld, flags):
+    """The two-call protocol of csvb200_seek_values / csvb200_multi_seek_values: the first call sizes the output
+    (CSVB200_ERR_CAPACITY is expected), the second fills it -> (offsets, values, found)."""
+    rec = np.ascontiguousarray(rec, dtype=np.uint32)
+    if fld is not None:
+        fld = np.ascontiguousarray(fld, dtype=np.uint32)
+        if fld.size != rec.size:
+            raise ValueError("rec and fld differ in length")
+    nq = int(rec.size)
+    offs = np.zeros(nq + 1, dtype=np.uint64)
+    words = np.zeros(max((nq + 63) // 64, 1), dtype=np.uint64)
+    ln = C.c_size_t()
+    p_fld = fld.ctypes.data if fld is not None else None
+    rc = call(rec.ctypes.data, p_fld, nq, flags, offs.ctypes.data, None, 0, C.byref(ln), words.ctypes.data)
+    if rc not in (0, 9):
+        return rc, None
+    out = np.empty(ln.value, dtype=np.uint8)
+    if out.size:
+        rc = call(rec.ctypes.data, p_fld, nq, flags, offs.ctypes.data, out.ctypes.data, out.size, C.byref(ln),
+                  words.ctypes.data)
+        if rc:
+            return rc, None
+    found = np.unpackbits(words.view(np.uint8), bitorder="little")[:nq].astype(bool)
+    return 0, (offs, out, found)
+
+
 class Context:
     """csvb200_ctx: one per GPU (process-per-GPU model)."""
 
@@ -507,6 +533,20 @@ class MultiIndex:
         self._check(self._lib.csvb200_multi_seek_fields_device(self._h, k, C.c_void_p(d_rec), C.c_void_p(d_fld), nq,
                                                                C.c_void_p(d_out)))
 
+    def seek_values(self, rec: np.ndarray, fld: np.ndarray | None = None, flags: int = FIELD_RAW):
+        """csvb200_multi_seek_values: as StructureIndex.seek_values, every device resolving a share of the batch and
+        reading the values straight from the shards -> (offsets[nq + 1], values, found[nq] as bools)."""
+        rc, res = _values_call(lambda *a: self._lib.csvb200_multi_seek_values(self._h, *a), rec, fld, flags)
+        self._check(rc)
+        return res
+
+    def seek_values_device(self, k: int, d_rec: int, d_fld: int | None, nq: int, flags: int, d_offsets: int,
+                           d_out: int | None = None, out_cap: int = 0, d_found_bits: int | None = None):
+        """csvb200_multi_seek_values_device: device arrays on device k of the list, asynchronous on its stream."""
+        self._check(self._lib.csvb200_multi_seek_values_device(self._h, k, C.c_void_p(d_rec), C.c_void_p(d_fld or 0), nq,
+                                                               flags, C.c_void_p(d_offsets), C.c_void_p(d_out or 0), out_cap,
+                                                               C.c_void_p(d_found_bits or 0)))
+
     def free(self):
         if getattr(self, "_h", None) and getattr(self.multi, "_h", None):
             self._lib.csvb200_multi_index_free(self._h)
@@ -710,6 +750,23 @@ class StructureIndex:
         self.ctx._check(self._lib.csvb200_materialize_column_device(self._h, field_idx, first_record, nrec, flags,
                                                                     C.c_void_p(d_offsets), C.c_void_p(d_out or 0),
                                                                     out_cap))
+
+    def seek_values(self, rec: np.ndarray, fld: np.ndarray | None = None, flags: int = FIELD_RAW):
+        """csvb200_seek_values: the values behind a batch of lookups -> (offsets[nq + 1], values, found[nq] as bools).
+        fld given: value q is field fld[q] of record rec[q], trimmed / unquoted by flags as in materialize_column;
+        fld None: value q is the text of record rec[q] (flags must be 0).  A lookup that finds nothing is an empty
+        value with found False."""
+        rc, res = _values_call(lambda *a: self._lib.csvb200_seek_values(self._h, *a), rec, fld, flags)
+        self.ctx._check(rc)
+        return res
+
+    def seek_values_device(self, d_rec: int, d_fld: int | None, nq: int, flags: int, d_offsets: int,
+                           d_out: int | None = None, out_cap: int = 0, d_found_bits: int | None = None):
+        """csvb200_seek_values_device: device arrays, asynchronous on the context's stream; d_out None = offsets only,
+        a value that would end past out_cap is skipped whole."""
+        self.ctx._check(self._lib.csvb200_seek_values_device(self._h, C.c_void_p(d_rec), C.c_void_p(d_fld or 0), nq, flags,
+                                                             C.c_void_p(d_offsets), C.c_void_p(d_out or 0), out_cap,
+                                                             C.c_void_p(d_found_bits or 0)))
 
     def gather_fields(self, rec: np.ndarray, fld: np.ndarray):
         rec = np.ascontiguousarray(rec, dtype=np.uint32)

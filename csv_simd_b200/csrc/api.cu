@@ -1800,46 +1800,187 @@ int csvb200_seek_records_device(csvb200_index* idx, const uint32_t* d_rec, size_
     return seek_device(idx, d_rec, nullptr, nq, d_out, reinterpret_cast<uint32_t*>(idx->ctx->d_cells + (kCells - 1) * kCellWords));
 }
 
-int csvb200_gather_fields(csvb200_index* idx, const uint32_t* rec, const uint32_t* fld, size_t nq,
-                          uint64_t* out_offsets, uint8_t* out, size_t out_cap)
+static int values_prepare(csvb200_index* idx)
 {
     int rc = seek_prepare(idx);
     if (rc) return rc;
-    csvb200_ctx* ctx = idx->ctx;
     if (!idx->d_bytes_owned && !idx->src)
-        return fail(ctx, CSVB200_ERR_INVALID_STATE, "index was built without CSVB200_BUILD_KEEP_BYTES");
-    if (!out_offsets || (nq && (!rec || !fld))) return fail(ctx, CSVB200_ERR_INVALID_ARG, "null argument");
+        return fail(idx->ctx, CSVB200_ERR_INVALID_STATE, "index was built without CSVB200_BUILD_KEEP_BYTES");
+    return CSVB200_OK;
+}
+
+static int values_args(csvb200_index* idx, const void* rec, const void* fld, size_t nq, uint32_t flags, const void* offsets)
+{
+    if (!offsets || (nq && !rec)) return fail(idx->ctx, CSVB200_ERR_INVALID_ARG, "null argument");
+    if (flags & ~(CSVB200_FIELD_UNQUOTE | CSVB200_FIELD_TRIM)) return fail(idx->ctx, CSVB200_ERR_INVALID_ARG, "unknown field flags");
+    if (flags && !fld) return fail(idx->ctx, CSVB200_ERR_INVALID_ARG, "flags apply to fields only (fld == NULL: records)");
+    return CSVB200_OK;
+}
+
+static ValuesParams values_params(const csvb200_index* idx, const uint32_t* rec, const uint32_t* fld, size_t nq, uint32_t flags)
+{
+    ValuesParams p{};
+    p.index_len = idx->len;
+    p.record_cnt = idx->record_cnt;
+    p.field_cnt = idx->field_cnt;
+    p.row_size = (uint32_t)idx->jump;
+    p.flags = flags;
+    p.rec = rec;
+    p.fld = fld;
+    p.nq = nq;
+    return p;
+}
+
+static ValuesLocal values_source(const csvb200_index* idx)
+{
+    return ValuesLocal{idx->d_entries, idx->entry_bytes, idx->d_bytes_owned ? idx->d_bytes_owned : idx->src, idx->n, idx->pos_bias};
+}
+
+}  // extern "C"
+
+namespace csvb200 {
+
+int values_enqueue(csvb200_ctx* ctx, ValuesParams p, const ValuesLocal* local, const SegmentTable* seg, const ShardBytes* sb,
+                   bool write_pass)
+{
+    const size_t sbytes = values_scratch_bytes(p.nq);
+    int rc = ensure_scratch(ctx, sbytes);
+    if (rc) return rc;
+    CU_TRY(ctx, cudaMemsetAsync(ctx->d_scratch, 0, sbytes, ctx->stream));
+    p.ticket = reinterpret_cast<uint32_t*>(ctx->d_scratch);
+    p.tile_desc = reinterpret_cast<uint64_t*>(ctx->d_scratch + 128);
+    if (p.nq == 0) {   // every caller of an empty batch asks for offsets that start at 0
+        CU_TRY(ctx, cudaMemsetAsync(p.offsets, 0, sizeof(uint64_t), ctx->stream));
+        return CSVB200_OK;
+    }
+    CU_TRY(ctx, local ? launch_values_offsets(p, *local, ctx->stream) : launch_values_offsets_sharded(p, *seg, *sb, ctx->stream));
+    ctx->launches += 1;
+    if (write_pass && p.out) {
+        CU_TRY(ctx, local ? launch_values_write(p, *local, ctx->stream) : launch_values_write_sharded(p, *seg, *sb, ctx->stream));
+        ctx->launches += 1;
+    }
+    return CSVB200_OK;
+}
+
+}  // namespace csvb200
+
+extern "C" {
+
+// Host arrays in / out, in chunks of kValuesChunk queries.  Sweep 1: per chunk, the queries go up, the offsets pass
+// runs with the running total as its base, and the offsets and found bits come down in place; the counters decide
+// OUT_OF_BOUNDS and the total decides CAPACITY before anything is written.  Sweep 2: per chunk, the values are written
+// into one device buffer sized by the largest chunk's values and go down to their place in `out`.
+int csvb200_seek_values(csvb200_index* idx, const uint32_t* rec, const uint32_t* fld, size_t nq, uint32_t flags,
+                        uint64_t* out_offsets, uint8_t* out, size_t out_cap, size_t* out_len, uint64_t* found_bits)
+{
+    int rc = values_prepare(idx);
+    if (rc) return rc;
+    csvb200_ctx* ctx = idx->ctx;
+    if (!out_len) return fail(ctx, CSVB200_ERR_INVALID_ARG, "null argument");
+    rc = values_args(idx, rec, fld, nq, flags, out_offsets);
+    if (rc) return rc;
+    *out_len = 0;
     out_offsets[0] = 0;
     if (nq == 0) return CSVB200_OK;
-    std::vector<csvb200_range> ranges(nq);
-    rc = seek_host(idx, rec, fld, nq, ranges.data());
-    if (rc) return rc;
-    // positions are global; the bytes this index object holds are [pos_bias, pos_bias + n) (a shard of a sharded build)
-    const uint64_t lo = idx->pos_bias, hi = idx->pos_bias + idx->n;
-    for (size_t i = 0; i < nq; ++i) {
-        const csvb200_range& r = ranges[i];
-        const uint64_t len = (r.start == UINT64_MAX || r.end < r.start) ? 0 : r.end - r.start;
-        if (len && (r.start < lo || r.end > hi))
-            return fail(ctx, CSVB200_ERR_OUT_OF_BOUNDS, "field lies outside the bytes this index object holds (another shard)");
-        out_offsets[i + 1] = out_offsets[i] + len;
+    constexpr size_t kValuesChunk = 1u << 20;   // a multiple of 64: every chunk writes whole found-bit words
+    const size_t chunk = std::min(nq, kValuesChunk);
+    const size_t nchunks = (nq + chunk - 1) / chunk;
+    DevBuf d_rec, d_fld, d_off, d_found, d_cnt, d_out;
+    CU_TRY(ctx, d_rec.alloc(chunk * sizeof(uint32_t), ctx->stream));
+    if (fld) CU_TRY(ctx, d_fld.alloc(chunk * sizeof(uint32_t), ctx->stream));
+    CU_TRY(ctx, d_off.alloc((chunk + 1) * sizeof(uint64_t), ctx->stream));
+    if (found_bits) CU_TRY(ctx, d_found.alloc((chunk + 63) / 64 * sizeof(uint64_t), ctx->stream));
+    CU_TRY(ctx, d_cnt.alloc(2 * sizeof(uint32_t), ctx->stream));
+    CU_TRY(ctx, cudaMemsetAsync(d_cnt.p, 0, 2 * sizeof(uint32_t), ctx->stream));
+    const ValuesLocal src = values_source(idx);
+    auto upload_queries = [&](size_t off, size_t len) -> int {
+        CU_TRY(ctx, cudaMemcpyAsync(d_rec.p, rec + off, len * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+        if (fld) CU_TRY(ctx, cudaMemcpyAsync(d_fld.p, fld + off, len * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+        return CSVB200_OK;
+    };
+    uint64_t total = 0, largest = 0;
+    for (size_t c = 0; c < nchunks; ++c) {
+        const size_t off = c * chunk, len = std::min(chunk, nq - off);
+        rc = upload_queries(off, len);
+        if (rc) return rc;
+        ValuesParams p = values_params(idx, d_rec.as<uint32_t>(), fld ? d_fld.as<uint32_t>() : nullptr, len, flags);
+        p.offsets = d_off.as<uint64_t>();
+        p.offset_base = total;
+        p.found = found_bits ? d_found.as<uint32_t>() : nullptr;
+        p.counts = d_cnt.as<uint32_t>();
+        rc = values_enqueue(ctx, p, &src, nullptr, nullptr, false);
+        if (rc) return rc;
+        CU_TRY(ctx, cudaMemcpyAsync(out_offsets + off, d_off.p, (len + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
+        if (found_bits)
+            CU_TRY(ctx, cudaMemcpyAsync(found_bits + off / 64, d_found.p, (len + 63) / 64 * sizeof(uint64_t), cudaMemcpyDeviceToHost,
+                                        ctx->stream));
+        CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+        largest = std::max<uint64_t>(largest, out_offsets[off + len] - total);
+        total = out_offsets[off + len];
     }
-    const uint64_t total = out_offsets[nq];
-    if (total > out_cap) return fail(ctx, CSVB200_ERR_CAPACITY, "gather destination too small");
+    uint32_t counts[2] = {0, 0};
+    CU_TRY(ctx, cudaMemcpyAsync(counts, d_cnt.p, sizeof(counts), cudaMemcpyDeviceToHost, ctx->stream));
+    CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    if (counts[0]) return fail(ctx, CSVB200_ERR_OUT_OF_BOUNDS, "lookup slot past the end of the index");
+    // positions are global; the bytes this index object holds are [pos_bias, pos_bias + n) (a shard of a sharded build)
+    if (counts[1]) return fail(ctx, CSVB200_ERR_OUT_OF_BOUNDS, "value lies outside the bytes this index object holds (another shard)");
+    *out_len = (size_t)total;
+    if (total > out_cap) return fail(ctx, CSVB200_ERR_CAPACITY, "values destination too small");
     if (total == 0) return CSVB200_OK;
     if (!out) return fail(ctx, CSVB200_ERR_INVALID_ARG, "null argument");
-    DevBuf d_ranges, d_off, d_out;
-    CU_TRY(ctx, d_ranges.alloc(nq * sizeof(csvb200_range), ctx->stream));
-    CU_TRY(ctx, d_off.alloc((nq + 1) * sizeof(uint64_t), ctx->stream));
-    CU_TRY(ctx, d_out.alloc(total, ctx->stream));
-    CU_TRY(ctx, cudaMemcpyAsync(d_ranges.p, ranges.data(), nq * sizeof(csvb200_range), cudaMemcpyHostToDevice, ctx->stream));
-    CU_TRY(ctx, cudaMemcpyAsync(d_off.p, out_offsets, (nq + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream));
-    const uint8_t* bytes = idx->d_bytes_owned ? idx->d_bytes_owned : idx->src;
-    CU_TRY(ctx, launch_gather_bytes(bytes, idx->n, idx->pos_bias, d_ranges.as<uint64_t>(), d_off.as<uint64_t>(), nq,
-                                    d_out.as<uint8_t>(), ctx->stream));
-    ctx->launches += 1;
-    CU_TRY(ctx, cudaMemcpyAsync(out, d_out.p, total, cudaMemcpyDeviceToHost, ctx->stream));
+    CU_TRY(ctx, d_out.alloc(largest, ctx->stream));
+    for (size_t c = 0; c < nchunks; ++c) {
+        const size_t off = c * chunk, len = std::min(chunk, nq - off);
+        const uint64_t base = out_offsets[off], bytes = out_offsets[off + len] - base;
+        if (bytes == 0) continue;
+        if (nchunks > 1) {   // one chunk: its queries and offsets are still on the device
+            rc = upload_queries(off, len);
+            if (rc) return rc;
+            CU_TRY(ctx, cudaMemcpyAsync(d_off.p, out_offsets + off, (len + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream));
+        }
+        ValuesParams p = values_params(idx, d_rec.as<uint32_t>(), fld ? d_fld.as<uint32_t>() : nullptr, len, flags);
+        p.offsets = d_off.as<uint64_t>();
+        p.offset_base = base;
+        p.out = d_out.as<uint8_t>();
+        p.out_cap = bytes;
+        CU_TRY(ctx, launch_values_write(p, src, ctx->stream));
+        ctx->launches += 1;
+        CU_TRY(ctx, cudaMemcpyAsync(out + base, d_out.p, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    }
     CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     return CSVB200_OK;
+}
+
+int csvb200_seek_values_device(csvb200_index* idx, const uint32_t* d_rec, const uint32_t* d_fld, size_t nq, uint32_t flags,
+                               uint64_t* d_offsets, uint8_t* d_out, size_t out_cap, uint64_t* d_found_bits)
+{
+    int rc = values_prepare(idx);
+    if (rc) return rc;
+    rc = values_args(idx, d_rec, d_fld, nq, flags, d_offsets);
+    if (rc) return rc;
+    ValuesParams p = values_params(idx, d_rec, d_fld, nq, flags);
+    p.offsets = d_offsets;
+    p.out = d_out;
+    p.out_cap = out_cap;
+    p.found = reinterpret_cast<uint32_t*>(d_found_bits);
+    // out-of-bounds slots are reported as None on this asynchronous path
+    p.counts = reinterpret_cast<uint32_t*>(idx->ctx->d_cells + (kCells - 1) * kCellWords);
+    const ValuesLocal src = values_source(idx);
+    return values_enqueue(idx->ctx, p, &src, nullptr, nullptr, true);
+}
+
+// the values of flags == 0: the old two-kernel gather (ranges to the host, a serial prefix sum there, ranges and
+// offsets back up) is the same computation as the raw form of csvb200_seek_values
+int csvb200_gather_fields(csvb200_index* idx, const uint32_t* rec, const uint32_t* fld, size_t nq,
+                          uint64_t* out_offsets, uint8_t* out, size_t out_cap)
+{
+    int rc = values_prepare(idx);
+    if (rc) return rc;
+    if (!out_offsets || (nq && (!rec || !fld))) return fail(idx->ctx, CSVB200_ERR_INVALID_ARG, "null argument");
+    out_offsets[0] = 0;
+    if (nq == 0) return CSVB200_OK;
+    size_t len = 0;
+    return csvb200_seek_values(idx, rec, fld, nq, CSVB200_FIELD_RAW, out_offsets, out, out_cap, &len, nullptr);
 }
 
 // enqueue lengths + scan (+ write when d_out != nullptr) of one column on the context's stream

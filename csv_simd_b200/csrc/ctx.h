@@ -238,6 +238,11 @@ int materialize_multi_enqueue(csvb200_ctx* ctx, const MatSource& src, const uint
                               uint32_t first_record, uint32_t nrec, uint32_t flags, uint64_t* const* d_offsets,
                               uint8_t* const* d_outs, const size_t* out_caps, const uint64_t* offset_base, bool offsets_pass,
                               bool write_pass);
+// Enqueues the offsets pass of csvb200_seek_values (p.offsets, p.found, p.counts filled by the caller; the scratch is
+// the context's) and, when write_pass and p.out, the write pass, on the context's stream.  The source is one index
+// object (local) or the segments and shards of a distributed index (seg, sb).
+int values_enqueue(csvb200_ctx* ctx, ValuesParams p, const ValuesLocal* local, const SegmentTable* seg, const ShardBytes* sb,
+                   bool write_pass);
 // The slots of Tape::chunks(num) (src/tape.rs:95-140) over boundaries(record_cnt, num): every field of out[0 .. *n_out)
 // but byte_start / byte_end.  CSVB200_ERR_INVALID_STATE when record_cnt or num is 0, CSVB200_ERR_CAPACITY (with *n_out
 // set) when out_cap is short; tape_chunk_error gives the message the chunk calls report with either.

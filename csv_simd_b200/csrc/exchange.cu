@@ -650,6 +650,198 @@ int csvb200_multi_index_build_to_host(csvb200_multi* m, const uint8_t* host_byte
 }  // extern "C"
 
 // ---------------------------------------------------------------------------------------------------------------
+// the values behind a batch of lookups over the distributed index: every device resolves a share of the batch, reading
+// index slots and bytes from whichever device holds them (peer loads into the shards, nothing is staged)
+// ---------------------------------------------------------------------------------------------------------------
+namespace {
+
+int first_device_error(csvb200_multi* m, const std::vector<int>& rcs);
+
+ShardBytes shard_bytes(const csvb200_multi_index* mi)
+{
+    ShardBytes sb{};
+    sb.nshard = (uint32_t)mi->seg.size();
+    for (size_t k = 0; k < mi->seg.size(); ++k) sb.ptr[k] = mi->d_bytes[k];
+    for (size_t k = 0; k < mi->cuts.size(); ++k) sb.cut[k] = mi->cuts[k];
+    return sb;
+}
+
+ValuesParams multi_values_params(const csvb200_multi_index* mi, const uint32_t* rec, const uint32_t* fld, size_t nq,
+                                 uint32_t flags)
+{
+    ValuesParams p{};
+    p.index_len = mi->base.back();
+    p.record_cnt = mi->record_cnt;
+    p.field_cnt = mi->field_cnt;
+    p.row_size = (uint32_t)mi->jump;
+    p.flags = flags;
+    p.rec = rec;
+    p.fld = fld;
+    p.nq = nq;
+    return p;
+}
+
+int multi_values_args(csvb200_multi_index* mi, const void* rec, const void* fld, size_t nq, uint32_t flags, const void* offsets)
+{
+    csvb200_multi* m = mi->m;
+    if (!mi->tape_ready) return mfail(m, CSVB200_ERR_INVALID_STATE, "csvb200_multi_tape_init has not been called");
+    if (!offsets || (nq && !rec)) return mfail(m, CSVB200_ERR_INVALID_ARG, "null argument");
+    if (flags & ~(CSVB200_FIELD_UNQUOTE | CSVB200_FIELD_TRIM)) return mfail(m, CSVB200_ERR_INVALID_ARG, "unknown field flags");
+    if (flags && !fld) return mfail(m, CSVB200_ERR_INVALID_ARG, "flags apply to fields only (fld == NULL: records)");
+    return CSVB200_OK;
+}
+
+// one device's share of a batch: queries [q0, q1) and what its device made of them
+struct ValuesShare {
+    size_t q0 = 0, q1 = 0;
+    DevBuf rec, fld, off, found, cnt, out;
+    uint64_t total = 0, start = 0;
+    uint32_t counts[2] = {0, 0};
+};
+
+}  // namespace
+
+extern "C" int csvb200_multi_seek_values(csvb200_multi_index* mi, const uint32_t* rec, const uint32_t* fld, size_t nq,
+                                         uint32_t flags, uint64_t* out_offsets, uint8_t* out, size_t out_cap, size_t* out_len,
+                                         uint64_t* found_bits)
+{
+    if (!mi) return CSVB200_ERR_INVALID_ARG;
+    csvb200_multi* m = mi->m;
+    int rc = multi_values_args(mi, rec, fld, nq, flags, out_offsets);
+    if (rc) return rc;
+    if (!out_len) return mfail(m, CSVB200_ERR_INVALID_ARG, "null argument");
+    *out_len = 0;
+    out_offsets[0] = 0;
+    if (nq == 0) return CSVB200_OK;
+    // one share per device, as multi_seek splits a batch; the boundaries are multiples of 64 queries, so that every
+    // device writes whole words of the found bits
+    const int G = (int)mi->seg.size();
+    std::vector<ValuesShare> sh(G);
+    for (int k = 0; k < G; ++k) {
+        sh[k].q0 = k == 0 ? 0 : sh[k - 1].q1;
+        sh[k].q1 = k + 1 == G ? nq : std::max(sh[k].q0, std::min(nq, (nq * (k + 1) / G + 63) / 64 * 64));
+    }
+    const ShardBytes sb = shard_bytes(mi);
+    std::vector<int> rcs(G, CSVB200_OK);
+    // pass 1: lengths, offsets from 0 and found bits of every share on its device; only the totals come back
+    run_phase(m, [&](int k) {
+        csvb200_ctx* ctx = m->ctx[k];
+        ValuesShare& s = sh[k];
+        const size_t n = s.q1 - s.q0;
+        if (n == 0) return;
+        rcs[k] = [&]() -> int {
+            CU_TRY(ctx, cudaSetDevice(ctx->device));
+            CU_TRY(ctx, s.rec.alloc(n * sizeof(uint32_t), ctx->stream));
+            if (fld) CU_TRY(ctx, s.fld.alloc(n * sizeof(uint32_t), ctx->stream));
+            CU_TRY(ctx, s.off.alloc((n + 1) * sizeof(uint64_t), ctx->stream));
+            if (found_bits) CU_TRY(ctx, s.found.alloc((n + 63) / 64 * sizeof(uint64_t), ctx->stream));
+            CU_TRY(ctx, s.cnt.alloc(2 * sizeof(uint32_t), ctx->stream));
+            CU_TRY(ctx, cudaMemsetAsync(s.cnt.p, 0, 2 * sizeof(uint32_t), ctx->stream));
+            CU_TRY(ctx, cudaMemcpyAsync(s.rec.p, rec + s.q0, n * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+            if (fld) CU_TRY(ctx, cudaMemcpyAsync(s.fld.p, fld + s.q0, n * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+            ValuesParams p = multi_values_params(mi, s.rec.as<uint32_t>(), fld ? s.fld.as<uint32_t>() : nullptr, n, flags);
+            p.offsets = s.off.as<uint64_t>();
+            p.found = found_bits ? s.found.as<uint32_t>() : nullptr;
+            p.counts = s.cnt.as<uint32_t>();
+            int rc2 = values_enqueue(ctx, p, nullptr, &mi->table, &sb, false);
+            if (rc2) return rc2;
+            CU_TRY(ctx, cudaMemcpyAsync(&s.total, s.off.as<uint64_t>() + n, sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
+            CU_TRY(ctx, cudaMemcpyAsync(s.counts, s.cnt.p, sizeof(s.counts), cudaMemcpyDeviceToHost, ctx->stream));
+            CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+            return CSVB200_OK;
+        }();
+    });
+    rc = first_device_error(m, rcs);
+    uint64_t total = 0;
+    bool oob = false, outside = false;
+    for (ValuesShare& s : sh) {
+        s.start = total;
+        total += s.total;
+        oob = oob || s.counts[0];
+        outside = outside || s.counts[1];
+    }
+    if (!rc && oob) rc = mfail(m, CSVB200_ERR_OUT_OF_BOUNDS, "lookup slot past the end of the index");
+    if (!rc && outside) rc = mfail(m, CSVB200_ERR_OUT_OF_BOUNDS, "value lies outside the input");
+    const bool small = total > out_cap, write = !small && out != nullptr;
+    if (!rc) {
+        *out_len = (size_t)total;
+        // pass 2: the values (when they fit), the offsets again with the share's start added, and the found bits go
+        // from every device straight to their place in the caller's arrays; the offsets come down even when the values
+        // do not (CSVB200_ERR_CAPACITY, the sizing call)
+        run_phase(m, [&](int k) {
+            csvb200_ctx* ctx = m->ctx[k];
+            ValuesShare& s = sh[k];
+            const size_t n = s.q1 - s.q0;
+            if (n == 0) return;
+            rcs[k] = [&]() -> int {
+                CU_TRY(ctx, cudaSetDevice(ctx->device));
+                ValuesParams p = multi_values_params(mi, s.rec.as<uint32_t>(), fld ? s.fld.as<uint32_t>() : nullptr, n, flags);
+                p.offsets = s.off.as<uint64_t>();
+                if (write && s.total) {
+                    CU_TRY(ctx, s.out.alloc(s.total, ctx->stream));
+                    p.out = s.out.as<uint8_t>();
+                    p.out_cap = s.total;
+                    CU_TRY(ctx, launch_values_write_sharded(p, mi->table, sb, ctx->stream));
+                    ctx->launches += 1;
+                }
+                p.out = nullptr;
+                p.offset_base = s.start;
+                p.counts = s.cnt.as<uint32_t>();
+                int rc2 = values_enqueue(ctx, p, nullptr, &mi->table, &sb, false);
+                if (rc2) return rc2;
+                // adjacent shares share one offset: each brings its own queries' offsets, the last share the end too
+                const size_t n_off = n + (s.q1 == nq ? 1 : 0);
+                CU_TRY(ctx, cudaMemcpyAsync(out_offsets + s.q0, s.off.p, n_off * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
+                if (found_bits)
+                    CU_TRY(ctx, cudaMemcpyAsync(found_bits + s.q0 / 64, s.found.p, (n + 63) / 64 * sizeof(uint64_t),
+                                                cudaMemcpyDeviceToHost, ctx->stream));
+                if (write && s.total)
+                    CU_TRY(ctx, cudaMemcpyAsync(out + s.start, s.out.p, s.total, cudaMemcpyDeviceToHost, ctx->stream));
+                CU_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+                return CSVB200_OK;
+            }();
+        });
+        rc = first_device_error(m, rcs);
+    }
+    // every buffer goes back to the pool of the device it came from, on that device's stream
+    run_phase(m, [&](int k) {
+        cudaSetDevice(m->ctx[k]->device);
+        ValuesShare& s = sh[k];
+        s.rec.reset();
+        s.fld.reset();
+        s.off.reset();
+        s.found.reset();
+        s.cnt.reset();
+        s.out.reset();
+    });
+    cudaGetLastError();
+    if (rc) return rc;
+    if (small) return mfail(m, CSVB200_ERR_CAPACITY, "values destination too small");
+    if (total && !out) return mfail(m, CSVB200_ERR_INVALID_ARG, "null argument");
+    return CSVB200_OK;
+}
+
+extern "C" int csvb200_multi_seek_values_device(csvb200_multi_index* mi, int k, const uint32_t* d_rec, const uint32_t* d_fld,
+                                                size_t nq, uint32_t flags, uint64_t* d_offsets, uint8_t* d_out, size_t out_cap,
+                                                uint64_t* d_found_bits)
+{
+    if (!mi || k < 0 || k >= (int)mi->seg.size()) return CSVB200_ERR_INVALID_ARG;
+    int rc = multi_values_args(mi, d_rec, d_fld, nq, flags, d_offsets);
+    if (rc) return rc;
+    csvb200_ctx* ctx = mi->m->ctx[k];
+    CU_TRY(ctx, cudaSetDevice(ctx->device));
+    ValuesParams p = multi_values_params(mi, d_rec, d_fld, nq, flags);
+    p.offsets = d_offsets;
+    p.out = d_out;
+    p.out_cap = out_cap;
+    p.found = reinterpret_cast<uint32_t*>(d_found_bits);
+    // out-of-bounds slots are reported as None on this asynchronous path
+    p.counts = reinterpret_cast<uint32_t*>(ctx->d_cells + (kCells - 1) * kCellWords);
+    const ShardBytes sb = shard_bytes(mi);
+    return values_enqueue(ctx, p, nullptr, &mi->table, &sb, true);
+}
+
+// ---------------------------------------------------------------------------------------------------------------
 // column materialisation over the distributed index: every device materialises the records whose bytes it holds
 // ---------------------------------------------------------------------------------------------------------------
 namespace {

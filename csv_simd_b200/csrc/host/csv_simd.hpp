@@ -463,6 +463,36 @@ public:
                                              reinterpret_cast<uint8_t*>(&c.bytes[0]), total, &total), index_.ctx());
         return c;
     }
+    // the values behind a batch of lookups: fld non-empty = field fld[q] of record rec[q] (trimmed / unquoted by flags,
+    // as column()), fld empty = the text of record rec[q]; get(q) is nullopt exactly where seek_field / seek_record is
+    struct Values {
+        std::vector<uint64_t> offsets;   // nq + 1
+        std::string bytes;
+        std::vector<uint64_t> found;     // bit q % 64 of word q / 64
+        std::optional<std::string_view> get(size_t q) const
+        {
+            if (!(found[q / 64] >> (q % 64) & 1u)) return std::nullopt;
+            return std::string_view(bytes).substr(offsets[q], offsets[q + 1] - offsets[q]);
+        }
+        size_t size() const { return offsets.empty() ? 0 : offsets.size() - 1; }
+    };
+    Values seek_values(const std::vector<uint32_t>& rec, const std::vector<uint32_t>& fld, uint32_t flags = CSVB200_FIELD_RAW) const
+    {
+        if (!fld.empty() && rec.size() != fld.size()) throw std::invalid_argument("rec / fld size mismatch");
+        Values v;
+        v.offsets.assign(rec.size() + 1, 0);
+        v.found.assign((rec.size() + 63) / 64 + 1, 0);
+        const uint32_t* f = fld.empty() ? nullptr : fld.data();
+        size_t total = 0;
+        int rc = csvb200_seek_values(index_.raw(), rec.data(), f, rec.size(), flags, v.offsets.data(), nullptr, 0, &total,
+                                     v.found.data());
+        if (rc != CSVB200_ERR_CAPACITY) check(rc, index_.ctx());
+        v.bytes.resize(total);
+        if (total)
+            check(csvb200_seek_values(index_.raw(), rec.data(), f, rec.size(), flags, v.offsets.data(),
+                                      reinterpret_cast<uint8_t*>(&v.bytes[0]), total, &total, v.found.data()), index_.ctx());
+        return v;
+    }
     // core::str::from_utf8 over the whole file: nullopt = well-formed (seek_record hands out &str unchecked, record_source.rs:97-101)
     std::optional<uint64_t> utf8_valid_up_to() const
     {

@@ -161,11 +161,45 @@ struct SegmentTable {
 };
 cudaError_t launch_seek_sharded(const LookupParams& p, const SegmentTable& seg, cudaStream_t stream);
 
-// gather the bytes of resolved ranges into a packed buffer: out[out_off[i] .. out_off[i+1]) = the input bytes
-// [start, end); ranges are GLOBAL positions, bytes[0] is global byte pos_bias and n bytes are addressable
-cudaError_t launch_gather_bytes(const uint8_t* bytes, uint64_t n, uint64_t pos_bias, const uint64_t* ranges,
-                                const uint64_t* out_off, uint64_t nq, uint8_t* out, cudaStream_t stream);
-cudaError_t launch_range_lengths(const uint64_t* ranges, uint64_t nq, uint64_t* lens, cudaStream_t stream);
+// K8 the values behind a batch of lookups (materialize.cu): value q is the field (rec[q], fld[q]) trimmed / unquoted
+// by `flags` as in the materialisation, or, with fld == nullptr, the raw record text of rec[q].  Two passes: lengths +
+// exclusive scan (+ found bits + counters), then the write.
+struct ValuesParams {
+    uint64_t index_len;
+    uint32_t record_cnt, field_cnt, row_size;
+    uint32_t flags;          // 1 = unquote, 2 = trim; 0 for records
+    const uint32_t* rec;
+    const uint32_t* fld;     // nullptr => records
+    uint64_t nq;
+    uint64_t* offsets;       // [nq + 1] exclusive prefix sums of the value lengths, offset_base added
+    uint8_t* out;            // write pass: value q at out + offsets[q] - offset_base; nullptr = no write pass
+    uint64_t out_cap;        // a value that would end past out_cap is skipped whole
+    uint64_t offset_base;
+    uint32_t* found;         // optional: bit q % 32 of word q / 32 = the lookup found a range (whole words are written)
+    uint32_t* counts;        // offsets pass: [0] += slots past the index end, [1] += non-empty ranges outside the bytes
+    uint64_t* tile_desc;     // look-back descriptors (zeroed), values_scratch_bytes(nq) - 128 bytes
+    uint32_t* ticket;        // zeroed
+};
+size_t values_scratch_bytes(uint64_t nq);   // [128 B ticket cell][descriptors]
+// one index object: its entries (entry_bytes each) and the bytes it holds (bytes[0] is global byte pos_bias)
+struct ValuesLocal {
+    const void* index;
+    uint32_t entry_bytes;
+    const uint8_t* bytes;
+    uint64_t n, pos_bias;
+};
+// the shards of a distributed input: global bytes [cut[k], cut[k + 1]) are ptr[k][0 ..), on device k, peer-mapped
+struct ShardBytes {
+    const uint8_t* ptr[kExMaxWorld];
+    uint64_t cut[kExMaxWorld + 1];
+    uint32_t nshard;
+};
+cudaError_t launch_values_offsets(const ValuesParams& p, const ValuesLocal& src, cudaStream_t stream);
+cudaError_t launch_values_write(const ValuesParams& p, const ValuesLocal& src, cudaStream_t stream);
+cudaError_t launch_values_offsets_sharded(const ValuesParams& p, const SegmentTable& seg, const ShardBytes& sb,
+                                          cudaStream_t stream);
+cudaError_t launch_values_write_sharded(const ValuesParams& p, const SegmentTable& seg, const ShardBytes& sb,
+                                        cudaStream_t stream);
 
 // K5 tape validation (tape.cu): first index slot whose separator class does not fit its place in the record
 struct TapeValidateParams {
@@ -272,6 +306,16 @@ __device__ __forceinline__ uint64_t ldg_entry(const uint32_t* p)
     uint32_t v;
     asm volatile("ld.global.nc.u32 %0, [%1];" : "=r"(v) : "l"(p));
     return v;
+}
+// One entry of an index whose segments live on different GPUs: a register-resident search over <= 16 bases, then a
+// plain 8-byte load through the peer mapping (an NVLink read when the slot's owner is another GPU).
+__device__ __forceinline__ uint64_t sharded_entry(const SegmentTable& seg, uint64_t s)
+{
+    uint32_t k = 0;
+#pragma unroll
+    for (uint32_t j = 1; j < kExMaxWorld; ++j)
+        if (j < seg.nseg && s >= seg.base[j]) k = j;
+    return ldg_entry(seg.ptr[k] + (s - seg.base[k]));
 }
 #endif
 

@@ -52,17 +52,7 @@ __global__ void __launch_bounds__(256) seek_kernel(const LookupParams p)
     }
 }
 
-// One entry of an index whose segments live on different GPUs: a register-resident search over <= 16 bases, then a
-// plain 8-byte load through the peer mapping (an NVLink read when the slot's owner is another GPU).
-__device__ __forceinline__ uint64_t sharded_entry(const SegmentTable& seg, uint64_t s)
-{
-    uint32_t k = 0;
-#pragma unroll
-    for (uint32_t j = 1; j < kExMaxWorld; ++j)
-        if (j < seg.nseg && s >= seg.base[j]) k = j;
-    return ldg_entry(seg.ptr[k] + (s - seg.base[k]));
-}
-
+// (sharded_entry, in internal.h, resolves a slot to the segment that holds it)
 __global__ void __launch_bounds__(256) seek_sharded_kernel(const LookupParams p, const SegmentTable seg)
 {
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
@@ -90,37 +80,6 @@ __global__ void __launch_bounds__(256) seek_sharded_kernel(const LookupParams p,
             }
         }
         asm volatile("st.global.v2.u64 [%0], {%1, %2};" ::"l"(p.ranges + 2 * q), "l"(start), "l"(end) : "memory");
-    }
-}
-
-__global__ void __launch_bounds__(256) range_lengths_kernel(const uint64_t* __restrict__ ranges, uint64_t nq,
-                                                            uint64_t* __restrict__ lens)
-{
-    const uint64_t q = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (q >= nq) return;
-    const uint64_t a = ranges[2 * q], b = ranges[2 * q + 1];
-    lens[q] = (a == UINT64_MAX || b < a) ? 0 : b - a;
-}
-
-// eight lanes per range: fields are a few bytes long, so a whole warp per range left 3/4 of every request empty
-// (ncu, round 1: 1.0 sectors per request, 0.15 of the HBM peak); four ranges per warp instruction keep four
-// independent sectors in flight per request.  Positions are global: bytes[0] is global byte pos_bias, and a range
-// that does not lie inside [pos_bias, pos_bias + n) (an index of another shard) is skipped, never dereferenced.
-constexpr uint32_t kGatherLanes = 8;
-
-__global__ void __launch_bounds__(256) gather_bytes_kernel(const uint8_t* __restrict__ bytes, uint64_t n, uint64_t pos_bias,
-                                                           const uint64_t* __restrict__ ranges,
-                                                           const uint64_t* __restrict__ out_off, uint64_t nq,
-                                                           uint8_t* __restrict__ out)
-{
-    const uint32_t sub = threadIdx.x & (kGatherLanes - 1u);
-    const uint64_t groups = ((uint64_t)gridDim.x * blockDim.x) / kGatherLanes;
-    for (uint64_t q = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) / kGatherLanes; q < nq; q += groups) {
-        const uint64_t a = ranges[2 * q], b = ranges[2 * q + 1];
-        if (a == UINT64_MAX || b <= a || a < pos_bias || b - pos_bias > n) continue;
-        const uint8_t* src = bytes + (a - pos_bias);
-        uint8_t* dst = out + out_off[q];
-        for (uint64_t i = sub; i < b - a; i += kGatherLanes) dst[i] = src[i];
     }
 }
 
@@ -152,27 +111,6 @@ cudaError_t launch_seek_sharded(const LookupParams& p, const SegmentTable& seg, 
     const uint64_t max_blocks = (uint64_t)sms * 32;
     if (blocks > max_blocks) blocks = max_blocks;
     seek_sharded_kernel<<<(unsigned)blocks, 256, 0, stream>>>(p, seg);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_range_lengths(const uint64_t* ranges, uint64_t nq, uint64_t* lens, cudaStream_t stream)
-{
-    if (nq == 0) return cudaSuccess;
-    range_lengths_kernel<<<(unsigned)((nq + 255) / 256), 256, 0, stream>>>(ranges, nq, lens);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_gather_bytes(const uint8_t* bytes, uint64_t n, uint64_t pos_bias, const uint64_t* ranges,
-                                const uint64_t* out_off, uint64_t nq, uint8_t* out, cudaStream_t stream)
-{
-    if (nq == 0) return cudaSuccess;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    uint64_t blocks = (nq * kGatherLanes + 255) / 256;
-    const uint64_t max_blocks = (uint64_t)sms * 16;
-    if (blocks > max_blocks) blocks = max_blocks;
-    gather_bytes_kernel<<<(unsigned)blocks, 256, 0, stream>>>(bytes, n, pos_bias, ranges, out_off, nq, out);
     return cudaGetLastError();
 }
 

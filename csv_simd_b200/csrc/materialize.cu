@@ -9,6 +9,8 @@
 //   offsets[r - first_record] = exclusive prefix sum of the value lengths, out = values back to back
 // Two kernels: (1) lengths + exclusive scan fused (one pass, decoupled look-back over 62-bit sums),
 // (2) the write.  Both read two index entries per record and the field's bytes: HBM sector-bound.
+// The same helpers serve K8, the values behind a batch of random (record, field) or record lookups, on one index object
+// or straight from the shards of a distributed input (values_offsets_kernel / values_write_kernel below).
 #include "internal.h"
 
 namespace csvb200 {
@@ -482,7 +484,337 @@ __global__ void __launch_bounds__(kMultiThreads) materialize_multi_write_kernel(
     }
 }
 
+// ---- the values behind a batch of lookups ------------------------------------------------------------------------
+// A query resolves as the seek kernels resolve it (lookup.cu), to a range [a, b) of GLOBAL byte positions; its value is
+// that slice, trimmed / unquoted by the field helpers above.  A source says where the bytes of a range live: one buffer
+// (an index object and the bytes it holds), or the shards of a distributed input on several GPUs.
+struct Piece {
+    const uint8_t* x;   // 16-byte aligned buffer holding global bytes [bias, bias + n)
+    uint64_t n, bias;
+};
+
+template <class E>
+struct LocalSource {
+    const E* index;
+    const uint8_t* bytes;
+    uint64_t n, pos_bias;
+    __device__ __forceinline__ uint64_t entry(uint64_t s) const { return ldg_entry(index + s); }
+    // a non-empty range the bytes hold in full
+    __device__ __forceinline__ bool holds(uint64_t a, uint64_t b) const { return a >= pos_bias && b - pos_bias <= n; }
+    __device__ __forceinline__ bool piece(uint64_t, uint64_t, Piece& pc) const
+    {
+        pc = Piece{bytes, n, pos_bias};
+        return true;
+    }
+    __device__ __forceinline__ uint32_t byte(uint64_t pos) const { return bytes[pos - pos_bias]; }
+    template <class F>
+    __device__ __forceinline__ void for_each_piece(uint64_t a, uint64_t b, F&& f) const
+    {
+        f(Piece{bytes, n, pos_bias}, a, b);
+    }
+};
+
+struct ShardedSource {
+    SegmentTable seg;
+    ShardBytes sb;
+    __device__ __forceinline__ uint64_t entry(uint64_t s) const { return sharded_entry(seg, s); }
+    __device__ __forceinline__ bool holds(uint64_t, uint64_t b) const { return b <= sb.cut[sb.nshard]; }
+    // the shard of global byte pos (< the input length): the last one starting at or before it, so empty shards are
+    // passed over
+    __device__ __forceinline__ uint32_t shard_of(uint64_t pos) const
+    {
+        uint32_t k = 0;
+#pragma unroll
+        for (uint32_t j = 1; j < kExMaxWorld; ++j)
+            if (j < sb.nshard && pos >= sb.cut[j]) k = j;
+        return k;
+    }
+    __device__ __forceinline__ Piece piece_of(uint32_t k) const { return Piece{sb.ptr[k], sb.cut[k + 1] - sb.cut[k], sb.cut[k]}; }
+    // false: the range contains a cut
+    __device__ __forceinline__ bool piece(uint64_t a, uint64_t b, Piece& pc) const
+    {
+        const uint32_t k = shard_of(a);
+        pc = piece_of(k);
+        return b <= sb.cut[k + 1];
+    }
+    __device__ __forceinline__ uint32_t byte(uint64_t pos) const
+    {
+        const uint32_t k = shard_of(pos);
+        return ldg_u8(sb.ptr[k] + (pos - sb.cut[k]));
+    }
+    template <class F>
+    __device__ __forceinline__ void for_each_piece(uint64_t a, uint64_t b, F&& f) const
+    {
+        for (uint32_t k = shard_of(a); k < sb.nshard && sb.cut[k] < b; ++k) {
+            const uint64_t lo = a > sb.cut[k] ? a : sb.cut[k], hi = b < sb.cut[k + 1] ? b : sb.cut[k + 1];
+            if (lo < hi) f(piece_of(k), lo, hi);
+        }
+    }
+};
+
+// the range of query q, as seek_kernel finds it; false = None (a slot past the index end also bumps *oob)
+template <class Src>
+__device__ __forceinline__ bool value_range(const ValuesParams& p, const Src& src, uint64_t q, uint32_t* oob, uint64_t& a,
+                                            uint64_t& b)
+{
+    const uint32_t r = p.rec[q];
+    bool live = (uint32_t)(r + 1u) < p.record_cnt;
+    uint32_t s;
+    uint64_t e_slot;
+    if (p.fld != nullptr) {
+        const uint32_t f = p.fld[q];
+        live = live && f < p.field_cnt;
+        s = (uint32_t)(r + 1u) * p.row_size + f;   // u32 arithmetic, as the reference
+        e_slot = (uint64_t)s + 1;
+    } else {
+        s = (uint32_t)(r + 1u) * p.row_size;
+        e_slot = (uint64_t)s + p.field_cnt;
+    }
+    if (!live) return false;
+    if (e_slot >= p.index_len) {
+        if (oob) atomicAdd(oob, 1u);
+        return false;
+    }
+    a = src.entry(s) + 1;
+    b = src.entry(e_slot);
+    return true;
+}
+
+// The value of a range that contains a cut, a byte at a time (each byte from the shard that holds it): the same trim,
+// quote test and Unquoter as emit_value.  At most one field gap per cut takes this path.
+template <class Src, class Put>
+__device__ __forceinline__ void walk_value(const Src& src, uint32_t flags, uint64_t a, uint64_t b, Put put)
+{
+    if (flags & 2u) {
+        while (a < b && (src.byte(a) == 0x20u || src.byte(a) == 0x09u)) ++a;
+        while (b > a && (src.byte(b - 1) == 0x20u || src.byte(b - 1) == 0x09u)) --b;
+    }
+    if ((flags & 1u) && b - a >= 2 && src.byte(a) == 0x22u && src.byte(b - 1) == 0x22u) {
+        Unquoter<Put> u{put};
+        for (uint64_t i = a + 1; i + 1 < b; ++i) u(src.byte(i));
+        u.finish();
+        return;
+    }
+    for (uint64_t i = a; i < b; ++i) put(src.byte(i));
+}
+
+template <class Src>
+__device__ __forceinline__ uint64_t value_length(const Src& src, uint32_t flags, uint64_t a, uint64_t b)
+{
+    if (flags == 0u) return b - a;
+    Piece pc;
+    if (src.piece(a, b, pc)) {
+        const FieldView<uint64_t> fv{nullptr, 0, pc.x, pc.n, pc.bias, 0, 0, 0, 0, flags};
+        return value_len_range(fv, a - pc.bias, b - pc.bias);
+    }
+    uint64_t o = 0;
+    walk_value(src, flags, a, b, [&](uint32_t) { ++o; });
+    return o;
+}
+
+constexpr int kValThreads = 256;
+constexpr int kValItems = 4;
+constexpr int kValTile = kValThreads * kValItems;
+
+// Lengths, found bits and exclusive offsets of a tile of 1024 queries.  Item k of thread t is query tile * 1024 +
+// 256 k + t, so that a warp's ballot is 32 consecutive found bits (one u32 word); the lengths go through shared memory
+// to the blocked layout of the scan (thread t sums queries 4 t .. 4 t + 3), then a decoupled look-back over the tiles.
+template <class Src>
+__global__ void __launch_bounds__(kValThreads) values_offsets_kernel(const ValuesParams p, const Src src)
+{
+    __shared__ uint64_t s_len[kValTile];
+    __shared__ uint64_t s_warp[kValThreads / 32];
+    __shared__ uint64_t s_prefix;
+    __shared__ uint32_t s_tile;
+    const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
+    if (tid == 0) s_tile = atomicAdd(p.ticket, 1u);   // tiles are taken in order: look-back only waits on started tiles
+    __syncthreads();
+    const uint32_t tile = s_tile;
+    const uint64_t t0 = (uint64_t)tile * kValTile;
+#pragma unroll 1
+    for (int k = 0; k < kValItems; ++k) {
+        const uint64_t q = t0 + (uint64_t)k * kValThreads + tid;
+        uint64_t a = 0, b = 0, len = 0;
+        const bool found = q < p.nq && value_range(p, src, q, p.counts, a, b);
+        if (found && b > a) {
+            if (src.holds(a, b))
+                len = value_length(src, p.flags, a, b);
+            else
+                atomicAdd(p.counts + 1, 1u);
+        }
+        const uint32_t bits = __ballot_sync(0xffffffffu, found);
+        const uint64_t q_warp = q - lane;
+        if (p.found && lane == 0 && q_warp < ((p.nq + 63) & ~63ull)) p.found[q_warp / 32] = bits;   // whole u64 words
+        s_len[k * kValThreads + tid] = len;
+    }
+    __syncthreads();
+    const uint64_t i0 = t0 + (uint64_t)tid * kValItems;
+    uint64_t len[kValItems], tsum = 0;
+#pragma unroll
+    for (int k = 0; k < kValItems; ++k) {
+        len[k] = s_len[tid * kValItems + k];
+        tsum += len[k];
+    }
+    uint64_t inc = tsum;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const uint64_t v = __shfl_up_sync(0xffffffffu, inc, d);
+        if (lane >= (uint32_t)d) inc += v;
+    }
+    if (lane == 31) s_warp[warp] = inc;
+    __syncthreads();
+    uint64_t wbase = 0, total = 0;
+#pragma unroll
+    for (int w = 0; w < kValThreads / 32; ++w) {
+        if (w < (int)warp) wbase += s_warp[w];
+        total += s_warp[w];
+    }
+    if (tid == 0) s_prefix = lookback(p.tile_desc, tile, total);
+    __syncthreads();
+    uint64_t off = p.offset_base + s_prefix + wbase + (inc - tsum);
+#pragma unroll
+    for (int k = 0; k < kValItems; ++k) {
+        if (i0 + k < p.nq) p.offsets[i0 + k] = off;
+        off += len[k];
+    }
+    if (i0 < p.nq && i0 + kValItems >= p.nq) p.offsets[p.nq] = off;   // the thread owning the last query
+}
+
+__device__ __forceinline__ void st_128(void* p, uint4 v)
+{
+    asm volatile("st.global.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
+}
+
+// x[a, b) -> dst[0, b - a) by the kL lanes of a group (sub = lane in the group): each lane takes aligned 16-byte words
+// of the source in turn; a word that lands 16-byte aligned in dst and lies inside the range goes out as one store,
+// the others byte by byte.  Words that would read past n are fetched bytewise.
+template <int kL>
+__device__ __forceinline__ void group_copy(uint8_t* __restrict__ dst, const uint8_t* __restrict__ x, uint64_t n, uint64_t a,
+                                           uint64_t b, uint32_t sub)
+{
+    for (uint64_t base = (a & ~15ull) + 16ull * sub; base < b; base += 16ull * kL) {
+        uint4 v;
+        if (base + 16 <= n) {
+            v = ldg_128(x + base);
+        } else {
+            uint32_t w[4];
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                uint32_t t = 0;
+                for (int j = 0; j < 4; ++j)
+                    if (base + 4 * k + j < n) t |= (uint32_t)x[base + 4 * k + j] << (8 * j);
+                w[k] = t;
+            }
+            v = make_uint4(w[0], w[1], w[2], w[3]);
+        }
+        const uint32_t lo = a > base ? (uint32_t)(a - base) : 0u;
+        const uint32_t hi = b - base < 16 ? (uint32_t)(b - base) : 16u;
+        if (lo == 0 && hi == 16 && ((reinterpret_cast<uintptr_t>(dst) + (base - a)) & 15u) == 0) {
+            st_128(dst + (base - a), v);
+            continue;
+        }
+        const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+        for (int k = 0; k < 16; ++k)
+            if ((uint32_t)k >= lo && (uint32_t)k < hi) dst[base + k - a] = (uint8_t)(w[k >> 2] >> (8 * (k & 3)));
+    }
+}
+
+// kL lanes per value: raw values (records, fields with flags == 0) are range copies, 8 lanes for fields (a few bytes
+// each: four values per warp instruction keep four independent sectors in flight) and 32 for records (kilobytes);
+// kL == 1: one thread per value through emit_value (TRIM / UNQUOTE).
+template <class Src, int kL>
+__global__ void __launch_bounds__(256) values_write_kernel(const ValuesParams p, const Src src)
+{
+    const uint32_t sub = threadIdx.x & (kL - 1u);
+    const uint64_t groups = ((uint64_t)gridDim.x * blockDim.x) / kL;
+    uint8_t* __restrict__ out = p.out;
+    for (uint64_t q = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) / kL; q < p.nq; q += groups) {
+        uint64_t a, b;
+        if (!value_range(p, src, q, nullptr, a, b) || b <= a || !src.holds(a, b)) continue;
+        const uint64_t o = p.offsets[q] - p.offset_base, o_end = p.offsets[q + 1] - p.offset_base;
+        if (o_end > p.out_cap || o_end == o) continue;   // the device form skips whole values past out_cap
+        if (kL > 1) {
+            src.for_each_piece(a, b, [&](const Piece& pc, uint64_t lo, uint64_t hi) {
+                group_copy<kL>(out + o + (lo - a), pc.x, pc.n, lo - pc.bias, hi - pc.bias, sub);
+            });
+            continue;
+        }
+        uint64_t at = o;
+        auto put = [&](uint32_t c) { out[at++] = (uint8_t)c; };
+        Piece pc;
+        if (src.piece(a, b, pc)) {
+            const FieldView<uint64_t> fv{nullptr, 0, pc.x, pc.n, pc.bias, 0, 0, 0, 0, p.flags};
+            const uint8_t* __restrict__ x = pc.x;
+            emit_value(fv, x, a - pc.bias, b - pc.bias, put);
+        } else {
+            walk_value(src, p.flags, a, b, put);
+        }
+    }
+}
+
+template <class Src>
+cudaError_t values_offsets(const ValuesParams& p, const Src& src, cudaStream_t stream)
+{
+    const uint64_t tiles = (p.nq + kValTile - 1) / kValTile;
+    if (tiles == 0) return cudaSuccess;
+    values_offsets_kernel<Src><<<(unsigned)tiles, kValThreads, 0, stream>>>(p, src);
+    return cudaGetLastError();
+}
+
+template <class Src>
+cudaError_t values_write(const ValuesParams& p, const Src& src, cudaStream_t stream)
+{
+    if (p.nq == 0 || p.out == nullptr) return cudaSuccess;
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int lanes = p.flags ? 1 : p.fld ? 8 : 32;
+    uint64_t blocks = (p.nq * lanes + 255) / 256;
+    const uint64_t max_blocks = (uint64_t)sms * 16;
+    if (blocks > max_blocks) blocks = max_blocks;
+    if (lanes == 1)
+        values_write_kernel<Src, 1><<<(unsigned)blocks, 256, 0, stream>>>(p, src);
+    else if (lanes == 8)
+        values_write_kernel<Src, 8><<<(unsigned)blocks, 256, 0, stream>>>(p, src);
+    else
+        values_write_kernel<Src, 32><<<(unsigned)blocks, 256, 0, stream>>>(p, src);
+    return cudaGetLastError();
+}
+
+template <class E>
+LocalSource<E> local_source(const ValuesLocal& s)
+{
+    return LocalSource<E>{static_cast<const E*>(s.index), s.bytes, s.n, s.pos_bias};
+}
+
 }  // namespace
+
+size_t values_scratch_bytes(uint64_t nq) { return 128 + ((nq + kValTile - 1) / kValTile + 1) * sizeof(uint64_t); }
+
+cudaError_t launch_values_offsets(const ValuesParams& p, const ValuesLocal& src, cudaStream_t stream)
+{
+    return src.entry_bytes == 4 ? values_offsets(p, local_source<uint32_t>(src), stream)
+                                : values_offsets(p, local_source<uint64_t>(src), stream);
+}
+
+cudaError_t launch_values_write(const ValuesParams& p, const ValuesLocal& src, cudaStream_t stream)
+{
+    return src.entry_bytes == 4 ? values_write(p, local_source<uint32_t>(src), stream)
+                                : values_write(p, local_source<uint64_t>(src), stream);
+}
+
+cudaError_t launch_values_offsets_sharded(const ValuesParams& p, const SegmentTable& seg, const ShardBytes& sb,
+                                          cudaStream_t stream)
+{
+    return values_offsets(p, ShardedSource{seg, sb}, stream);
+}
+
+cudaError_t launch_values_write_sharded(const ValuesParams& p, const SegmentTable& seg, const ShardBytes& sb,
+                                        cudaStream_t stream)
+{
+    return values_write(p, ShardedSource{seg, sb}, stream);
+}
 
 size_t materialize_multi_scratch_bytes(uint32_t nrec, uint32_t ncols)
 {

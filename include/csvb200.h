@@ -378,9 +378,37 @@ int csvb200_seek_fields_device(csvb200_index* idx, const uint32_t* d_rec, const 
                                csvb200_range* d_out);
 int csvb200_seek_records_device(csvb200_index* idx, const uint32_t* d_rec, size_t nq, csvb200_range* d_out);
 /* materialise the field bytes of a batch (needs CSVB200_BUILD_KEEP_BYTES): out_offsets[nq+1] are
- * exclusive prefix sums of the lengths, out receives the packed bytes (out_cap bytes). */
+ * exclusive prefix sums of the lengths, out receives the packed bytes (out_cap bytes).  The raw form
+ * (flags 0) of csvb200_seek_values below. */
 int csvb200_gather_fields(csvb200_index* idx, const uint32_t* rec, const uint32_t* fld, size_t nq,
                           uint64_t* out_offsets, uint8_t* out, size_t out_cap);
+
+/* ---- the values behind a batch of lookups (record number + index -> record; record + field index + index -> field
+ * value: what the caller of seek_record / seek_field does with the range it gets back) -------------------------- */
+/* The values behind a batch of lookups.  fld != NULL: value q is the field that csvb200_seek_fields returns for
+ * (rec[q], fld[q]), trimmed / unquoted by `flags` exactly as csvb200_materialize_column does (CSVB200_FIELD_*).
+ * fld == NULL: value q is the record text that csvb200_seek_records returns for rec[q]; flags must be 0.
+ * A query seek_* answers with None contributes an empty value and a 0 bit in found_bits (optional, (nq + 63) / 64
+ * words, bit q % 64 of word q / 64).  out_offsets[nq + 1] = exclusive prefix sums of the lengths.  Needs the input
+ * bytes (CSVB200_BUILD_KEEP_BYTES, or a device-built index whose input is still alive), else
+ * CSVB200_ERR_INVALID_STATE.  Host form: *out_len = total; CSVB200_ERR_OUT_OF_BOUNDS when a slot lies past the index
+ * end or a non-empty range outside the bytes the index object holds (checked before the capacity);
+ * CSVB200_ERR_CAPACITY (offsets and *out_len valid, out not written) when out_cap is too small. */
+int csvb200_seek_values(csvb200_index* idx, const uint32_t* rec, const uint32_t* fld, size_t nq, uint32_t flags,
+                        uint64_t* out_offsets, uint8_t* out, size_t out_cap, size_t* out_len, uint64_t* found_bits);
+/* device arrays in / out, asynchronous on the context's stream; d_out NULL = offsets only; a value that would end
+ * past out_cap is skipped whole; a slot past the index end is None (as csvb200_seek_fields_device) */
+int csvb200_seek_values_device(csvb200_index* idx, const uint32_t* d_rec, const uint32_t* d_fld, size_t nq, uint32_t flags,
+                               uint64_t* d_offsets, uint8_t* d_out, size_t out_cap, uint64_t* d_found_bits);
+/* the same over the distributed index, host arrays; values equal byte for byte to csvb200_seek_values on a one-GPU
+ * index of the same bytes.  Every device resolves an equal share of the batch and reads the index slots and the bytes
+ * of its values from whichever device holds them; offsets and values go from every device straight to their place. */
+int csvb200_multi_seek_values(csvb200_multi_index* mi, const uint32_t* rec, const uint32_t* fld, size_t nq, uint32_t flags,
+                              uint64_t* out_offsets, uint8_t* out, size_t out_cap, size_t* out_len, uint64_t* found_bits);
+/* device arrays on device number k of the list, asynchronous on that device's stream (csvb200_multi_stream) */
+int csvb200_multi_seek_values_device(csvb200_multi_index* mi, int k, const uint32_t* d_rec, const uint32_t* d_fld, size_t nq,
+                                     uint32_t flags, uint64_t* d_offsets, uint8_t* d_out, size_t out_cap,
+                                     uint64_t* d_found_bits);
 
 /* ---- column materialisation (beyond the reference: seek_field returns the RAW slice incl. quotes and
  * padding, src/record_source.rs:135-139) ----------------------------------------------------------- */

@@ -40,6 +40,35 @@ pub trait BatchedSeeks {
     /// `(start, end)` byte ranges of many `(record, field)` pairs; `None` exactly where `seek_field` returns `Ok(None)`.
     fn seek_fields(&self, rec: &[u32], fld: &[u32]) -> Result<Vec<Option<(usize, usize)>>, StructureError>;
     fn seek_records(&self, rec: &[u32]) -> Result<Vec<Option<(usize, usize)>>, StructureError>;
+    /// The values behind `seek_fields`: field `fld[q]` of record `rec[q]`, trimmed / unquoted by `flags`
+    /// (`sys::CSVB200_FIELD_*`), packed on the GPU.
+    fn field_values(&self, rec: &[u32], fld: &[u32], flags: u32) -> Result<Values, StructureError>;
+    /// The record text behind `seek_records`.
+    fn record_values(&self, rec: &[u32]) -> Result<Values, StructureError>;
+}
+
+/// Packed values of a batch: value `q` is `bytes[offsets[q]..offsets[q + 1]]`.
+pub struct Values {
+    pub offsets: Vec<u64>,
+    pub bytes: Vec<u8>,
+    /// bit `q % 64` of word `q / 64`: the lookup found a range
+    pub found: Vec<u64>,
+}
+
+impl Values {
+    /// `None` exactly where `seek_field` / `seek_record` return `Ok(None)`.
+    pub fn get(&self, q: usize) -> Option<&[u8]> {
+        if (self.found[q / 64] >> (q % 64)) & 1 == 0 {
+            return None;
+        }
+        Some(&self.bytes[self.offsets[q] as usize..self.offsets[q + 1] as usize])
+    }
+    pub fn len(&self) -> usize {
+        self.offsets.len() - 1
+    }
+    pub fn is_empty(&self) -> bool {
+        self.len() == 0
+    }
 }
 
 fn ranges(out: Vec<sys::csvb200_range>) -> Vec<Option<(usize, usize)>> {
@@ -59,5 +88,36 @@ impl BatchedSeeks for DeviceTape<'_> {
         check(unsafe { sys::csvb200_seek_records(self.idx, rec.as_ptr(), rec.len(), out.as_mut_ptr()) },
               || self.gpu.last_error())?;
         Ok(ranges(out))
+    }
+    fn field_values(&self, rec: &[u32], fld: &[u32], flags: u32) -> Result<Values, StructureError> {
+        assert_eq!(rec.len(), fld.len());
+        self.values(rec, fld.as_ptr(), flags)
+    }
+    fn record_values(&self, rec: &[u32]) -> Result<Values, StructureError> {
+        self.values(rec, ptr::null(), 0)
+    }
+}
+
+impl DeviceTape<'_> {
+    // csvb200_seek_values twice: the first call sizes the bytes (CSVB200_ERR_CAPACITY), the second fills them
+    fn values(&self, rec: &[u32], fld: *const u32, flags: u32) -> Result<Values, StructureError> {
+        let nq = rec.len();
+        let mut v = Values { offsets: vec![0; nq + 1], bytes: Vec::new(), found: vec![0; (nq + 63) / 64 + 1] };
+        let mut total = 0usize;
+        let rc = unsafe {
+            sys::csvb200_seek_values(self.idx, rec.as_ptr(), fld, nq, flags, v.offsets.as_mut_ptr(), ptr::null_mut(), 0,
+                                     &mut total, v.found.as_mut_ptr())
+        };
+        if rc != sys::CSVB200_ERR_CAPACITY {
+            check(rc, || self.gpu.last_error())?;
+        }
+        v.bytes = vec![0; total];
+        if total > 0 {
+            check(unsafe {
+                sys::csvb200_seek_values(self.idx, rec.as_ptr(), fld, nq, flags, v.offsets.as_mut_ptr(), v.bytes.as_mut_ptr(),
+                                         total, &mut total, v.found.as_mut_ptr())
+            }, || self.gpu.last_error())?;
+        }
+        Ok(v)
     }
 }

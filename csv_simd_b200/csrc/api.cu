@@ -2053,6 +2053,18 @@ int materialize_multi_enqueue(csvb200_ctx* ctx, const MatSource& src, const uint
     if (ncols == 1)   // one column: the single-column kernels (1024-record tiles) are the faster form
         return materialize_enqueue(ctx, src, fields[0], first_record, nrec, flags, d_offsets[0], d_outs ? d_outs[0] : nullptr,
                                    out_caps ? out_caps[0] : 0, offset_base ? offset_base[0] : 0, offsets_pass, write_pass);
+    // The multi-column kernels keep lengths and tile totals in u32.  Up to 4 GiB that is exact: one column's values over
+    // distinct records are disjoint slices of the input without their line ends, so a tile's total stays below 2^32.
+    // Past 4 GiB a value or a tile can reach 2^32: the columns go one after the other through the u64 kernels.
+    if (src.n > UINT32_MAX) {
+        for (uint32_t c = 0; c < ncols; ++c) {
+            int rc = materialize_enqueue(ctx, src, fields[c], first_record, nrec, flags, d_offsets[c],
+                                         d_outs ? d_outs[c] : nullptr, out_caps ? out_caps[c] : 0,
+                                         offset_base ? offset_base[c] : 0, offsets_pass, write_pass);
+            if (rc) return rc;
+        }
+        return CSVB200_OK;
+    }
     MaterializeMultiParams p{};
     p.index = src.index;
     p.entry_bytes = src.entry_bytes;
